@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: tracked frames/sec of the per-frame hot path (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 The frame is BASELINE.json config 2 (the config the metric is quoted on): ROI Align of a
 [1,512,40,40] map at 64 boxes -> [64,512,10,10], then the association step (predict, cost + gate,
@@ -362,6 +362,25 @@ def dist_summary(ms):
             "first_us": [int(round(v * 1e3)) for v in a[:64]]}
 
 
+DUMP_ROIS = 128          # 26 MB of ROI Align patches: a sample, since a step's whole output is 839 MB for 64 c2 streams
+
+
+def dump_outputs(grp, i, out_dir):
+    """Writes what step i of the stream group handed its caller to out_dir as .npy: the ROI Align patches of a fixed,
+    seeded sample of the step's ROIs (float32 [DUMP_ROIS, 512, 10, 10], rows in the order of roi_align_rows) and the
+    tracker's int32 result table [streams, stride], exactly, as float64.  The inputs are seeded, so two builds run with
+    the same arguments can be compared output for output."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n_roi = grp.S * grp.sh.NBOX
+    rows = np.sort(np.random.default_rng(0).choice(n_roi, min(DUMP_ROIS, n_roi), replace=False))
+    torch.cuda.synchronize(grp.dev)
+    patches = grp.outs[i % grp.nout][torch.from_numpy(rows).to(grp.dev)]
+    np.save(os.path.join(out_dir, "roi_align_patches.npy"), patches.cpu().numpy())
+    np.save(os.path.join(out_dir, "roi_align_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "tracker_results.npy"), grp.results[i].cpu().numpy().astype(np.float64))
+
+
 def oracle_check(dev, frames=40):
     """A fresh 2-stream device-side run (b200_tracker_step with device-resident inputs, the call the timed region
     makes) against the oracle tracker, every result row of every frame."""
@@ -398,7 +417,11 @@ def main():
     ap.add_argument("--gather-every", type=int, default=16,
                     help="N > 1: all-gather the result tables every this many frames")
     ap.add_argument("--no-extra", action="store_true", help="skip the side measurements (other BASELINE configs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 path (--impl b200)")
     quiet_stdout()
     if args.impl == "reference":
         return run_reference(args)
@@ -523,6 +546,8 @@ def main():
     close_gather()
     last = grp.results[pre + W + K - 1].cpu().numpy()
     assert (last[:, 5] == 0).all() and (last[:, 0] > 0).all(), "device path produced no matches"
+    if args.dump_outputs and rank == 0:        # before the roofline probe, which writes into the same output buffers
+        dump_outputs(grp, pre + W + K - 1, args.dump_outputs)
 
     # ---- roofline probe: ROI Align launches alone, after the timed region ---------------------------------
     roi_us = grp.probe_roi(16, first=pre + W)

@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import assert_close, load_golden
+from conftest import assert_close, load_golden, load_roi_wrappers_golden
 from oracle import native
 
 pytestmark = pytest.mark.gpu
@@ -110,7 +110,7 @@ def test_roi_wrappers_match_reference_call_conventions():
 def test_roi_wrappers_vs_reference_golden():
     """roi_align_from_input_boxes / preprocess_roi against fixtures recorded from the reference's OWN methods
     (tracking.py:193-221, trainingCard.py:24-79; tests/golden/make_golden.py::run_roi_wrapper_cases)."""
-    g = load_golden("roi_wrappers")
+    g = load_roi_wrappers_golden()
     for tag in ("sq", "wide"):
         boxes, hw = g[tag + "_boxes"], tuple(int(v) for v in g[tag + "_hw"])
         f = torch.from_numpy(g[tag + "_feat"]).cuda()

@@ -3,7 +3,7 @@
 import numpy as np
 import pytest
 
-from conftest import assert_close, load_golden
+from conftest import assert_close, load_golden, load_roi_wrappers_golden
 from oracle import cost_ref, kalman_ref, lsap_ref, native, roi_wrappers_ref, tracker_ref
 
 
@@ -18,7 +18,7 @@ def test_roi_oracle_vs_golden():
 def test_roi_wrapper_oracle_vs_golden():
     """tracking.py:193-221 and trainingCard.py:24-79 restated, against fixtures recorded from the reference's own
     methods (make_golden.py::run_roi_wrapper_cases)."""
-    g = load_golden("roi_wrappers")
+    g = load_roi_wrappers_golden()
     for tag in ("sq", "wide"):
         feat, boxes, hw = g[tag + "_feat"], g[tag + "_boxes"], tuple(int(v) for v in g[tag + "_hw"])
         for ps in (7, 10):

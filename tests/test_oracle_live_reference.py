@@ -1,74 +1,62 @@
-"""Build-container only (skipped where /root/reference is not mounted): the oracle restatements against the
-UNMODIFIED live reference on randomised inputs, beyond the committed golden fixtures.  This is what pins
-oracle/tracker_ref.py, cost_ref.py and lsap_ref.py; nothing on the GPU / smoke / bench paths imports the reference."""
+"""The oracle restatements against the original project on randomised hyper-parameters, scenes and matrices, beyond the
+cases of test_oracle_golden.py: against the recorded outputs of these cases (tests/golden/live_fuzz.npz; where they
+come from: make_golden.py::run_live_fuzz_cases) and, where the original's tree is mounted, against the original
+itself.  This is
+what pins oracle/tracker_ref.py, cost_ref.py and lsap_ref.py away from the shipped hyper-parameters; nothing on the
+GPU / smoke / bench paths imports the original."""
 import numpy as np
 import pytest
 
-from conftest import assert_close
+from conftest import assert_close, load_golden
+from golden import make_golden
 from oracle import cost_ref, lsap_ref, reference_loader, tracker_ref
 
-import alufe_b200  # noqa: E402,F401
-from alufe_b200 import synth  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not reference_loader.available(), reason="reference tree not mounted")
+def _oracle_tracker(over):
+    return tracker_ref.TrackerRef(dict(tracker_ref.SHIPPED_CONF, **over))
 
-TUNABLE = ("hist_max", "emb_top_k", "max_age", "lost_reid_after", "init_conf_min", "conf_update_min", "cost_max",
-           "cost_update_max", "maha_thr", "reid_only_cost_max", "ema_alpha", "w_bbox")
+
+def _oracle_state(tr):
+    return tr.kf.x, tr.kf.P, tr.ema, len(tr.bank), tr.miss_count, tr.age
+
+
+def _oracle_cal_cost(**kw):
+    return cost_ref.cal_cost(input_hw=(720, 1280), **kw)
+
+
+def _recorded(prefix):
+    g = load_golden("live_fuzz")
+    return {k[len(prefix):]: g[k] for k in g.files if k.startswith(prefix)}
+
+
+def _check_same(got, want, what):
+    """Assignments, ids, counters and inputs exactly; Kalman states and embeddings within the parity bar."""
+    assert sorted(got) == sorted(want), what
+    for k in sorted(want):
+        if "C_" in k or k.endswith(("_x", "_ema")):
+            assert_close(got[k], want[k], what="%s %s" % (what, k))
+        elif k.endswith("_P"):
+            assert_close(got[k], want[k], rtol=1e-5, atol=1e-5, what="%s %s" % (what, k))
+        elif k.endswith("inputs"):
+            assert_close(got[k], want[k], rtol=1e-12, atol=0, what="%s %s: the seeded inputs changed" % (what, k))
+        else:
+            assert np.array_equal(got[k], want[k]), "%s %s" % (what, k)
 
 
 @pytest.mark.parametrize("seed", range(6))
 def test_tracker_oracle_vs_live_reference_fuzz(seed):
     """Random hyper-parameters and scene dynamics (misses, births, empty frames, the ReID-only stage): the oracle
     returns exactly what the reference's Tracking.update returns, frame by frame, and ends in the same state."""
-    rng = np.random.default_rng(500 + seed)
-    over = dict(hist_max=int(rng.choice([1, 3, 30])), emb_top_k=int(rng.choice([1, 5])),
-                max_age=int(rng.choice([1, 6, 40])), lost_reid_after=int(rng.choice([0, 2, 50])),
-                init_conf_min=float(rng.choice([0.0, 0.5, 0.7])), conf_update_min=float(rng.choice([0.0, 0.55, 0.8])),
-                cost_max=float(rng.choice([50.0, 1.0])), cost_update_max=float(rng.choice([30.0, 0.5])),
-                maha_thr=float(rng.choice([9.49, 2.0, 1e6])), reid_only_cost_max=float(rng.choice([0.4, 2.0])),
-                ema_alpha=float(rng.choice([0.9, 0.5])), w_bbox=float(rng.choice([0.3, 2.0])))
-    live = reference_loader.new_tracking()
-    for k, v in over.items():
-        assert hasattr(live, k), k
-        setattr(live, k, v)
-    ref = tracker_ref.TrackerRef(dict(tracker_ref.SHIPPED_CONF, **over))
-    n = int(rng.integers(2, 14))
-    scene = synth.Scene(int(rng.integers(1 << 30)), n, 720, 1280, drop=float(rng.choice([0.0, 0.3])),
-                        churn=float(rng.choice([0.0, 0.3])), churn_every=int(rng.integers(2, 7)))
-    for f in range(18):
-        obj = scene.step()
-        if rng.uniform() < 0.1:
-            obj["embs"], obj["bboxes"], obj["confs"] = [], [], []
-        want = live.update(obj)
-        got = ref.update(obj)
-        assert got[0] == [tuple(m) for m in want[0]] and got[1] == list(want[1]) and got[2] == list(want[2]), \
-            "seed %d frame %d %s" % (seed, f, over)
-    assert sorted(ref.tracks) == sorted(live.tracks) and ref.next_id == live.next_id
-    for tid in sorted(live.tracks):
-        a, b = live.tracks[tid], ref.tracks[tid]
-        assert (a.miss_count, a.age) == (b.miss_count, b.age)
-        assert_close(np.asarray(b.kf.x, np.float64).reshape(-1), np.asarray(a.kf.x, np.float64).reshape(-1), what="x")
-        assert_close(np.asarray(b.kf.P, np.float64), np.asarray(a.kf.P, np.float64), rtol=1e-5, atol=1e-5, what="P")
-        assert_close(np.asarray(b.ema, np.float32), np.asarray(a.memory.encoder_feat, np.float32), what="ema")
-        assert len(b.bank) == len(a.memory.feat_historical)
+    got = make_golden.record_tracker_fuzz(seed, _oracle_tracker, _oracle_state)
+    _check_same(got, _recorded("t%d_" % seed), "seed %d vs recorded" % seed)
+    if reference_loader.available():
+        live = make_golden.record_tracker_fuzz(seed, make_golden.reference_tracker, make_golden.reference_state)
+        _check_same(got, live, "seed %d vs live" % seed)
 
 
 def test_cost_and_assignment_oracles_vs_live_reference_random():
-    ref = reference_loader.load()
-    rng = np.random.default_rng(77)
-    for _ in range(10):
-        M, N = int(rng.integers(1, 20)), int(rng.integers(1, 20))
-        C_app = rng.uniform(0, 2, (M, N)).astype(np.float32)
-        bp = synth.random_boxes(rng, M, 720, 1280)
-        bc = synth.random_boxes(rng, N, 720, 1280)
-        cp, cc = rng.uniform(0.05, 1, M), rng.uniform(0.05, 1, N)
-        import torch
-        live = ref.costCard.cal_cost(C_app=torch.from_numpy(C_app), boxes_prev=bp.tolist(), boxes_cur=bc.tolist(),
-                                     input_hw=(720, 1280), conf_prev=cp.tolist(), conf_cur=cc.tolist())
-        mine = cost_ref.cal_cost(C_app=C_app, boxes_prev=bp, boxes_cur=bc, input_hw=(720, 1280), conf_prev=cp, conf_cur=cc)
-        for k in ("C_total", "C_bbox", "C_center", "C_scale", "C_conf"):
-            assert_close(np.asarray(mine[k], np.float32), live[k].cpu().numpy(), what=k)
-        C = synth.lsap_matrix(rng, M, N, float(rng.choice([0.0, 0.8])))
-        want = ref.hung.hungarian_assign(C, cost_max=50.0)
-        got = lsap_ref.hungarian_assign(C, cost_max=50.0)
-        assert got[0] == [tuple(m) for m in want[0]] and got[1] == list(want[1]) and got[2] == list(want[2])
+    got = make_golden.record_cost_fuzz(_oracle_cal_cost, lsap_ref.hungarian_assign)
+    _check_same(got, _recorded("cost_"), "cost vs recorded")
+    if reference_loader.available():
+        live = make_golden.record_cost_fuzz(make_golden.reference_cal_cost, reference_loader.load().hung.hungarian_assign)
+        _check_same(got, live, "cost vs live")
