@@ -49,6 +49,7 @@ SIGNATURES = {
     "b200_roi_align_fwd_f32": (_I, [_P, _I, _I, _I, _I, _I, _P, _L, _I, _I, _F, _I, _I, _P, _P]),
     "b200_roi_align_fwd_f16": (_I, [_P, _I, _I, _I, _I, _I, _P, _L, _I, _I, _F, _I, _I, _P, _P]),
     "b200_roi_align_fwd_ex": (_I, [_P, _I, _I, _I, _I, _I, _I, _P, _L, _I, _I, _F, _I, _I, _P, _I, _P]),
+    "b200_roi_align_bwd_ex": (_I, [_P, _I, _I, _P, _L, _I, _I, _F, _I, _I, _P, _I, _I, _I, _I, _I, _P]),
     "b200_roi_boxes_prep_f32": (_I, [_P, _L, _I, _P, _I, _I, _I, _I, _I, _F, _P, _P]),
     "b200_app_cost_topk_f32": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _I, _P]),
     "b200_pair_cost_f32": (_I, [_P, _P, _P, _P, _P, _I, _I, _F, _F, _F, _F, _F, _F, _P, _P, _P, _P, _P, _I, _P]),

@@ -1493,6 +1493,447 @@ int roi_align_dispatch(const T* feat, int layout, int B, int C, int H, int W, co
     return check_launch("roi_align_generic_kernel");
 }
 
+// ---- ROI Align backward (torchvision's _roi_align_backward) ---------------------------------------------------
+// The forward pass contracts a footprint with two weight tables, out[ph][pw] = sum_y,x Wy[y][ph] Wx[x][pw] V[y][x];
+// the gradient is its transpose, G[y][x] = sum_ph Wy[y][ph] * (sum_pw Wx[x][pw] * g[ph][pw]), ADDED into grad_in because
+// the footprints of different ROIs overlap.  Same work unit (one warp per (ROI, 32-channel tile), lane = channel), same
+// tables (built per warp, or once per ROI by roi_prep_kernel), G[8][8] in registers.  Kernels, by launch:
+//   roi_align_bwd_tile_kernel  small launches (tables built per warp), and on large ones with prep tables whenever the
+//                              TMA kernel does not apply; scalar red.global.add per cell (NHWC grad_in: one 128-byte line
+//                              per warp instruction);
+//   roi_align_bwd_tma_kernel   large launches into float32 NCHW grad_in: G is written to shared memory in the forward
+//                              pass's box layout V[channel][row][8 cells] and added to the map by the TMA engine
+//                              (cp.reduce.async.bulk.tensor .add, SASS UTMAREDG), 1 / 3 / 5-row boxes as in the forward
+//                              kernel; the grad_out chunk and the tables of the next tile arrive while the current one
+//                              contracts;
+//   footprints the staged path cannot hold take torchvision's algorithm (per-sample scalar atomics) inside the tile
+//   kernel -- after the TMA kernel, in a launch of their own, so that generic-proxy atomics and TMA reductions never
+//   target the same cells concurrently; roi_align_bwd_generic_kernel: output sizes without a template, one thread per
+//   grad_out element, the same algorithm.
+// The order of the additions is not fixed, so the result is not bit-reproducible.
+__device__ __forceinline__ void red_add(float* p, float v) { atomicAdd(p, v); }     // result unused: RED
+
+// grad_in += the four taps of one sample, scaled like torchvision: (g * w) / count.
+__device__ __forceinline__ void bwd_sample(float* __restrict__ gi, size_t ps, int W, const Tap& ty, const Tap& tx, float g,
+                                           float count) {
+    if (!(ty.valid && tx.valid)) return;
+    red_add(gi + ((size_t)ty.lo * W + tx.lo) * ps, __fdiv_rn(g * (ty.wlo * tx.wlo), count));
+    red_add(gi + ((size_t)ty.lo * W + tx.hi) * ps, __fdiv_rn(g * (ty.wlo * tx.whi), count));
+    red_add(gi + ((size_t)ty.hi * W + tx.lo) * ps, __fdiv_rn(g * (ty.whi * tx.wlo), count));
+    red_add(gi + ((size_t)ty.hi * W + tx.hi) * ps, __fdiv_rn(g * (ty.whi * tx.whi), count));
+}
+
+// Element (k, c, bin) of grad_out, stored [K][C][PH*PW] or channels-last [K][PH*PW][C].
+template <typename T, bool GCL>
+__device__ __forceinline__ float grad_at(const T* __restrict__ go, long long k, int C, int NB, int c, int bin) {
+    return ldf<T>(GCL ? go + ((size_t)k * NB + bin) * C + c : go + ((size_t)k * C + c) * NB + bin);
+}
+
+// G[y][x] = sum_ph Wy[y][ph] * sum_pw Wx[x][pw] * g(ph, pw) over the 8 x 8 staged footprint (rows / columns outside the
+// footprint have zero weights, so their G is zero).
+template <int PH, int PW, typename LoadG>
+__device__ __forceinline__ void bwd_contract(float (&G)[kFootCap][kFootCap], const float* sWy, const float* sWx, LoadG loadg) {
+    constexpr int PHP = (PH + 3) & ~3, PWP = (PW + 3) & ~3;
+#pragma unroll
+    for (int y = 0; y < kFootCap; ++y)
+#pragma unroll
+        for (int x = 0; x < kFootCap; ++x) G[y][x] = 0.0f;
+#pragma unroll 1
+    for (int ph = 0; ph < PH; ++ph) {
+        float g[PW];
+#pragma unroll
+        for (int pw = 0; pw < PW; ++pw) g[pw] = loadg(ph, pw);
+        float t[kFootCap];
+#pragma unroll
+        for (int x = 0; x < kFootCap; ++x) {
+            const float4* w4 = reinterpret_cast<const float4*>(sWx + x * PWP);
+            float s = 0.0f;
+#pragma unroll
+            for (int q = 0; q < PWP / 4; ++q) {
+                const float4 w = w4[q];
+                if (4 * q + 0 < PW) s = fmaf(w.x, g[4 * q + 0], s);
+                if (4 * q + 1 < PW) s = fmaf(w.y, g[4 * q + 1], s);
+                if (4 * q + 2 < PW) s = fmaf(w.z, g[4 * q + 2], s);
+                if (4 * q + 3 < PW) s = fmaf(w.w, g[4 * q + 3], s);
+            }
+            t[x] = s;
+        }
+#pragma unroll
+        for (int y = 0; y < kFootCap; ++y) {
+            const float wy = sWy[y * PHP + ph];
+#pragma unroll
+            for (int x = 0; x < kFootCap; ++x) G[y][x] = fmaf(wy, t[x], G[y][x]);
+        }
+    }
+}
+
+// Tiles of a footprint the staged path cannot hold: every sample of every bin, lane = channel.
+template <int PH, int PW, typename T, bool GCL, bool ICL>
+__device__ __forceinline__ void bwd_tile_exact(const T* __restrict__ go, const float* __restrict__ rois, long long k, int c0,
+                                               int cn, float scale, int sr, int aligned, float* __restrict__ gi, int B,
+                                               int C, int H, int W, int lane) {
+    const Geom g = roi_geometry(rois + 5 * k, scale, sr, aligned, PH, PW);
+    if (g.b < 0 || g.b >= B || lane >= cn) return;
+    const int c = c0 + lane;
+    float* base = gi + (ICL ? (size_t)g.b * H * W * C + c : ((size_t)g.b * C + c) * H * W);
+    const size_t ps = ICL ? (size_t)C : 1;
+#pragma unroll 1
+    for (int bin = 0; bin < PH * PW; ++bin) {
+        const int ph = bin / PW, pw = bin - ph * PW;
+        const float gv = grad_at<T, GCL>(go, k, C, PH * PW, c, bin);
+        for (int iy = 0; iy < g.gh; ++iy) {
+            const Tap ty = make_tap(sample_pos(g.sh, ph, g.bh, iy, g.gh), H);
+            for (int ix = 0; ix < g.gw; ++ix)
+                bwd_sample(base, ps, W, ty, make_tap(sample_pos(g.sw, pw, g.bw, ix, g.gw), W), gv, g.count);
+        }
+    }
+}
+
+// One warp per (ROI, 32-channel tile).  MODE 0: tables built by the warp (small launches); 1: footprint and tables from
+// roi_prep_kernel; 2: as 1 but only the tiles roi_prep_kernel did not stage (the rest went through the TMA kernel).
+template <int PH, int PW, typename T, bool GCL, bool ICL, int MODE>
+__global__ void __launch_bounds__(kWarpsPerCta * 32)
+roi_align_bwd_tile_kernel(const T* __restrict__ go, const float* __restrict__ rois, long long K, float scale, int sr,
+                          int aligned, float* __restrict__ gi, int B, int C, int H, int W, int ctiles,
+                          const RoiPrep* __restrict__ prep, const float* __restrict__ prep_tabs) {
+    using L = TileSmem<PH, PW>;
+    __shared__ __align__(16) float sTabs[kWarpsPerCta][L::kTabFloats];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const long long wi = (long long)blockIdx.x * kWarpsPerCta + warp;
+    if (wi >= K * ctiles) return;
+    const long long k = wi / ctiles;
+    const int c0 = (int)(wi - k * ctiles) * 32, cn = min(32, C - c0);
+    float* sWy = sTabs[warp];
+    float* sWx = sWy + kFootCap * L::kPHP;
+    int b, ymin, xmin, FY, FX;
+    bool staged;
+    if (MODE == 0) {
+        const Geom g = roi_geometry(rois + 5 * k, scale, sr, aligned, PH, PW);
+        axis_footprint(g.sh, g.bh, PH, g.gh, H, &ymin, &FY);
+        axis_footprint(g.sw, g.bw, PW, g.gw, W, &xmin, &FX);
+        if (g.b < 0 || g.b >= B || FY == 0 || FX == 0) return;
+        b = g.b;
+        staged = FY <= kFootCap && FX <= kFootCap;
+        if (staged) build_tables<PH, PW>(g, __fdiv_rn(1.0f, g.count), H, W, ymin, xmin, FY, sWy, sWx, L::kTabFloats, lane);
+    } else {
+        const int4 h0 = reinterpret_cast<const int4*>(prep + k)[0], h1 = reinterpret_cast<const int4*>(prep + k)[1];
+        b = h0.x; ymin = h0.y; xmin = h0.z; FY = h0.w; FX = h1.x;
+        staged = h1.y != 0;
+        if (MODE == 2 && staged) return;
+        if (staged) {
+            if (FY == 0) return;
+            const float4* src = reinterpret_cast<const float4*>(prep_tabs + (size_t)k * L::kTabFloats);
+            for (int i = lane; i < L::kTabFloats / 4; i += 32) reinterpret_cast<float4*>(sWy)[i] = src[i];
+        }
+    }
+    if (!staged) {
+        bwd_tile_exact<PH, PW, T, GCL, ICL>(go, rois, k, c0, cn, scale, sr, aligned, gi, B, C, H, W, lane);
+        return;
+    }
+    __syncwarp();
+    const int c = c0 + (lane < cn ? lane : 0);
+    float G[kFootCap][kFootCap];
+    bwd_contract<PH, PW>(G, sWy, sWx, [&](int ph, int pw) {
+        return lane < cn ? grad_at<T, GCL>(go, k, C, PH * PW, c, ph * PW + pw) : 0.0f;
+    });
+    if (lane >= cn) return;
+    float* base = gi + (ICL ? (((size_t)b * H + ymin) * W + xmin) * C + c : (((size_t)b * C + c) * H + ymin) * W + xmin);
+    const size_t rs = ICL ? (size_t)W * C : (size_t)W, xs = ICL ? (size_t)C : 1;
+#pragma unroll
+    for (int y = 0; y < kFootCap; ++y)
+        if (y < FY) {
+#pragma unroll
+            for (int x = 0; x < kFootCap; ++x)
+                if (x < FX) red_add(base + y * rs + x * xs, G[y][x]);
+        }
+}
+
+template <bool GCL, typename T>
+__global__ void __launch_bounds__(256)
+roi_align_bwd_generic_kernel(const T* __restrict__ go, const float* __restrict__ rois, long long total, int PH, int PW,
+                             float scale, int sr, int aligned, float* __restrict__ gi, int ICL, int B, int C, int H, int W) {
+    for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
+         idx += (long long)gridDim.x * blockDim.x) {
+        // idx is the linear index of the grad_out element in its own layout ([K][C][PH][PW] or [K][PH][PW][C])
+        int pw, ph, c;
+        if (GCL) {
+            c = (int)(idx % C); pw = (int)((idx / C) % PW); ph = (int)((idx / ((long long)C * PW)) % PH);
+        } else {
+            pw = (int)(idx % PW); ph = (int)((idx / PW) % PH); c = (int)((idx / ((long long)PW * PH)) % C);
+        }
+        const long long k = idx / ((long long)PW * PH * C);
+        const Geom g = roi_geometry(rois + 5 * k, scale, sr, aligned, PH, PW);
+        if (g.b < 0 || g.b >= B) continue;
+        const float gv = to_f32(go[idx]);
+        float* base = gi + (ICL ? (size_t)g.b * H * W * C + c : ((size_t)g.b * C + c) * H * W);
+        const size_t ps = ICL ? (size_t)C : 1;
+        for (int iy = 0; iy < g.gh; ++iy) {
+            const Tap ty = make_tap(sample_pos(g.sh, ph, g.bh, iy, g.gh), H);
+            for (int ix = 0; ix < g.gw; ++ix)
+                bwd_sample(base, ps, W, ty, make_tap(sample_pos(g.sw, pw, g.bw, ix, g.gw), W), gv, g.count);
+        }
+    }
+}
+
+// Per-warp shared memory of the TMA kernel: two slots of (grad_out chunk, tables) -- the current tile and the next --
+// and one box buffer of up to 8 rows (a 5-row box and the 1 / 3-row box below it).
+template <int PH, int PW, typename T>
+struct BwdTmaSmem {
+    using L = TileSmem<PH, PW>;
+    static constexpr int kGBytes = (32 * PH * PW * (int)sizeof(T) + 15) & ~15;
+    static constexpr int kTabBytes = L::kTabFloats * 4;
+    static constexpr int kSlotBytes = (kGBytes + kTabBytes + 127) & ~127;
+    static constexpr int kOffBox = 2 * kSlotBytes, kOffBar = kOffBox + kFootCap * kTmaRowBytes;   // box: 128-byte aligned
+    static constexpr int kBytesPerWarp = (kOffBar + 16 + 127) & ~127;
+    static_assert(kTabBytes % 16 == 0, "bulk-copy alignment");
+};
+#ifndef B200_ROI_BWD_TMA_WARPS
+#define B200_ROI_BWD_TMA_WARPS 2
+#endif
+constexpr int kBwdTmaWarps = B200_ROI_BWD_TMA_WARPS;
+
+__device__ __forceinline__ void tma_reduce_add_4d(const CUtensorMap* tm, unsigned src, int x, int y, int c, int b) {
+    asm volatile("cp.reduce.async.bulk.tensor.4d.global.shared::cta.add.tile.bulk_group [%0, {%1, %2, %3, %4}], [%5];\n"
+                 ::"l"(tm), "r"(x), "r"(y), "r"(c), "r"(b), "r"(src) : "memory");
+}
+
+// Requests tile (k, c0)'s tables and, with an NCHW grad_out, its contiguous [cn][PH*PW] chunk on one mbarrier.
+template <int PH, int PW, typename T, bool GCL>
+__device__ __forceinline__ void bwd_tma_issue(const T* __restrict__ go, int C, unsigned k, int c0, const float* prep_tabs,
+                                              unsigned sslot, unsigned bar) {
+    using S = BwdTmaSmem<PH, PW, T>;
+    constexpr int NB = PH * PW;
+    const unsigned ku = (unsigned)bcast0((int)k), su = (unsigned)bcast0((int)sslot), baru = (unsigned)bcast0((int)bar);
+    const int cu = bcast0(c0), cn = min(32, C - cu);
+    const unsigned gbytes = GCL ? 0u : (unsigned)(cn * NB * (int)sizeof(T));
+    if (elect_one()) {
+        mbar_expect_tx(baru, (unsigned)S::kTabBytes + gbytes);
+        bulk_load(su + S::kGBytes, prep_tabs + (size_t)ku * S::L::kTabFloats, S::kTabBytes, baru);
+        if (!GCL) bulk_load(su, go + ((size_t)ku * C + cu) * NB, gbytes, baru);
+    }
+    __syncwarp();
+}
+
+// Large launches into a float32 NCHW grad_in (tma_applies).  Tiles are handed out as in roi_align_tma_kernel; tiles that
+// roi_prep_kernel did not stage are left to a later roi_align_bwd_tile_kernel<MODE 2> launch.
+template <int PH, int PW, typename T, bool GCL>
+__global__ void __launch_bounds__(kBwdTmaWarps * 32)
+roi_align_bwd_tma_kernel(const __grid_constant__ TmaMaps tmap, const T* __restrict__ go, long long K, int C, int ctiles,
+                         const RoiPrep* __restrict__ prep, const float* __restrict__ prep_tabs, int group_warps,
+                         int tiles_per_warp) {
+    using S = BwdTmaSmem<PH, PW, T>;
+    constexpr int NB = PH * PW, PHP = S::L::kPHP;
+    extern __shared__ __align__(128) unsigned char smem_bwd[];
+    const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
+    unsigned char* base = smem_bwd + (size_t)warp * S::kBytesPerWarp;
+    const unsigned sbase = (unsigned)__cvta_generic_to_shared(base);
+    const unsigned sbar = sbase + S::kOffBar, sbox = sbase + S::kOffBox;
+    const unsigned gw = blockIdx.x * kBwdTmaWarps + warp, grp = gw / (unsigned)group_warps;
+    const unsigned stride = (unsigned)group_warps, window = stride * (unsigned)tiles_per_warp;
+    unsigned t = grp * window + (gw - grp * stride);
+    const unsigned total = (unsigned)min((long long)(grp + 1) * window, K * ctiles);
+    if (t >= total) return;
+    if (lane == 0) {
+        mbar_init(sbar, 1);
+        mbar_init(sbar + 8, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+    }
+    __syncwarp();
+    auto wanted = [](int4 h0, int4 h1) { return h1.y != 0 && h0.w != 0; };     // staged and sampling something
+    unsigned ka = t / (unsigned)ctiles;
+    int ca = (int)(t - ka * (unsigned)ctiles) * 32;
+    int4 a0 = reinterpret_cast<const int4*>(prep + ka)[0], a1 = reinterpret_cast<const int4*>(prep + ka)[1];
+    if (wanted(a0, a1)) bwd_tma_issue<PH, PW, T, GCL>(go, C, ka, ca, prep_tabs, sbase, sbar);
+    int par = 0;
+    unsigned phase = 0;                // bit p = parity the next wait on mbarrier p expects
+    bool pending = false;              // a reduction may still be reading the box buffer
+    for (;;) {
+        const unsigned tn = t + stride;
+        const bool have_next = tn < total;
+        unsigned kn = 0;
+        int cnx = 0;
+        int4 n0 = make_int4(0, 0, 0, 0), n1 = n0;
+        if (have_next) {
+            kn = tn / (unsigned)ctiles;
+            cnx = (int)(tn - kn * (unsigned)ctiles) * 32;
+            n0 = reinterpret_cast<const int4*>(prep + kn)[0];
+            n1 = reinterpret_cast<const int4*>(prep + kn)[1];
+            // slot par ^ 1 was consumed by the previous tile (the warp converged after reading it)
+            if (wanted(n0, n1))
+                bwd_tma_issue<PH, PW, T, GCL>(go, C, kn, cnx, prep_tabs, sbase + (par ^ 1) * S::kSlotBytes, sbar + 8 * (par ^ 1));
+        }
+        if (wanted(a0, a1)) {
+            mbar_wait(sbar + 8 * par, (phase >> par) & 1u);
+            phase ^= 1u << par;
+            const unsigned char* slot = base + par * S::kSlotBytes;
+            const float* sWy = reinterpret_cast<const float*>(slot + S::kGBytes);
+            const T* sg = reinterpret_cast<const T*>(slot);
+            const int cn = min(32, C - ca);
+            const int c = ca + (lane < cn ? lane : 0);
+            float G[kFootCap][kFootCap];
+            bwd_contract<PH, PW>(G, sWy, sWy + kFootCap * PHP, [&](int ph, int pw) {
+                if (lane >= cn) return 0.0f;
+                return GCL ? grad_at<T, true>(go, ka, C, NB, c, ph * PW + pw) : to_f32(sg[lane * NB + ph * PW + pw]);
+            });
+            __syncwarp();              // this slot is free for the tile after next
+            if (pending && lane == 0) bulk_store_wait_read();
+            __syncwarp();
+            // G -> box buffer: rows 0-4 (or fewer) in the first box [32][r0][8], rows 5-7 in the second box [32][r1][8]
+            const int FY = a0.w, ymin = a0.y, xmin = a0.z, b = a0.x;
+            const int r0 = FY > kTmaRows ? kTmaRows : tma_box_rows(FY);
+            const int r1 = FY > kTmaRows ? tma_box_rows(FY - kTmaRows) : 0;
+            unsigned char* box0 = base + S::kOffBox + lane * (r0 * 32);
+            unsigned char* box1 = base + S::kOffBox + kTmaRows * kTmaRowBytes + lane * (r1 * 32);
+#pragma unroll
+            for (int y = 0; y < kFootCap; ++y) {
+                if (y < r0 || (y >= kTmaRows && y < kTmaRows + r1)) {
+                    float4* row = reinterpret_cast<float4*>(y < kTmaRows ? box0 + y * 32 : box1 + (y - kTmaRows) * 32);
+                    row[0] = make_float4(G[y][0], G[y][1], G[y][2], G[y][3]);
+                    row[1] = make_float4(G[y][4], G[y][5], G[y][6], G[y][7]);
+                }
+            }
+            asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");
+            __syncwarp();
+            if (lane == 0) {
+                tma_reduce_add_4d(&tmap.m[r0 >> 1], sbox, xmin, ymin, ca, b);
+                if (r1) tma_reduce_add_4d(&tmap.m[r1 >> 1], sbox + kTmaRows * kTmaRowBytes, xmin, ymin + kTmaRows, ca, b);
+                asm volatile("cp.async.bulk.commit_group;\n" ::: "memory");
+            }
+            pending = true;
+        }
+        if (!have_next) break;
+        t = tn; ka = kn; ca = cnx; a0 = n0; a1 = n1;
+        par ^= 1;
+    }
+    if (pending && lane == 0) asm volatile("cp.async.bulk.wait_group 0;\n" ::: "memory");
+    __syncwarp();
+}
+
+template <int PH, int PW, typename T, bool GCL, bool ICL, int MODE>
+int launch_bwd_tile(const T* go, const float* rois, long long K, float scale, int sr, int aligned, float* gi, int B, int C,
+                    int H, int W, int ctiles, const RoiPrep* prep, const float* tabs, cudaStream_t st) {
+    const long long blocks = (K * ctiles + kWarpsPerCta - 1) / kWarpsPerCta;
+    roi_align_bwd_tile_kernel<PH, PW, T, GCL, ICL, MODE><<<(unsigned)blocks, kWarpsPerCta * 32, 0, st>>>(
+        go, rois, K, scale, sr, aligned, gi, B, C, H, W, ctiles, prep, tabs);
+    return check_launch("roi_align_bwd_tile_kernel");
+}
+
+// Launches the TMA kernel when it applies; returns 1 when it does not.
+template <int PH, int PW, typename T, bool GCL>
+int launch_bwd_tma(const T* go, long long K, float* gi, int B, int C, int H, int W, int ctiles, const RoiPrep* prep,
+                   const float* tabs, long long tiles, cudaStream_t st) {
+    using S = BwdTmaSmem<PH, PW, T>;
+    if (reinterpret_cast<uintptr_t>(tabs) & 15) return 1;
+    EncodeTiledFn encode = encode_tiled_fn();
+    if (!encode) return 1;
+    TmaMaps tmap;
+    const cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)C, (cuuint64_t)B};
+    const cuuint64_t strides[3] = {(cuuint64_t)W * 4, (cuuint64_t)H * W * 4, (cuuint64_t)C * H * W * 4};
+    const cuuint32_t estr[4] = {1u, 1u, 1u, 1u};
+    for (int i = 0; i < 3; ++i) {                // boxes of 1, 3 and 5 rows, as launch_tma's
+        const cuuint32_t box[4] = {(cuuint32_t)kTmaCols, (cuuint32_t)(2 * i + 1), 32u, 1u};
+        const CUresult r = encode(&tmap.m[i], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, gi, dims, strides, box, estr,
+                                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
+                                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) return 1;
+    }
+    static int cache[kMaxDevices];               // per instantiation and device
+    auto kern = roi_align_bwd_tma_kernel<PH, PW, T, GCL>;
+    constexpr int smem_bytes = S::kBytesPerWarp * kBwdTmaWarps;
+    int resident = 0;
+    const int rc = resident_warps_of(kern, cache, kBwdTmaWarps, smem_bytes, &resident);
+    if (rc) return rc;
+    long long tpw = tiles / ((long long)resident * 4);            // at least four waves of warps, 2 .. 16 tiles each
+    tpw = tpw < 2 ? 2 : tpw > 16 ? 16 : tpw;
+    const long long window = (long long)resident * tpw;
+    const long long groups = (tiles + window - 1) / window;
+    const long long last = tiles - (groups - 1) * window;
+    const long long warps = (groups - 1) * resident + (last < resident ? last : resident);
+    kern<<<(unsigned)((warps + kBwdTmaWarps - 1) / kBwdTmaWarps), kBwdTmaWarps * 32, smem_bytes, st>>>(
+        tmap, go, K, C, ctiles, prep, tabs, resident, (int)tpw);
+    return check_launch("roi_align_bwd_tma_kernel");
+}
+
+template <int PH, int PW, typename T, bool GCL, bool ICL>
+int launch_bwd(const T* go, const float* rois, long long K, float scale, int sr, int aligned, float* gi, int B, int C, int H,
+               int W, cudaStream_t st) {
+    using L = TileSmem<PH, PW>;
+    const int ctiles = (C + 31) / 32;
+    const long long tiles = K * ctiles;
+    if ((tiles + kWarpsPerCta - 1) / kWarpsPerCta > 0x7fffffffLL || tiles >= (1LL << 32))
+        return fail(B200_EINVAL, "roi_align_backward: too many ROI tiles (%lld)", tiles);
+    if (tiles < kPrepMinTiles || ctiles < 4)
+        return launch_bwd_tile<PH, PW, T, GCL, ICL, 0>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, ctiles, nullptr,
+                                                       nullptr, st);
+    cudaMemPool_t pool = nullptr;
+    int rc = scratch_pool(&pool);
+    if (rc) return rc;
+    char* ws = nullptr;                          // stream-ordered scratch: K records + K tables
+    const size_t rec = (size_t)K * sizeof(RoiPrep), tab = (size_t)K * L::kTabFloats * sizeof(float);
+    B200_CUDA(cudaMallocFromPoolAsync(reinterpret_cast<void**>(&ws), rec + tab, pool, st));
+    RoiPrep* prep = reinterpret_cast<RoiPrep*>(ws);
+    float* tabs = reinterpret_cast<float*>(ws + rec);
+    // the TMA kernel also bulk-loads NCHW grad_out chunks [cn][PH*PW]: each must be whole 16-byte units at a 16-byte boundary
+    const bool use_tma = !ICL && tma_applies(gi, C, H, W) &&
+                         (GCL || (((size_t)C * PH * PW * sizeof(T)) & 15) == 0 && (reinterpret_cast<uintptr_t>(go) & 15) == 0);
+    roi_prep_kernel<PH, PW><<<(unsigned)((K + 3) / 4), 128, 0, st>>>(rois, K, B, H, W, scale, sr, aligned, prep, tabs,
+                                                                     use_tma ? kTmaXAlign : 1);
+    rc = check_launch("roi_prep_kernel");
+    if (rc == B200_OK) {
+        rc = 1;
+        if constexpr (!ICL) {
+            if (use_tma) {
+                rc = launch_bwd_tma<PH, PW, T, GCL>(go, K, gi, B, C, H, W, ctiles, prep, tabs, tiles, st);
+                if (rc == B200_OK)
+                    rc = launch_bwd_tile<PH, PW, T, GCL, ICL, 2>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, ctiles,
+                                                                 prep, tabs, st);
+            }
+        }
+        // no TMA kernel (channels-last grad_in, alignment): the tile kernel with the prep records
+        if (rc == 1)
+            rc = launch_bwd_tile<PH, PW, T, GCL, ICL, 1>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, ctiles, prep,
+                                                         tabs, st);
+    }
+    B200_CUDA(cudaFreeAsync(ws, st));
+    return rc;
+}
+
+template <typename T>
+int roi_align_bwd_dispatch(const T* go, int go_layout, const float* rois, int64_t K, int PH, int PW, float scale, int sr,
+                           int aligned, float* gi, int layout, int B, int C, int H, int W, void* stream) {
+    B200_REQUIRE(layout == B200_LAYOUT_NCHW || layout == B200_LAYOUT_NHWC, "roi_align_backward: bad layout %d", layout);
+    B200_REQUIRE(go_layout == B200_LAYOUT_NCHW || go_layout == B200_LAYOUT_NHWC,
+                 "roi_align_backward: bad grad_out layout %d", go_layout);
+    B200_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, "roi_align_backward: bad input shape [%d,%d,%d,%d]", B, C, H, W);
+    B200_REQUIRE(PH > 0 && PW > 0, "roi_align_backward: bad output size (%d,%d)", PH, PW);
+    B200_REQUIRE(K >= 0, "roi_align_backward: negative ROI count");
+    if (K == 0) return B200_OK;
+    B200_REQUIRE(go && rois && gi, "roi_align_backward: null pointer");
+    cudaStream_t st = as_stream(stream);
+    const bool gcl = go_layout == B200_LAYOUT_NHWC, icl = layout == B200_LAYOUT_NHWC;
+#define B200_BWD(ph, pw)                                                                                                 \
+    if (PH == ph && PW == pw) {                                                                                          \
+        if (gcl)                                                                                                         \
+            return icl ? launch_bwd<ph, pw, T, true, true>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, st)          \
+                       : launch_bwd<ph, pw, T, true, false>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, st);        \
+        return icl ? launch_bwd<ph, pw, T, false, true>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, st)             \
+                   : launch_bwd<ph, pw, T, false, false>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, st);           \
+    }
+    B200_BWD(10, 10)
+    B200_BWD(7, 7)
+#undef B200_BWD
+    const long long total = (long long)K * C * PH * PW;
+    const long long want = (total + 255) / 256;
+    const unsigned blocks = (unsigned)(want < (long long)kSMs * 32 ? want : (long long)kSMs * 32);
+    if (gcl)
+        roi_align_bwd_generic_kernel<true, T><<<blocks, 256, 0, st>>>(go, rois, total, PH, PW, scale, sr, aligned, gi,
+                                                                      icl, B, C, H, W);
+    else
+        roi_align_bwd_generic_kernel<false, T><<<blocks, 256, 0, st>>>(go, rois, total, PH, PW, scale, sr, aligned, gi,
+                                                                       icl, B, C, H, W);
+    return check_launch("roi_align_bwd_generic_kernel");
+}
+
 // ---- box preparation in front of ROI Align (tracking.py:209-213, trainingCard.py:38-69) as one launch -----------
 // torch.minimum / maximum / clamp propagate NaN; fminf / fmaxf do not.
 __device__ __forceinline__ float t_min(float a, float b) { return (a != a || b != b) ? __int_as_float(0x7fc00000) : fminf(a, b); }
@@ -1571,6 +2012,18 @@ extern "C" int b200_roi_align_fwd_ex(const void* feat, int dtype, int layout, in
                                                 spatial_scale, sampling_ratio, aligned, static_cast<__half*>(out),
                                                 out_layout, stream);
     return b200::fail(B200_EINVAL, "roi_align: bad dtype %d", dtype);
+}
+
+extern "C" int b200_roi_align_bwd_ex(const void* grad_out, int dtype, int grad_out_layout, const float* rois, int64_t K,
+                                     int PH, int PW, float spatial_scale, int sampling_ratio, int aligned, float* grad_in,
+                                     int layout, int B, int C, int H, int W, void* stream) {
+    if (dtype == B200_DTYPE_F32)
+        return b200::roi_align_bwd_dispatch<float>(static_cast<const float*>(grad_out), grad_out_layout, rois, K, PH, PW,
+                                                   spatial_scale, sampling_ratio, aligned, grad_in, layout, B, C, H, W, stream);
+    if (dtype == B200_DTYPE_F16)
+        return b200::roi_align_bwd_dispatch<__half>(static_cast<const __half*>(grad_out), grad_out_layout, rois, K, PH, PW,
+                                                    spatial_scale, sampling_ratio, aligned, grad_in, layout, B, C, H, W, stream);
+    return b200::fail(B200_EINVAL, "roi_align_backward: bad dtype %d", dtype);
 }
 
 B200_SPAN_GETTER(b200_debug_spans_roi)

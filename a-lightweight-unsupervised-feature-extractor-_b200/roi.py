@@ -5,10 +5,12 @@
                                    (= tracking_win.py:239-267, infer.py:143-170).
 * ``preprocess_roi``             - PreProcess._preprocess_roi, trainingCard.py:24-79.
 """
+import warnings
 from typing import Sequence, Tuple, Union
 
 import numpy as np
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import _lib
 
@@ -36,7 +38,7 @@ def _boxes_to_rois(boxes, device):
 def roi_align(input: torch.Tensor, boxes: Union[torch.Tensor, Sequence[torch.Tensor]],
               output_size: Union[int, Tuple[int, int]], spatial_scale: float = 1.0,
               sampling_ratio: int = -1, aligned: bool = False, *, out_channels_last: bool = False) -> torch.Tensor:
-    """Drop-in for ``torchvision.ops.roi_align`` (forward only).
+    """Drop-in for ``torchvision.ops.roi_align``, differentiable with respect to ``input`` like torchvision's op.
 
     ``input`` may be contiguous NCHW or ``torch.channels_last``; both are read in place.  float32 maps are
     the parity contract; float16 maps (what the reference's live CUDA path feeds, tracking.py:177-178) are
@@ -47,12 +49,25 @@ def roi_align(input: torch.Tensor, boxes: Union[torch.Tensor, Sequence[torch.Ten
     ``out_channels_last=True`` (extension; SURVEY 8f-3, the ROI -> encoder hand-off) returns the same values as a
     ``[K, C, PH, PW]`` tensor in ``torch.channels_last`` memory format, which a channels_last encoder
     (model/utils/encoder/card.py:24-41) consumes without a copy and which the kernel writes as whole cache lines.
+
+    When grad mode is on and ``input`` requires grad, the result carries a ``grad_fn`` whose backward is
+    ``roi_align_backward``: ``input.grad`` gets ``input``'s dtype and memory format, the boxes get no gradient.  The
+    gradient is summed with atomic additions in an order that is not fixed (not bit-reproducible, and refused under
+    ``torch.use_deterministic_algorithms(True)`` as torchvision's CUDA backward is); a float16 map's gradient is
+    accumulated in float32 and rounded once.  Otherwise exactly the forward kernel runs, as before.
     """
     _lib.require_cuda(input, "input")
     if input.dim() != 4:
         raise ValueError("input must be [B, C, H, W]")
     if input.dtype not in (torch.float32, torch.float16):
         raise TypeError("roi_align: float32 or float16 feature maps only (got %s)" % input.dtype)
+    if torch.is_grad_enabled() and input.requires_grad:
+        rois = _boxes_to_rois(boxes, input.device)
+        return _RoIAlign.apply(input, rois, _pair(output_size), spatial_scale, sampling_ratio, aligned, out_channels_last)
+    return _roi_align_forward(input, boxes, output_size, spatial_scale, sampling_ratio, aligned, out_channels_last)
+
+
+def _roi_align_forward(input, boxes, output_size, spatial_scale, sampling_ratio, aligned, out_channels_last):
     B, C, H, W = input.shape
     if input.is_contiguous():
         layout = _lib.LAYOUT_NCHW
@@ -73,6 +88,85 @@ def roi_align(input: torch.Tensor, boxes: Union[torch.Tensor, Sequence[torch.Ten
             _lib.LAYOUT_NHWC if out_channels_last else _lib.LAYOUT_NCHW, _lib.stream_ptr(input.device))
     _lib.check(rc)
     return out
+
+
+def _memory_format_of(t):
+    if not t.is_contiguous() and t.is_contiguous(memory_format=torch.channels_last):
+        return torch.channels_last
+    return torch.contiguous_format
+
+
+class _RoIAlign(torch.autograd.Function):
+    """roi_align with a gradient for the map.  Saves the float32 rois and the input's metadata, not the input."""
+
+    @staticmethod
+    def forward(ctx, input, rois, output_size, spatial_scale, sampling_ratio, aligned, out_channels_last):
+        ctx.save_for_backward(rois)
+        ctx.input_shape = tuple(input.shape)
+        ctx.dtype, ctx.memory_format = input.dtype, _memory_format_of(input)
+        ctx.args = (output_size, spatial_scale, sampling_ratio, aligned)
+        return _roi_align_forward(input, rois, output_size, spatial_scale, sampling_ratio, aligned, out_channels_last)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_output):
+        if torch.are_deterministic_algorithms_enabled():
+            msg = ("roi_align_backward does not have a deterministic implementation, but you set "
+                   "'torch.use_deterministic_algorithms(True)'.")
+            if not torch.is_deterministic_algorithms_warn_only_enabled():
+                raise RuntimeError(msg)
+            warnings.warn(msg)
+        rois, = ctx.saved_tensors
+        grad_input = roi_align_backward(grad_output, rois, ctx.input_shape, *ctx.args, dtype=ctx.dtype,
+                                        memory_format=ctx.memory_format)
+        return grad_input, None, None, None, None, None, None
+
+
+def roi_align_backward(grad_output: torch.Tensor, boxes: Union[torch.Tensor, Sequence[torch.Tensor]],
+                       input_shape: Sequence[int], output_size: Union[int, Tuple[int, int]], spatial_scale: float = 1.0,
+                       sampling_ratio: int = -1, aligned: bool = False, *, dtype: torch.dtype = torch.float32,
+                       memory_format: torch.memory_format = torch.contiguous_format) -> torch.Tensor:
+    """Gradient of ``roi_align`` with respect to its input (torchvision's ``_roi_align_backward``).
+
+    ``grad_output``: ``[K, C, PH, PW]`` float32 or float16 on a CUDA device, read in place when it is contiguous or
+    ``torch.channels_last`` (otherwise copied); ``boxes`` and the scalar arguments exactly as given to ``roi_align``;
+    ``input_shape``: ``(B, C, H, W)`` of the map.  Returns a new ``[B, C, H, W]`` tensor of ``dtype`` (float32 or
+    float16) in ``memory_format`` (contiguous or channels_last): zeros plus the contributions of every ROI whose batch
+    index is in ``[0, B)``.  The contributions are accumulated in float32 with atomic additions in an order that is not
+    fixed, then rounded to ``dtype`` once; torchvision's float16 backward accumulates in float16 and differs.
+    """
+    _lib.require_cuda(grad_output, "grad_output")
+    B, C, H, W = (int(v) for v in input_shape)
+    PH, PW = _pair(output_size)
+    if grad_output.dim() != 4 or tuple(grad_output.shape[1:]) != (C, PH, PW):
+        raise ValueError("grad_output must be [K, %d, %d, %d] (got %s)" % (C, PH, PW, tuple(grad_output.shape)))
+    if grad_output.dtype not in (torch.float32, torch.float16):
+        raise TypeError("roi_align_backward: float32 or float16 grad_output only (got %s)" % grad_output.dtype)
+    if dtype not in (torch.float32, torch.float16):
+        raise TypeError("roi_align_backward: float32 or float16 result only (got %s)" % dtype)
+    if memory_format not in (torch.contiguous_format, torch.channels_last):
+        raise ValueError("roi_align_backward: memory_format must be contiguous_format or channels_last")
+    rois = _boxes_to_rois(boxes, grad_output.device)
+    K = rois.size(0)
+    if grad_output.size(0) != K:
+        raise ValueError("grad_output has %d ROIs, boxes %d" % (grad_output.size(0), K))
+    if grad_output.is_contiguous():
+        go_layout = _lib.LAYOUT_NCHW
+    elif grad_output.is_contiguous(memory_format=torch.channels_last):
+        go_layout = _lib.LAYOUT_NHWC
+    else:
+        grad_output, go_layout = grad_output.contiguous(), _lib.LAYOUT_NCHW
+    grad_input = torch.empty((B, C, H, W), dtype=torch.float32, device=grad_output.device,
+                             memory_format=memory_format).zero_()
+    layout = _lib.LAYOUT_NHWC if memory_format == torch.channels_last else _lib.LAYOUT_NCHW
+    gdtype = _lib.DTYPE_F32 if grad_output.dtype == torch.float32 else _lib.DTYPE_F16
+    with torch.cuda.device(grad_output.device):
+        rc = _lib.lib().b200_roi_align_bwd_ex(
+            _lib.ptr(grad_output), gdtype, go_layout, _lib.ptr(rois), K, PH, PW, float(spatial_scale),
+            int(sampling_ratio), int(bool(aligned)), _lib.ptr(grad_input), layout, B, C, H, W,
+            _lib.stream_ptr(grad_output.device))
+    _lib.check(rc)
+    return grad_input if dtype == torch.float32 else grad_input.to(dtype)
 
 
 def _prep_boxes(boxes: torch.Tensor, device, mode: int, batch_index=None, img_hw=(0, 0), map_hw=(0, 0),

@@ -73,6 +73,17 @@ int b200_roi_align_fwd_ex(const void* feat, int dtype, int layout, int B, int C,
                           const float* rois, int64_t K, int PH, int PW, float spatial_scale,
                           int sampling_ratio, int aligned, void* out, int out_layout, void* stream);
 
+/* Backward of b200_roi_align_fwd_ex (torchvision's _roi_align_backward): ADDS d(loss)/d(feat) into grad_in.
+ * grad_out: [K,C,PH,PW] of element type `dtype` (B200_DTYPE_F32 / _F16), stored NCHW or NHWC (grad_out_layout);
+ * rois, spatial_scale, sampling_ratio, aligned: exactly as given to the forward call;
+ * grad_in: float32 [B,C,H,W] in `layout` (NCHW or NHWC), caller-zeroed or holding a gradient to add to.
+ * ROIs with a batch index outside [0,B) contribute nothing.  The summation order is not deterministic.
+ * Half grad_out is read as stored and all arithmetic and accumulation is float32 (torchvision's half backward
+ * accumulates with half atomics, so its result differs). */
+int b200_roi_align_bwd_ex(const void* grad_out, int dtype, int grad_out_layout, const float* rois, int64_t K,
+                          int PH, int PW, float spatial_scale, int sampling_ratio, int aligned,
+                          float* grad_in, int layout, int B, int C, int H, int W, void* stream);
+
 /* Box preparation in front of ROI Align, one launch: boxes [n, box_stride >= 4] float32 (first four columns xyxy; the
  * detector's NMS rows [x1,y1,x2,y2,conf,cls] qualify, yoloDetects2.py:135-157) -> rois [n,5] = (batch, x1, y1, x2, y2).
  * batch_index: int32 [n] or NULL (= 0, what both reference wrappers use: one map per call).

@@ -1,7 +1,13 @@
 """Micro-benchmark of the ROI Align kernel at the BASELINE.json shapes (CUDA events, L2 flushed
-or inputs larger than L2).  Prints one JSON line per case.  Not the headline bench (bench.py)."""
+or inputs larger than L2).  Prints one JSON line per case.  Not the headline bench (bench.py).
+
+--backward times the gradient instead: the public roi_align_backward call (zero fill of grad_in included; "nhwc" =
+channels-last grad_in) against torchvision's CUDA _roi_align_backward (which zero-fills too).  Algorithmic bytes are
+the forward's formula -- each upstream gradient read once, each input gradient written once -- a floor that the zero
+fill and the read-modify-write of the additions in L2 put out of reach; the fraction is reported against it anyway."""
 import json
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -31,7 +37,8 @@ def timed(fn, iters, flush):
     return t[len(t) // 2] * 1e-3, t[0] * 1e-3
 
 
-def case(name, Bm, Hf, Wf, H_in, W_in, per_map, ps=(10, 10), nhwc=False, tv=False, iters=20, half=False, out_cl=False):
+def case(name, Bm, Hf, Wf, H_in, W_in, per_map, ps=(10, 10), nhwc=False, tv=False, iters=20, half=False, out_cl=False,
+         backward=False):
     rng = np.random.default_rng(0)
     boxes = np.concatenate([synth.random_boxes(rng, per_map, H_in, W_in) for _ in range(Bm)])
     rois = np.concatenate([np.repeat(np.arange(Bm), per_map)[:, None].astype(np.float64), boxes], 1).astype(np.float32)
@@ -45,7 +52,18 @@ def case(name, Bm, Hf, Wf, H_in, W_in, per_map, ps=(10, 10), nhwc=False, tv=Fals
     es = 2 if half else 4
     alg = K * 512 * ps[0] * ps[1] * es + Bm * 512 * Hf * Wf * es + K * 20
     flush = torch.empty(256 * 1024 * 1024 // 4, device="cuda") if alg < 512e6 else None
-    if tv:
+    if backward:
+        alg = K * 512 * ps[0] * ps[1] * es + Bm * 512 * Hf * Wf * 4 + K * 20      # grad_in is float32
+        flush = torch.empty(256 * 1024 * 1024 // 4, device="cuda") if alg < 512e6 else None
+        g = torch.randn((K, 512) + tuple(ps), device="cuda", dtype=torch.float16 if half else torch.float32)
+        if tv:
+            import torchvision  # noqa: F401  (registers torch.ops.torchvision)
+            fn = lambda: torch.ops.torchvision._roi_align_backward(g, r, Hf / float(H_in), ps[0], ps[1], Bm, 512, Hf, Wf, 2,
+                                                                   True)
+        else:
+            mf = torch.channels_last if nhwc else torch.contiguous_format
+            fn = lambda: roi.roi_align_backward(g, r, (Bm, 512, Hf, Wf), ps, Hf / float(H_in), 2, True, memory_format=mf)
+    elif tv:
         import torchvision
         fn = lambda: torchvision.ops.roi_align(feat, r, ps, Hf / float(H_in), 2, True)
     else:
@@ -53,7 +71,8 @@ def case(name, Bm, Hf, Wf, H_in, W_in, per_map, ps=(10, 10), nhwc=False, tv=Fals
     for _ in range(3):
         fn()
     med, best = timed(fn, iters, flush)
-    print(json.dumps({"case": name, "impl": "torchvision" if tv else "b200", "layout": ("nhwc" if nhwc else "nchw") + ("->nhwc" if out_cl else ""), "dtype": "f16" if half else "f32",
+    print(json.dumps({**({"pass": "backward"} if backward else {}), "case": name,
+                      "impl": "torchvision" if tv else "b200", "layout": ("nhwc" if nhwc else "nchw") + ("->nhwc" if out_cl else ""), "dtype": "f16" if half else "f32",
                       "K": K, "out": list(ps), "alg_MB": round(alg / 1e6, 2), "us_median": round(med * 1e6, 2),
                       "us_best": round(best * 1e6, 2), "GBps_median": round(alg / med / 1e9, 1),
                       "frac_of_measured_peak": round(alg / med / 1e9 / PEAK, 3)}), flush=True)
@@ -65,6 +84,22 @@ if __name__ == "__main__":
     which = args or ["c1", "c2", "c3", "c5"]
     impls = (False,) if "--b200" in flags else (False, True)
     layouts = (False,) if "--nchw" in flags else (True,) if "--nhwc" in flags else (False, True)
+    if "--backward" in flags:
+        which = args or ["c1", "c2", "c3", "c5", "g64"]
+        print(subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                             capture_output=True, text=True).stdout.strip(), flush=True)
+        shapes = {"c1": ("c1", 1, 20, 20, 640, 640, 8, 20), "c2": ("c2", 1, 40, 40, 1280, 1280, 64, 20),
+                  "c3": ("c3", 256, 40, 40, 1280, 1280, 16, 10), "c5": ("c5x64", 64, 34, 60, 1088, 1920, 128, 10),
+                  "g64": ("g64", 64, 40, 40, 1280, 1280, 64, 10)}
+        for w in which:
+            name, Bm, Hf, Wf, H_in, W_in, per_map, iters = shapes[w]
+            for tv in impls:        # torchvision's gradient is NCHW only
+                for nhwc in (layouts if not tv else (False,)):
+                    case(name, Bm, Hf, Wf, H_in, W_in, per_map, nhwc=nhwc, tv=tv, iters=iters, backward=True)
+            if "--half" in flags:
+                for nhwc in layouts:
+                    case(name, Bm, Hf, Wf, H_in, W_in, per_map, nhwc=nhwc, iters=iters, half=True, backward=True)
+        sys.exit(0)
     for tv in impls:
         for nhwc in layouts:
             if "c1" in which:
