@@ -64,6 +64,7 @@ SIGNATURES = {
     "b200_tracker_result_stride": (_I, [_P]),
     "b200_tracker_live_counts": (_I, [_P, _P, _P, _P]),
     "b200_tracker_step": (_I, [_P, _P, _P, _P, _P, _P, _P, _P]),
+    "b200_tracker_step_packed": (_I, [_P, _L, _P, _I, _P, _I, _I, _P, _I, _P, _P, _P, _P, _P, _P]),
     "b200_tracker_step_host": (_I, [_P, _P, _P, _P, _P, _P, _P, _P]),
     "b200_tracker_step_host_async": (_I, [_P, _P, _P, _P, _P, _P, ctypes.POINTER(ctypes.c_int64), _P]),
     "b200_tracker_step_pinned_async": (_I, [_P, _P, _P, _P, _P, _P, ctypes.POINTER(ctypes.c_int64), _P]),

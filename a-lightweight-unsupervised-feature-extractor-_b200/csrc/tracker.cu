@@ -18,6 +18,8 @@
 
 #include <new>
 
+#include <cuda_fp16.h>
+
 #include "assoc_cost.cuh"
 #include "kalman.cuh"
 #include "lsap.cuh"
@@ -1223,6 +1225,79 @@ __global__ void reset_kernel(Dev d) {
     }
 }
 
+// ---- b200_tracker_step_packed: detections in the detector's / encoder's layout -> the step's padded per-stream layout ----
+// pack_kernel (one CTA per stream) selects the stream's detections in input order with block_compact, widens them into the
+// handle's packed-input block, writes n_det and sets every track_of_det entry to -1; b200_tracker_step runs on that block;
+// finish_kernel (one CTA per stream) reports overflowing streams and writes the track id of every match of the result table
+// to the input row of its (stream, det_idx).  Each pack CTA walks all K stream indices (one ballot round per 1 024 rows), so
+// the CTA is as wide as possible: the walk is a chain of dependent rounds, not a bandwidth cost.
+struct Packed {
+    int S, MD, K, box_stride, conf_stride, det_half, emb_half;
+    const void *boxes, *confs, *embs;
+    const int *stream_index, *active;
+    // the handle's packed-input block
+    int* n_det;
+    double *p_boxes, *p_confs;
+    float* p_embs;
+    int* inv;                         // [S, MD] input row k of det_idx j of stream s
+    int* over;                        // [S] 1 = the stream had more than MD detections and was not stepped
+    int* track_of_det;                // [K] or null
+};
+
+constexpr int kPackThreads = 1024;
+
+__device__ __forceinline__ int stream_of(const Packed& p, int k) { return p.stream_index ? p.stream_index[k] : 0; }
+
+__device__ __forceinline__ double widen(const void* base, size_t i, int half) {      // exact: f16 -> f32 -> f64
+    return half ? (double)__half2float(static_cast<const __half*>(base)[i]) : (double)static_cast<const float*>(base)[i];
+}
+
+__global__ void __launch_bounds__(kPackThreads) pack_kernel(Packed p) {
+    __shared__ int scratch[kPackThreads / 32];
+    const int s = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const size_t db = (size_t)s * p.MD;
+    if (p.track_of_det)                              // finish_kernel overwrites the matched entries after the step
+        for (int k = s * kPackThreads + threadIdx.x; k < p.K; k += p.S * kPackThreads) p.track_of_det[k] = -1;
+    const bool on = p.active == nullptr || p.active[s] != 0;
+    int n = 0;
+    if (on)
+        n = block_compact(p.K, [&](int k) { return stream_of(p, k) == s; }, [&](int j, int k) {
+            if (j >= p.MD) return;
+            p.inv[db + j] = k;
+#pragma unroll
+            for (int c = 0; c < 4; ++c) p.p_boxes[(db + j) * 4 + c] = widen(p.boxes, (size_t)k * p.box_stride + c, p.det_half);
+            p.p_confs[db + j] = widen(p.confs, (size_t)k * p.conf_stride, p.det_half);
+        }, scratch);
+    const bool over = n > p.MD;
+    if (threadIdx.x == 0) { p.n_det[s] = on && !over ? n : -1; p.over[s] = over ? 1 : 0; }
+    if (!on || over) return;                         // uniform across the CTA
+    __syncthreads();                                 // inv[] of this stream is complete
+    for (int j = warp; j < n; j += kPackThreads / 32) {   // one warp per embedding row, four elements per lane
+        const size_t k = (size_t)p.inv[db + j];
+        float4 v;
+        if (p.emb_half) {
+            const uint2 raw = reinterpret_cast<const uint2*>(static_cast<const __half*>(p.embs) + k * cost::kD)[lane];
+            const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&raw.x));
+            const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&raw.y));
+            v = make_float4(a.x, a.y, b.x, b.y);
+        } else {
+            v = reinterpret_cast<const float4*>(static_cast<const float*>(p.embs) + k * cost::kD)[lane];
+        }
+        reinterpret_cast<float4*>(p.p_embs + (db + j) * cost::kD)[lane] = v;
+    }
+}
+
+__global__ void __launch_bounds__(kThreads) finish_kernel(Packed p, int* result, int res_stride) {
+    const int s = blockIdx.x;
+    int* res = result + (size_t)s * res_stride;
+    if (threadIdx.x == 0 && p.over[s]) res[R_STATUS] = B200_ECAPACITY;
+    if (p.track_of_det == nullptr) return;
+    // the matched rows (an idle, overflowing or failed stream has none in its row); every other entry is pack_kernel's -1
+    const int nm = res[R_NMATCH];
+    const int* m = res + R_HDR;
+    for (int i = threadIdx.x; i < nm; i += blockDim.x) p.track_of_det[p.inv[(size_t)s * p.MD + m[2 * i + 1]]] = m[2 * i];
+}
+
 }  // namespace trk
 }  // namespace b200
 
@@ -1245,6 +1320,10 @@ struct b200_tracker {
     long long next_ticket = 0;
     int* in_ndet = nullptr; int* in_frame = nullptr; double* in_boxes = nullptr; double* in_confs = nullptr;
     float* in_embs = nullptr; int* dev_result = nullptr;
+    // input block of b200_tracker_step_packed, separate from in_* and the ring so that a packed step queued on one stream
+    // never races with a host step or a step-by-step operation queued on another
+    int* pk_ndet = nullptr; double* pk_boxes = nullptr; double* pk_confs = nullptr; float* pk_embs = nullptr;
+    int* pk_inv = nullptr; int* pk_over = nullptr;
     int ctl_threads = 256;              // CTA width of the per-stream control kernels (assign)
 #ifndef B200_TRK_BEGIN_THREADS
 #define B200_TRK_BEGIN_THREADS 256
@@ -1315,6 +1394,8 @@ extern "C" int b200_tracker_create(b200_tracker** out, int n_streams, int max_tr
     TAKE(in_embs, float, S * MD * 128);
     const size_t in_end = c.off;
     TAKE(result, int, S * (size_t)d.res_stride);
+    TAKE(pk_ndet, int, S); TAKE(pk_boxes, double, S * MD * 4); TAKE(pk_confs, double, S * MD);
+    TAKE(pk_embs, float, S * MD * 128); TAKE(pk_inv, int, S * MD); TAKE(pk_over, int, S);
 #undef TAKE
     cudaError_t e = cudaMalloc(&t->arena, c.off);
     if (e != cudaSuccess) {
@@ -1340,6 +1421,12 @@ extern "C" int b200_tracker_create(b200_tracker** out, int n_streams, int max_tr
     t->in_confs = reinterpret_cast<double*>(base + o_in_confs);
     t->in_embs = reinterpret_cast<float*>(base + o_in_embs);
     t->dev_result = reinterpret_cast<int*>(base + o_result);
+    t->pk_ndet = reinterpret_cast<int*>(base + o_pk_ndet);
+    t->pk_boxes = reinterpret_cast<double*>(base + o_pk_boxes);
+    t->pk_confs = reinterpret_cast<double*>(base + o_pk_confs);
+    t->pk_embs = reinterpret_cast<float*>(base + o_pk_embs);
+    t->pk_inv = reinterpret_cast<int*>(base + o_pk_inv);
+    t->pk_over = reinterpret_cast<int*>(base + o_pk_over);
     t->in_bytes = in_end - o_in;
     t->res_bytes = S * (size_t)d.res_stride * sizeof(int);
     t->slot_bytes = ((t->in_bytes + 255) & ~(size_t)255) + ((t->res_bytes + 255) & ~(size_t)255);
@@ -1550,6 +1637,40 @@ extern "C" int b200_tracker_step(b200_tracker* t, const int32_t* n_det, const do
     launch(trk::update_kernel, dim3(t->upd_grid), dim3(trk::kUpdWarps * 32), 0, d);
     if ((rc = check_launch("trk update_kernel"))) return rc;
     return B200_OK;
+}
+
+extern "C" int b200_tracker_step_packed(b200_tracker* t, int64_t K, const void* boxes, int box_stride, const void* confs,
+                                        int conf_stride, int det_dtype, const void* embs, int emb_dtype,
+                                        const int32_t* stream_index, const int32_t* active, const int32_t* frame_id,
+                                        int32_t* result, int32_t* track_of_det, void* stream) {
+    B200_REQUIRE(t, "tracker_step_packed: null handle");
+    B200_REQUIRE(K >= 0 && K <= 0x7fffffff, "tracker_step_packed: K = %lld out of range", (long long)K);
+    B200_REQUIRE(box_stride >= 4, "tracker_step_packed: box_stride %d < 4", box_stride);
+    B200_REQUIRE(conf_stride >= 1, "tracker_step_packed: conf_stride %d < 1", conf_stride);
+    B200_REQUIRE(det_dtype == B200_DTYPE_F32 || det_dtype == B200_DTYPE_F16, "tracker_step_packed: unknown det_dtype %d", det_dtype);
+    B200_REQUIRE(emb_dtype == B200_DTYPE_F32 || emb_dtype == B200_DTYPE_F16, "tracker_step_packed: unknown emb_dtype %d", emb_dtype);
+    B200_REQUIRE(frame_id, "tracker_step_packed: null frame_id");
+    B200_REQUIRE(result, "tracker_step_packed: null result");
+    if (K > 0) {
+        B200_REQUIRE(boxes, "tracker_step_packed: null boxes");
+        B200_REQUIRE(confs, "tracker_step_packed: null confs");
+        B200_REQUIRE(embs, "tracker_step_packed: null embs");
+        B200_REQUIRE(reinterpret_cast<uintptr_t>(embs) % (emb_dtype == B200_DTYPE_F32 ? 16 : 8) == 0,
+                     "tracker_step_packed: embs must be %d-byte aligned", emb_dtype == B200_DTYPE_F32 ? 16 : 8);
+    }
+    cudaStream_t st = as_stream(stream);
+    trk::Packed p;
+    p.S = t->d.S; p.MD = t->d.MD; p.K = (int)K; p.box_stride = box_stride; p.conf_stride = conf_stride;
+    p.det_half = det_dtype == B200_DTYPE_F16; p.emb_half = emb_dtype == B200_DTYPE_F16;
+    p.boxes = boxes; p.confs = confs; p.embs = embs; p.stream_index = stream_index; p.active = active;
+    p.n_det = t->pk_ndet; p.p_boxes = t->pk_boxes; p.p_confs = t->pk_confs; p.p_embs = t->pk_embs;
+    p.inv = t->pk_inv; p.over = t->pk_over; p.track_of_det = track_of_det;
+    trk::pack_kernel<<<p.S, trk::kPackThreads, 0, st>>>(p);
+    int rc = check_launch("trk pack_kernel");
+    if (rc) return rc;
+    if ((rc = b200_tracker_step(t, t->pk_ndet, t->pk_boxes, t->pk_confs, t->pk_embs, frame_id, result, stream))) return rc;
+    trk::finish_kernel<<<p.S, trk::kThreads, 0, st>>>(p, result, t->d.res_stride);
+    return check_launch("trk finish_kernel");
 }
 
 // Host-buffer step, asynchronous: stages the detections in the next slot of a pinned ring, uploads them into the slot's

@@ -63,6 +63,8 @@ class MultiStreamTracker:
     Detections are passed as dense host arrays padded to ``max_dets`` per stream:
     ``n_det[S]`` (-1 = stream idle, 0 = empty frame), ``boxes[S,max_dets,4]`` float64 xyxy,
     ``confs[S,max_dets]`` float64, ``embs[S,max_dets,128]`` float32, ``frame_ids[S]``.
+    ``step_device`` takes the same layout on the device; ``step_detections`` takes the detector's rows and the
+    encoder's embeddings on the device as they come, with a stream index per row.
     """
 
     def __init__(self, n_streams: int, conf: Optional[Dict[str, Any]] = None, max_tracks: int = 256,
@@ -242,6 +244,70 @@ class MultiStreamTracker:
         self._n_live_stale = True
         return result
 
+    def step_detections(self, boxes: torch.Tensor, confs: torch.Tensor, embs: torch.Tensor, frame_ids: torch.Tensor,
+                        stream_index: Optional[torch.Tensor] = None, *, active: Optional[torch.Tensor] = None,
+                        result: Optional[torch.Tensor] = None, track_of_det: Optional[torch.Tensor] = None):
+        """``step_device`` fed with what a detector and an encoder produce, without the host round trip the reference
+        makes (tracking.py:315-324) and without padding on the caller's side (b200_tracker_step_packed).
+
+        ``boxes`` [K, >=4] (first four columns x1, y1, x2, y2) and ``confs`` [K]: float32 or float16, both the same;
+        views such as ``dets[:, :4]`` and ``dets[:, 4]`` of the detector's [K, 6] rows are read in place.  ``embs``
+        [K, 128] contiguous, float32 or float16.  ``stream_index`` int32 [K] (e.g. ROI Align's batch index), or None:
+        every detection belongs to stream 0; a detection with an index outside [0, S) is ignored.  ``active`` int32 [S]
+        or None: 0 leaves that stream idle this step (state untouched, like n_det = -1).  ``frame_ids`` int32 [S].
+        All on the device.  Half values are widened exactly, so they give what ``update()`` gives for the same values.
+
+        The j-th detection of stream s in input order is det_idx j of that stream in the result table.  Returns
+        ``(result, track_of_det)``: the table ``step_device`` returns, and int32 [K] holding the track id each detection
+        was matched to in this step, -1 otherwise.  Asynchronous on the current stream, no read-back, capturable in a
+        CUDA graph.  A stream with more than ``max_dets`` detections is not stepped and gets ECAPACITY in its R_STATUS
+        column (K <= max_dets rules that out); otherwise capacity is ``step_device``'s precondition."""
+        if boxes.dim() != 2 or boxes.shape[1] < 4:
+            raise ValueError("step_detections: boxes must be [K, >=4]")
+        K = boxes.shape[0]
+        if confs.dim() != 1 or confs.shape[0] != K or embs.dim() != 2 or embs.shape != (K, 128):
+            raise ValueError("step_detections: confs must be [K] and embs [K, 128] for K = %d boxes" % K)
+        if frame_ids.shape != (self.S,):
+            raise ValueError("step_detections: frame_ids must be [%d]" % self.S)
+        dtypes = {torch.float32: _lib.DTYPE_F32, torch.float16: _lib.DTYPE_F16}
+        if boxes.dtype not in dtypes or confs.dtype != boxes.dtype or embs.dtype not in dtypes:
+            raise TypeError("step_detections: boxes / confs must be float32 or float16 (the same), embs float32 or float16")
+        if (K > 0 and (boxes.stride(1) != 1 or not embs.is_contiguous())) or (K > 1 and boxes.stride(0) < 4):
+            raise TypeError("step_detections: boxes need unit column stride and embs must be contiguous")
+        ints = [(frame_ids, "frame_ids")]
+        if stream_index is not None:
+            if stream_index.shape != (K,):
+                raise ValueError("step_detections: stream_index must be [K]")
+            ints.append((stream_index, "stream_index"))
+        if active is not None:
+            if active.shape != (self.S,):
+                raise ValueError("step_detections: active must be [%d]" % self.S)
+            ints.append((active, "active"))
+        if result is None:
+            result = torch.empty((self.S, self.stride), dtype=torch.int32, device=self.device)
+        elif result.shape != (self.S, self.stride):
+            raise ValueError("step_detections: result must be [%d, %d]" % (self.S, self.stride))
+        if track_of_det is None:
+            track_of_det = torch.empty((K,), dtype=torch.int32, device=self.device)
+        elif track_of_det.shape != (K,):
+            raise ValueError("step_detections: track_of_det must be [K]")
+        ints += [(result, "result"), (track_of_det, "track_of_det")]
+        for t, name in [(boxes, "boxes"), (confs, "confs"), (embs, "embs")] + ints:
+            _lib.require_cuda(t, name)
+        for t, name in ints:
+            if t.dtype != torch.int32 or not t.is_contiguous():
+                raise TypeError("step_detections: %s must be a contiguous int32 tensor" % name)
+        box_stride = boxes.stride(0) if K > 1 else 4
+        conf_stride = confs.stride(0) if K > 1 else 1
+        with torch.cuda.device(self.device):
+            rc = _lib.lib().b200_tracker_step_packed(
+                self._h, K, _lib.ptr(boxes), box_stride, _lib.ptr(confs), conf_stride, dtypes[boxes.dtype], _lib.ptr(embs),
+                dtypes[embs.dtype], _lib.ptr(stream_index), _lib.ptr(active), _lib.ptr(frame_ids), _lib.ptr(result),
+                _lib.ptr(track_of_det), _lib.stream_ptr(self.device))
+        _lib.check(rc)
+        self._n_live_stale = True
+        return result, track_of_det
+
     def decode(self, row: np.ndarray):
         """Result-table row -> (matches_tid, unmatched_track_ids, unmatched_dets) as Tracking.update returns."""
         MD, MT = self.max_dets, self.max_tracks
@@ -381,6 +447,7 @@ class Tracking:
         self._confs = np.zeros((1, MD), np.float64)
         self._embs = np.zeros((1, MD, 128), np.float32)
         self._snap = None
+        self._frame_dev = None                       # update_tensors: the frame id on the device
 
     @property
     def device(self):
@@ -432,6 +499,40 @@ class Tracking:
         res = self._ms.step([N], self._boxes, self._confs, self._embs, [frame_id])
         self._snap = None
         return self._ms.decode(res[0])
+
+    def update_tensors(self, boxes: torch.Tensor, confs: torch.Tensor, embs: torch.Tensor, frame_id: int):
+        """``update`` fed from the detector's and the encoder's device tensors instead of host lists
+        (tracking.py:315-324 copies them to the host): ``boxes`` [N, >=4] (e.g. ``dets[:, :4]`` of the detector's
+        [N, 6] rows, read in place), ``confs`` [N] (e.g. ``dets[:, 4]``), both float32 or both float16, ``embs`` [N, 128]
+        float32 or float16.  Returns what ``update`` returns for the same values, with the same errors and the same
+        automatic growth; float16 inputs give exactly what ``update`` gives for their values, because both widen them
+        exactly.  The inputs stay on the device; the only device -> host copy is the small result table."""
+        ms = self._ms
+        if boxes.dim() != 2 or confs.dim() != 1 or embs.dim() != 2 or not (boxes.shape[0] == confs.shape[0] == embs.shape[0]):
+            raise ValueError("Length mismatch: embs/bboxes/confs must have same length")
+        if embs.shape[1] != 128:
+            raise ValueError(f"det_embs must be 128D, got sizes [{embs.shape[1]}]")
+        N = boxes.shape[0]
+        if N > ms.max_dets:
+            if not ms.auto_grow:
+                raise ValueError("%d detections exceed max_dets=%d" % (N, ms.max_dets))
+            ms.grow(max_dets=max(N, 2 * ms.max_dets))
+        bound = int(ms.n_live_now()[0]) + N
+        if bound > ms.max_tracks:                    # the reference is unbounded: migrate to a larger handle
+            if not ms.auto_grow:
+                raise _lib.B200Error("tracker capacity: live tracks + detections could exceed max_tracks=%d; "
+                                     "construct the tracker with a larger max_tracks" % ms.max_tracks)
+            ms.grow(max_tracks=max(bound, 2 * ms.max_tracks))
+        if self._frame_dev is None:
+            self._frame_dev = torch.empty((1,), dtype=torch.int32, device=self.device)
+        self._frame_dev.fill_(int(frame_id))
+        table, _ = ms.step_detections(boxes, confs, embs, self._frame_dev)
+        res = table.cpu().numpy()
+        self._snap = None
+        h = StepHandle(ms, -1, np.zeros(ms.S, np.int64))
+        h._finish(res)                               # live count from the table: the handle's count is current again
+        ms._n_live_stale = False
+        return ms.decode(h.result()[0])
 
     # -- the reference's methods one by one (mainTracking.py:340-448), on the device state -----------
     def _dets(self, det_embs, det_boxes, det_confs):

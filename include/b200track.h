@@ -187,6 +187,30 @@ int  b200_tracker_live_counts(b200_tracker* t, int32_t* n_live_host, int32_t* ne
 int  b200_tracker_step(b200_tracker* t, const int32_t* n_det, const double* boxes,
                        const double* confs, const float* embs, const int32_t* frame_id,
                        int32_t* result, void* stream);
+/* The same step from detections in the detector's / encoder's own layout (device pointers), K detections in any
+ * stream order -- no host round trip and no padding on the caller's side (tracking.py:315-324 rebuilds host lists):
+ *   boxes  : K rows at a stride of box_stride (>= 4) elements, first four = x1,y1,x2,y2 (the detector's NMS rows
+ *            [x1,y1,x2,y2,conf,cls] qualify, yoloDetects2.py:135-157)
+ *   confs  : K values at a stride of conf_stride (>= 1) elements (for NMS rows: boxes + 4, same stride)
+ *   det_dtype (B200_DTYPE_F32 / _F16) applies to boxes and confs; both are widened to float64 exactly
+ *   embs   : [K,128] contiguous rows of emb_dtype (F32 / F16; 16- / 8-byte aligned), widened to float32 exactly
+ *   stream_index : int32 [K] (e.g. the ROI batch index) or NULL = every detection belongs to stream 0;
+ *                  detections with an index outside [0,S) are ignored
+ *   active : int32 [S] or NULL = every stream steps (a stream with no detection gets an empty frame, :467-471);
+ *            0 = stream idle this step (state untouched, like n_det = -1 in b200_tracker_step)
+ *   frame_id : int32 [S];  result : int32 [S, stride], exactly what b200_tracker_step writes
+ *   track_of_det : int32 [K] or NULL: the track id detection k was matched to in this step, -1 otherwise (unmatched,
+ *                  ignored, or in a stream that did not step; births are not reported, as :607-610 does not)
+ * A stream's detections are taken in input order: the j-th detection of stream s in the input is det_idx j of that
+ * stream in the result table, as if the caller had compacted them in order and called b200_tracker_step.
+ * A stream with more than max_dets detections is not stepped (state untouched) and gets B200_ECAPACITY in its status
+ * column; the other streams step normally.  Same capacity precondition as b200_tracker_step.
+ * Three launches (pack, step, finish) through an input block owned by the handle: no allocation and no
+ * synchronisation, so the call can be captured in a CUDA graph. */
+int  b200_tracker_step_packed(b200_tracker* t, int64_t K, const void* boxes, int box_stride,
+                              const void* confs, int conf_stride, int det_dtype, const void* embs, int emb_dtype,
+                              const int32_t* stream_index, const int32_t* active, const int32_t* frame_id,
+                              int32_t* result, int32_t* track_of_det, void* stream);
 /* Same step with HOST buffers (pinned or pageable): copies inputs up, runs the step, copies
  * the result table back into result_host and synchronises the stream. */
 int  b200_tracker_step_host(b200_tracker* t, const int32_t* n_det_host, const double* boxes_host,
