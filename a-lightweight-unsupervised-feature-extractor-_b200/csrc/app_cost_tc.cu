@@ -524,18 +524,9 @@ int app_cost_tc(const float* bank, const int32_t* bank_len, const float* fallbac
             // it is off by default and kept as a tested option.
             int cl = 1;
             if (const char* e = getenv("B200TRACK_TC_CLUSTER")) cl = (atoi(e) == 2 && m_tiles % 2 == 0) ? 2 : 1;
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3((unsigned)m_tiles);
-            cfg.blockDim = dim3(kWalkThreads);
-            cfg.dynamicSmemBytes = kWalkSmem;
-            cfg.stream = st;
-            cudaLaunchAttribute attr[1];
-            attr[0].id = cudaLaunchAttributeClusterDimension;
-            attr[0].val.clusterDim.x = cl; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-            cfg.attrs = attr;
-            cfg.numAttrs = 1;
-            (void)cudaLaunchKernelEx(&cfg, app_tc_walk_kernel, (const unsigned char*)imgA, (const unsigned char*)imgB, bank_len,
-                                     (int)(fallback != nullptr), M, N, T, topk, use_topk_mean, C_app, ldc, n_tiles);
+            launch_ex(app_tc_walk_kernel, dim3((unsigned)m_tiles), dim3(kWalkThreads), kWalkSmem, st, false, cl,
+                      (const unsigned char*)imgA, (const unsigned char*)imgB, bank_len, (int)(fallback != nullptr), M, N, T, topk,
+                      use_topk_mean, C_app, ldc, n_tiles);
             rc = check_launch("app_tc_walk_kernel");
         } else {
             app_tc_kernel<<<dim3(n_tiles, m_tiles), 128, kTcSmem, st>>>(imgA, imgB, bank_len, fallback != nullptr, M, N, T, topk,

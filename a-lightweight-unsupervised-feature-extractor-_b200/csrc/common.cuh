@@ -23,6 +23,29 @@ inline int check_launch(const char* what) {
     return B200_OK;
 }
 
+// Launches kern with programmatic stream serialisation when pdl is set, and as clusters of cluster_x CTAs when
+// cluster_x > 0 (a cluster attribute of size 1 is still an attribute: the launch is not the same as one without).
+// Errors surface in check_launch().
+template <typename Kern, typename... Args>
+inline void launch_ex(Kern kern, dim3 grid, dim3 block, size_t smem, cudaStream_t stream, bool pdl, int cluster_x,
+                      Args... args) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+    cudaLaunchAttribute attr[2];
+    unsigned n = 0;
+    if (pdl) {
+        attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        attr[n++].val.programmaticStreamSerializationAllowed = 1;
+    }
+    if (cluster_x > 0) {
+        attr[n].id = cudaLaunchAttributeClusterDimension;
+        attr[n++].val.clusterDim = {(unsigned)cluster_x, 1, 1};
+    }
+    cfg.attrs = attr;
+    cfg.numAttrs = n;
+    (void)cudaLaunchKernelEx(&cfg, kern, args...);
+}
+
 #define B200_CUDA(expr)                                                                  \
     do {                                                                                 \
         cudaError_t _e = (expr);                                                         \

@@ -1280,25 +1280,12 @@ EncodeTiledFn encode_tiled_fn() {
     return reinterpret_cast<EncodeTiledFn>(fn);
 }
 
-// Launch of a tile kernel that follows roi_prep_kernel in the stream.  dependent = as its programmatic dependent: it becomes
-// resident while the prep kernel still runs and waits for it with griddepcontrol.wait before it reads a record (-1.8 us per
-// launch).  Measured A/B on the overlapped 64-stream step (profiles/r02_roi_pdl_ab.txt): channels-last 221.0 -> 220.4 us, but
-// NCHW 235.4 -> 238.9 us -- the early-resident TMA CTAs take the SM slots that the association chain's first kernel, released
-// by the same event a few microseconds later, would otherwise get first -- so the TMA kernel stays an ordinary launch.
-template <typename Kern, typename... Args>
-void launch_after_prep(bool dependent, Kern kern, unsigned grid, unsigned block, size_t smem, cudaStream_t st, Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(block);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = dependent ? 1 : 0;
-    (void)cudaLaunchKernelEx(&cfg, kern, args...);      // errors surface in check_launch()
-}
+// The tile kernels that follow roi_prep_kernel in the stream are launched as its programmatic dependents (launch_ex with
+// pdl): they become resident while the prep kernel still runs and wait for it with griddepcontrol.wait before they read a
+// record (-1.8 us per launch).  Measured A/B on the overlapped 64-stream step (profiles/r02_roi_pdl_ab.txt): channels-last
+// 221.0 -> 220.4 us, but NCHW 235.4 -> 238.9 us -- the early-resident TMA CTAs take the SM slots that the association
+// chain's first kernel, released by the same event a few microseconds later, would otherwise get first -- so the TMA
+// kernel stays an ordinary launch.
 
 // Launches the TMA-staged kernel when it applies: NCHW map whose rows are a multiple of 16 bytes (the tensor map's
 // stride rule), 16-byte aligned base, dimensions inside the descriptor's limits.  Returns 1 when it does not.
@@ -1353,8 +1340,8 @@ int launch_tma(const T* feat, int B, int C, int H, int W, const float* rois, lon
     const long long groups = (tiles + window - 1) / window;
     const long long last = tiles - (groups - 1) * window;
     const long long warps = (groups - 1) * resident + (last < resident ? last : resident);
-    launch_after_prep(false, kern, (unsigned)((warps + kTmaWarps - 1) / kTmaWarps), kTmaWarps * 32, (size_t)smem_bytes, st, tmap, feat, B, C,
-                      H, W, rois, K, scale, sr, aligned, out, ctiles, prep, tabs, resident, (int)tpw);
+    launch_ex(kern, dim3((unsigned)((warps + kTmaWarps - 1) / kTmaWarps)), dim3(kTmaWarps * 32), (size_t)smem_bytes, st, false, 0,
+              tmap, feat, B, C, H, W, rois, K, scale, sr, aligned, out, ctiles, prep, tabs, resident, (int)tpw);
     return check_launch("roi_align_tma_kernel");
 }
 
@@ -1385,8 +1372,9 @@ int launch_pipe(const T* feat, int B, int C, int H, int W, const float* rois, lo
         const long long groups = (tiles + window - 1) / window;
         const long long last = tiles - (groups - 1) * window;                 // tiles in the last window
         const long long warps = (groups - 1) * resident_warps + (last < resident_warps ? last : resident_warps);
-        launch_after_prep(true, kern, (unsigned)((warps + kPipeWarps - 1) / kPipeWarps), kPipeWarps * 32, (size_t)P::kBytesPerCta, st, feat,
-                          B, C, H, W, rois, K, scale, sr, aligned, out, ctiles, prep, tabs, resident_warps, (int)kPipeTilesPerWarp);
+        launch_ex(kern, dim3((unsigned)((warps + kPipeWarps - 1) / kPipeWarps)), dim3(kPipeWarps * 32), (size_t)P::kBytesPerCta, st,
+                  true, 0, feat, B, C, H, W, rois, K, scale, sr, aligned, out, ctiles, prep, tabs, resident_warps,
+                  (int)kPipeTilesPerWarp);
         return check_launch("roi_align_pipe_kernel");
     } else {
         return 1;
@@ -1441,9 +1429,9 @@ int launch_tile(const T* feat, int B, int C, int H, int W, const float* rois, lo
                 const long long groups = (warps + window - 1) / window;
                 const long long last = warps - (groups - 1) * window;
                 const long long nw = (groups - 1) * resident_warps + (last < resident_warps ? last : resident_warps);
-                launch_after_prep(true, multi, (unsigned)((nw + kWarpsPerCta - 1) / kWarpsPerCta), kWarpsPerCta * 32, (size_t)L::kBytesPerCta,
-                                  st, feat, B, C, H, W, rois, K, scale, sr, aligned, out, ctiles, prep, tabs, resident_warps,
-                                  (int)B200_ROI_MULTI_TILES);
+                launch_ex(multi, dim3((unsigned)((nw + kWarpsPerCta - 1) / kWarpsPerCta)), dim3(kWarpsPerCta * 32),
+                          (size_t)L::kBytesPerCta, st, true, 0, feat, B, C, H, W, rois, K, scale, sr, aligned, out, ctiles, prep,
+                          tabs, resident_warps, (int)B200_ROI_MULTI_TILES);
                 rc = check_launch("roi_align_multi_kernel");
             }
         }

@@ -71,7 +71,7 @@ struct Dev {
     double* gate_SI;
     int* row_fc;                     // stage 1, written by the cost kernel: column of each row's unique minimum (-1: none, -2: NaN / -inf in the row)
     float* row_fv;                   //          that minimum
-    int *rows_main, *rows_reid, *cnt, *ud1, *det_used, *m_row, *m_det, *m_app, *tmp;
+    int *rows_main, *rows_reid, *cnt, *ud1, *det_used, *m_row, *m_det, *tmp;
     int* born;                       // [S, MD] detection index of each birth of the step, in order
     int2 *work1, *work2;             // (stream, row * 64 + detection tile) items of the two cost launches
     int* wcount;                     // [3] items queued for this step: cost1, cost2, updates
@@ -155,6 +155,47 @@ __device__ inline void purge(const Dev& d, int s, int nl, int* scratch) {
     __syncthreads();
 }
 
+// The header of a stream's row of the result table.
+__device__ __forceinline__ void put_result_header(int* res, int nmatch, int nut, int nud, int nlive, int next, int status,
+                                                  int m1, int m2) {
+    res[R_NMATCH] = nmatch; res[R_NUT] = nut; res[R_NUD] = nud; res[R_NLIVE] = nlive;
+    res[R_NEXT] = next; res[R_STATUS] = status; res[R_M1] = m1; res[R_M2] = m2;
+}
+
+// Start of a stream's step in the first kernel of every schedule: an idle stream (n < 0) and an empty frame (n == 0) are
+// the whole step.  Returns true when stream s is done for this step.  All threads of the CTA call; only the CTA with
+// `writer` set touches the stream's state and result row.
+__device__ __forceinline__ bool step_prologue(const Dev& d, int s, int n, int nl, bool writer, int* scratch) {
+    const int* hdr = d.hdr + s * kHdr;
+    int* cnt = d.cnt + s * kHdr;
+    int* res = d.result + (size_t)s * d.res_stride;
+    if (n < 0) {                                   // stream idle this step
+        if (writer && threadIdx.x == 0) {
+            cnt[C_MODE] = MODE_SKIP;
+            put_result_header(res, 0, 0, 0, nl, hdr[H_NEXT], 0, 0, 0);
+        }
+        return true;
+    }
+    if (n > 0) return false;
+    if (!writer) return true;
+    // :467-471 -- every track missed, NO predict
+    const size_t sb = (size_t)s * d.MT;
+    const int* order = d.order + sb;
+    int* ut = res_ut(d, res);
+    for (int p = threadIdx.x; p < nl; p += blockDim.x) {
+        const size_t slot = sb + order[p];
+        d.miss[slot] += 1;
+        ut[p] = d.tid[slot];
+    }
+    __syncthreads();
+    purge(d, s, nl, scratch);
+    if (threadIdx.x == 0) {
+        cnt[C_MODE] = MODE_EMPTY;
+        put_result_header(res, 0, nl, 0, hdr[H_NLIVE], hdr[H_NEXT], 0, 0, 0);
+    }
+    return true;
+}
+
 // Queues one work item per (row, 64-detection tile) of this stream for the persistent cost kernel.
 __device__ inline void enqueue_cost_work(int2* work, int* counter, int s, int M, int N, int* scratch) {
     const int tiles = (N + cost::kTileN - 1) / cost::kTileN, total = M * tiles;
@@ -214,11 +255,9 @@ __global__ void __launch_bounds__(kThreads) begin_kernel(Dev d) {
     Span span((d.frame_id[0] & 7) * 6 + 0);
     __shared__ int scratch[kThreads / 32];
     const int s = blockIdx.x, tid = threadIdx.x;
-    int* hdr = d.hdr + s * kHdr;
     int* cnt = d.cnt + s * kHdr;
-    int* res = d.result + (size_t)s * d.res_stride;
-    const size_t sb = (size_t)s * d.MT, db = (size_t)s * d.MD;
-    const int n = d.n_det[s], nl = hdr[H_NLIVE];
+    const size_t sb = (size_t)s * d.MT;
+    const int n = d.n_det[s], nl = d.hdr[s * kHdr + H_NLIVE];
     int* order = d.order + sb;
     if (blockIdx.y == 1) {                         // second CTA of the stream: detection prep only
         if (n <= 0) return;
@@ -226,32 +265,7 @@ __global__ void __launch_bounds__(kThreads) begin_kernel(Dev d) {
         return;
     }
     if (s == 0 && tid == 0) d.wcount[2] = 0;       // last step's update_kernel is done; nothing queued yet
-    if (n < 0) {                                   // stream idle this step
-        if (tid == 0) {
-            cnt[C_MODE] = MODE_SKIP;
-            res[R_NMATCH] = res[R_NUT] = res[R_NUD] = res[R_STATUS] = res[R_M1] = res[R_M2] = 0;
-            res[R_NLIVE] = nl;
-            res[R_NEXT] = hdr[H_NEXT];
-        }
-        return;
-    }
-    if (n == 0) {                                  // :467-471 -- every track missed, NO predict
-        int* ut = res_ut(d, res);
-        for (int p = tid; p < nl; p += blockDim.x) {
-            const size_t slot = sb + order[p];
-            d.miss[slot] += 1;
-            ut[p] = d.tid[slot];
-        }
-        __syncthreads();
-        purge(d, s, nl, scratch);
-        if (tid == 0) {
-            cnt[C_MODE] = MODE_EMPTY;
-            res[R_NMATCH] = 0; res[R_NUT] = nl; res[R_NUD] = 0; res[R_STATUS] = 0; res[R_M1] = res[R_M2] = 0;
-            res[R_NLIVE] = hdr[H_NLIVE];
-            res[R_NEXT] = hdr[H_NEXT];
-        }
-        return;
-    }
+    if (step_prologue(d, s, n, nl, true, scratch)) return;
     // ---- predict_all (:340-345) + per-track inputs of the stage-1 cost (by slot): predicted box and
     // confidence as float32, inverse innovation covariance for the gate -------------------------------
     for (int p = tid; p < nl; p += blockDim.x) predict_slot(d, sb + order[p]);
@@ -809,11 +823,7 @@ __device__ inline bool assign_body(const Dev& d, int s, unsigned char* smem_raw,
     if (STAGE == 2 && cnt[C_MODE] == MODE_FAILED) {
         // Stage 1 hit a NaN / infeasible matrix: the reference raises inside hungarian_assign (hung.py:28) before
         // any mark_missed / update_matched / birth / purge, so the stream's state stays "predict only".
-        if (tid == 0) {
-            res[R_NMATCH] = res[R_NUT] = res[R_NUD] = 0;
-            res[R_NLIVE] = hdr[H_NLIVE]; res[R_NEXT] = hdr[H_NEXT]; res[R_STATUS] = cnt[C_STATUS];
-            res[R_M1] = cnt[C_M1]; res[R_M2] = cnt[C_M2];
-        }
+        if (tid == 0) put_result_header(res, 0, 0, 0, hdr[H_NLIVE], hdr[H_NEXT], cnt[C_STATUS], cnt[C_M1], cnt[C_M2]);
         return true;
     }
     if (cnt[C_MODE] != MODE_NORMAL) return true;
@@ -900,11 +910,8 @@ __device__ inline bool assign_body(const Dev& d, int s, unsigned char* smem_raw,
 
     if (failed) {
         // The ReID-stage assignment raised (:560): stage 1's updates and misses stand, no births, no purge.
-        if (tid == 0) {
-            res[R_NMATCH] = match0; res[R_NUT] = ut0; res[R_NUD] = 0;
-            res[R_NLIVE] = hdr[H_NLIVE]; res[R_NEXT] = hdr[H_NEXT]; res[R_STATUS] = cnt[C_STATUS];
-            res[R_M1] = cnt[C_M1]; res[R_M2] = cnt[C_M2];
-        }
+        if (tid == 0)
+            put_result_header(res, match0, ut0, 0, hdr[H_NLIVE], hdr[H_NEXT], cnt[C_STATUS], cnt[C_M1], cnt[C_M2]);
         return true;
     }
     // ---- stage 2 tail: leftover dets, births (:362-373), purge (:357-360), result table ------------
@@ -917,16 +924,9 @@ __device__ inline bool assign_body(const Dev& d, int s, unsigned char* smem_raw,
     const int nl = hdr[H_NLIVE];
     const int nb = spawn_tracks(d, s, born, want);
     purge(d, s, nl + nb, scratch);
-    if (tid == 0) {
-        res[R_NMATCH] = match0 + n_match;
-        res[R_NUT] = ut0 + n_ut;
-        res[R_NUD] = n_left;
-        res[R_NLIVE] = hdr[H_NLIVE];
-        res[R_NEXT] = hdr[H_NEXT];
-        res[R_STATUS] = cnt[C_STATUS];
-        res[R_M1] = cnt[C_M1];
-        res[R_M2] = cnt[C_M2];
-    }
+    if (tid == 0)
+        put_result_header(res, match0 + n_match, ut0 + n_ut, n_left, hdr[H_NLIVE], hdr[H_NEXT], cnt[C_STATUS], cnt[C_M1],
+                          cnt[C_M2]);
     return true;
 }
 
@@ -959,40 +959,12 @@ __global__ void __launch_bounds__(kFrontWarps * 32, 2) front_kernel(Dev d) {
     __shared__ int scratch[kThreads / 32];
     const int s = blockIdx.y, g = blockIdx.x, G = gridDim.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     TRK_GSTAMP(0);
-    int* hdr = d.hdr + s * kHdr;
     int* cnt = d.cnt + s * kHdr;
-    int* res = d.result + (size_t)s * d.res_stride;
     const size_t sb = (size_t)s * d.MT;
-    const int n = d.n_det[s], nl = hdr[H_NLIVE];
+    const int n = d.n_det[s], nl = d.hdr[s * kHdr + H_NLIVE];
     const int* order = d.order + sb;
     if (s == 0 && g == 0 && tid == 0) d.wcount[2] = 0;     // three-launch chain: last step's update_kernel is done
-    if (n < 0) {                                   // stream idle this step
-        if (g == 0 && tid == 0) {
-            cnt[C_MODE] = MODE_SKIP;
-            res[R_NMATCH] = res[R_NUT] = res[R_NUD] = res[R_STATUS] = res[R_M1] = res[R_M2] = 0;
-            res[R_NLIVE] = nl;
-            res[R_NEXT] = hdr[H_NEXT];
-        }
-        return;
-    }
-    if (n == 0) {                                  // :467-471 -- every track missed, NO predict
-        if (g != 0) return;
-        int* ut = res_ut(d, res);
-        for (int p = tid; p < nl; p += blockDim.x) {
-            const size_t slot = sb + order[p];
-            d.miss[slot] += 1;
-            ut[p] = d.tid[slot];
-        }
-        __syncthreads();
-        purge(d, s, nl, scratch);
-        if (tid == 0) {
-            cnt[C_MODE] = MODE_EMPTY;
-            res[R_NMATCH] = 0; res[R_NUT] = nl; res[R_NUD] = 0; res[R_STATUS] = 0; res[R_M1] = res[R_M2] = 0;
-            res[R_NLIVE] = hdr[H_NLIVE];
-            res[R_NEXT] = hdr[H_NEXT];
-        }
-        return;
-    }
+    if (step_prologue(d, s, n, nl, g == 0, scratch)) return;
     // ---- rows_main / rows_reid in ascending track-id order (:478-487), in every CTA of the stream ----
     int* rm = s_rows;
     int* rr = s_rows + d.MT;
@@ -1298,6 +1270,54 @@ __global__ void __launch_bounds__(kThreads) finish_kernel(Packed p, int* result,
     for (int i = threadIdx.x; i < nm; i += blockDim.x) p.track_of_det[p.inv[(size_t)s * p.MD + m[2 * i + 1]]] = m[2 * i];
 }
 
+// ---- host-side buffer layouts ----------------------------------------------------------------------------------------
+// Lays buffers out one after another at 256-byte aligned offsets from `base`.  With base = nullptr it only measures: the
+// fields receive offsets and `off` ends as the size of the layout.
+struct Carver {
+    char* base = nullptr;
+    size_t off = 0;
+    static size_t aligned(size_t n) { return (n + 255) & ~(size_t)255; }
+    template <typename T> void take(T*& field, size_t n) {
+        off = aligned(off);
+        field = reinterpret_cast<T*>(reinterpret_cast<uintptr_t>(base) + off);
+        off += n * sizeof(T);
+    }
+};
+
+// One step's inputs in the padded per-stream layout b200_tracker_step reads.
+struct StepInputs {
+    int* n_det;
+    int* frame;
+    double* boxes;
+    double* confs;
+    float* embs;
+};
+
+// The inputs of S streams of MD detections as one contiguous range, so that a host step uploads them with a single copy.
+inline void take_inputs(Carver& c, StepInputs& in, size_t S, size_t MD) {
+    c.take(in.n_det, S);
+    c.take(in.frame, S);
+    c.take(in.boxes, S * MD * 4);
+    c.take(in.confs, S * MD);
+    c.take(in.embs, S * MD * 128);
+}
+
+// One slot of the host-step ring, pinned or device (the two sides share the layout): the step's inputs, then its result
+// table.
+struct Slot {
+    StepInputs in;
+    size_t in_bytes;                  // the inputs: one range from the slot's base
+    int* result;
+    size_t bytes;                     // the whole slot
+    Slot(void* base, const Dev& d) {
+        Carver c{static_cast<char*>(base)};
+        take_inputs(c, in, d.S, d.MD);
+        in_bytes = c.off;
+        c.take(result, (size_t)d.S * d.res_stride);
+        bytes = Carver::aligned(c.off);
+    }
+};
+
 }  // namespace trk
 }  // namespace b200
 
@@ -1307,8 +1327,8 @@ struct b200_tracker {
     trk::Dev d;
     void* arena = nullptr;          // one device allocation holding state + scratch + inputs + result
     static constexpr int kRing = 4;  // host staging slots: step_host_async may run this many steps ahead of their results
-    void* pinned = nullptr;         // host staging: kRing x (inputs then result)
-    size_t in_bytes = 0, res_bytes = 0, slot_bytes = 0;
+    void* pinned = nullptr;         // host staging: kRing x trk::Slot
+    size_t res_bytes = 0, slot_bytes = 0;
     cudaEvent_t done[kRing] = {};   // result of the step staged in slot i is on the host
     // Device side of the ring (inputs then result per slot, same layout as a pinned slot) and two private streams: the
     // upload of step k+1 and the download of step k's result run beside the kernels of step k instead of in line with
@@ -1318,13 +1338,12 @@ struct b200_tracker {
     cudaEvent_t up[kRing] = {}, ran[kRing] = {};
     long long ticket_of[kRing] = {-1, -1, -1, -1};
     long long next_ticket = 0;
-    int* in_ndet = nullptr; int* in_frame = nullptr; double* in_boxes = nullptr; double* in_confs = nullptr;
-    float* in_embs = nullptr; int* dev_result = nullptr;
-    // input block of b200_tracker_step_packed, separate from in_* and the ring so that a packed step queued on one stream
-    // never races with a host step or a step-by-step operation queued on another
-    int* pk_ndet = nullptr; double* pk_boxes = nullptr; double* pk_confs = nullptr; float* pk_embs = nullptr;
+    trk::StepInputs in = {};        // inputs of the step-by-step operations
+    int* dev_result = nullptr;
+    // input block of b200_tracker_step_packed (its frame ids are the caller's), separate from `in` and the ring so that a
+    // packed step queued on one stream never races with a host step or a step-by-step operation queued on another
+    trk::StepInputs pk = {};
     int* pk_inv = nullptr; int* pk_over = nullptr;
-    int ctl_threads = 256;              // CTA width of the per-stream control kernels (assign)
 #ifndef B200_TRK_BEGIN_THREADS
 #define B200_TRK_BEGIN_THREADS 256
 #endif
@@ -1338,20 +1357,6 @@ struct b200_tracker {
     int front_resident = 0;             // CTAs of front_kernel the device holds at once
     size_t front_smem = 0, back_smem = 0;
 };
-
-namespace {
-
-struct Carver {
-    size_t off = 0;
-    template <typename T> size_t take(size_t n) {
-        off = (off + 255) & ~(size_t)255;
-        const size_t at = off;
-        off += n * sizeof(T);
-        return at;
-    }
-};
-
-}  // namespace
 
 extern "C" int b200_tracker_create(b200_tracker** out, int n_streams, int max_tracks, int max_dets,
                                    const b200_tracker_conf* conf) {
@@ -1369,67 +1374,41 @@ extern "C" int b200_tracker_create(b200_tracker** out, int n_streams, int max_tr
     const size_t S = n_streams, MT = max_tracks, MD = max_dets, H = conf->hist_max;
     d.S = n_streams; d.MT = max_tracks; d.MD = max_dets; d.HIST = conf->hist_max;
     d.res_stride = trk::R_HDR + 2 * max_dets + max_tracks + max_dets;
-    Carver c;
-#define TAKE(field, T, n) const size_t o_##field = c.take<T>(n)
-    TAKE(kf_x, double, S * MT * 8); TAKE(kf_P, double, S * MT * 64); TAKE(last_bbox, double, S * MT * 4);
-    TAKE(last_conf, double, S * MT); TAKE(last_cost, double, S * MT); TAKE(kf_stage, uint8_t, S * MT);
-    TAKE(ema, float, S * MT * 128); TAKE(bank, float, S * MT * H * 128);
-    TAKE(bank_len, int, S * MT); TAKE(bank_head, int, S * MT); TAKE(tid, int, S * MT); TAKE(miss, int, S * MT);
-    TAKE(age, int, S * MT); TAKE(last_frame, int, S * MT); TAKE(order, int, S * MT); TAKE(free_list, int, S * MT);
-    TAKE(hdr, int, S * trk::kHdr);
-    TAKE(det_unit, float, S * MD * 128); TAKE(det_z, float, S * MD * 4); TAKE(det_boxf, float, S * MD * 4);
-    TAKE(det_conff, float, S * MD); TAKE(prev_boxf, float, S * MT * 4); TAKE(prev_conff, float, S * MT);
-    TAKE(C1, float, S * MT * MD); TAKE(C1T, float, S * MT * MD); TAKE(C2, float, S * MT * MD);
-    TAKE(C2T, float, S * MT * MD); TAKE(gate_SI, double, S * MT * 16);
-    TAKE(row_fc, int, S * MT); TAKE(row_fv, float, S * MT);
-    TAKE(rows_main, int, S * MT); TAKE(rows_reid, int, S * MT); TAKE(cnt, int, S * trk::kHdr);
-    TAKE(ud1, int, S * MD); TAKE(det_used, int, S * MD); TAKE(m_row, int, S * MT); TAKE(m_det, int, S * MT);
-    TAKE(m_app, int, S * MT); TAKE(tmp, int, S * MT); TAKE(born, int, S * MD);
     const size_t tiles_max = (MD + cost::kTileN - 1) / cost::kTileN;
-    TAKE(work1, int2, S * MT * tiles_max); TAKE(work2, int2, S * MT * tiles_max); TAKE(wcount, int, 4);
-    TAKE(upd_slot, int, S * MT); TAKE(upd_det, int, S * MT); TAKE(upd_cost, float, S * MT); TAKE(upd_flag, uint8_t, S * MT);
-    // inputs (one contiguous block so step_host needs a single H2D copy) and the result table
-    const size_t o_in = c.take<double>(0);
-    TAKE(in_ndet, int, S); TAKE(in_frame, int, S); TAKE(in_boxes, double, S * MD * 4); TAKE(in_confs, double, S * MD);
-    TAKE(in_embs, float, S * MD * 128);
-    const size_t in_end = c.off;
-    TAKE(result, int, S * (size_t)d.res_stride);
-    TAKE(pk_ndet, int, S); TAKE(pk_boxes, double, S * MD * 4); TAKE(pk_confs, double, S * MD);
-    TAKE(pk_embs, float, S * MD * 128); TAKE(pk_inv, int, S * MD); TAKE(pk_over, int, S);
-#undef TAKE
-    cudaError_t e = cudaMalloc(&t->arena, c.off);
+    auto carve_arena = [&](trk::Carver& c) {
+        c.take(d.kf_x, S * MT * 8); c.take(d.kf_P, S * MT * 64); c.take(d.last_bbox, S * MT * 4);
+        c.take(d.last_conf, S * MT); c.take(d.last_cost, S * MT); c.take(d.kf_stage, S * MT);
+        c.take(d.ema, S * MT * 128); c.take(d.bank, S * MT * H * 128);
+        c.take(d.bank_len, S * MT); c.take(d.bank_head, S * MT); c.take(d.tid, S * MT); c.take(d.miss, S * MT);
+        c.take(d.age, S * MT); c.take(d.last_frame, S * MT); c.take(d.order, S * MT); c.take(d.free_list, S * MT);
+        c.take(d.hdr, S * trk::kHdr);
+        c.take(d.det_unit, S * MD * 128); c.take(d.det_z, S * MD * 4); c.take(d.det_boxf, S * MD * 4);
+        c.take(d.det_conff, S * MD); c.take(d.prev_boxf, S * MT * 4); c.take(d.prev_conff, S * MT);
+        c.take(d.C1, S * MT * MD); c.take(d.C1T, S * MT * MD); c.take(d.C2, S * MT * MD);
+        c.take(d.C2T, S * MT * MD); c.take(d.gate_SI, S * MT * 16);
+        c.take(d.row_fc, S * MT); c.take(d.row_fv, S * MT);
+        c.take(d.rows_main, S * MT); c.take(d.rows_reid, S * MT); c.take(d.cnt, S * trk::kHdr);
+        c.take(d.ud1, S * MD); c.take(d.det_used, S * MD); c.take(d.m_row, S * MT); c.take(d.m_det, S * MT);
+        c.take(d.tmp, S * MT); c.take(d.born, S * MD);
+        c.take(d.work1, S * MT * tiles_max); c.take(d.work2, S * MT * tiles_max); c.take(d.wcount, 4);
+        c.take(d.upd_slot, S * MT); c.take(d.upd_det, S * MT); c.take(d.upd_cost, S * MT); c.take(d.upd_flag, S * MT);
+        trk::take_inputs(c, t->in, S, MD);
+        c.take(t->dev_result, S * (size_t)d.res_stride);
+        trk::take_inputs(c, t->pk, S, MD);
+        c.take(t->pk_inv, S * MD); c.take(t->pk_over, S);
+    };
+    trk::Carver size;
+    carve_arena(size);
+    cudaError_t e = cudaMalloc(&t->arena, size.off);
     if (e != cudaSuccess) {
         delete t;
-        return fail(B200_ECUDA, "tracker_create: cudaMalloc(%zu bytes): %s", c.off, cudaGetErrorString(e));
+        return fail(B200_ECUDA, "tracker_create: cudaMalloc(%zu bytes): %s", size.off, cudaGetErrorString(e));
     }
-    char* base = static_cast<char*>(t->arena);
-    cudaMemset(base, 0, c.off);
-#define PTR(field, T) d.field = reinterpret_cast<T*>(base + o_##field)
-    PTR(kf_x, double); PTR(kf_P, double); PTR(last_bbox, double); PTR(last_conf, double); PTR(last_cost, double);
-    PTR(kf_stage, uint8_t); PTR(ema, float); PTR(bank, float); PTR(bank_len, int); PTR(bank_head, int); PTR(tid, int);
-    PTR(miss, int); PTR(age, int); PTR(last_frame, int); PTR(order, int); PTR(free_list, int); PTR(hdr, int);
-    PTR(det_unit, float); PTR(det_z, float); PTR(det_boxf, float); PTR(det_conff, float); PTR(prev_boxf, float);
-    PTR(prev_conff, float); PTR(C1, float); PTR(C1T, float); PTR(C2, float); PTR(C2T, float); PTR(gate_SI, double);
-    PTR(row_fc, int); PTR(row_fv, float);
-    PTR(rows_main, int); PTR(rows_reid, int); PTR(cnt, int); PTR(ud1, int); PTR(det_used, int); PTR(m_row, int);
-    PTR(m_det, int); PTR(m_app, int); PTR(tmp, int); PTR(born, int); PTR(work1, int2); PTR(work2, int2); PTR(wcount, int);
-    PTR(upd_slot, int); PTR(upd_det, int); PTR(upd_cost, float); PTR(upd_flag, uint8_t);
-#undef PTR
-    t->in_ndet = reinterpret_cast<int*>(base + o_in_ndet);
-    t->in_frame = reinterpret_cast<int*>(base + o_in_frame);
-    t->in_boxes = reinterpret_cast<double*>(base + o_in_boxes);
-    t->in_confs = reinterpret_cast<double*>(base + o_in_confs);
-    t->in_embs = reinterpret_cast<float*>(base + o_in_embs);
-    t->dev_result = reinterpret_cast<int*>(base + o_result);
-    t->pk_ndet = reinterpret_cast<int*>(base + o_pk_ndet);
-    t->pk_boxes = reinterpret_cast<double*>(base + o_pk_boxes);
-    t->pk_confs = reinterpret_cast<double*>(base + o_pk_confs);
-    t->pk_embs = reinterpret_cast<float*>(base + o_pk_embs);
-    t->pk_inv = reinterpret_cast<int*>(base + o_pk_inv);
-    t->pk_over = reinterpret_cast<int*>(base + o_pk_over);
-    t->in_bytes = in_end - o_in;
+    trk::Carver c{static_cast<char*>(t->arena)};
+    carve_arena(c);
+    cudaMemset(t->arena, 0, c.off);
     t->res_bytes = S * (size_t)d.res_stride * sizeof(int);
-    t->slot_bytes = ((t->in_bytes + 255) & ~(size_t)255) + ((t->res_bytes + 255) & ~(size_t)255);
+    t->slot_bytes = trk::Slot(nullptr, d).bytes;
     e = cudaMallocHost(&t->pinned, t->slot_bytes * b200_tracker::kRing);
     if (e == cudaSuccess) e = cudaMalloc(&t->ring_dev, t->slot_bytes * b200_tracker::kRing);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&t->up_stream, cudaStreamNonBlocking);
@@ -1443,7 +1422,6 @@ extern "C" int b200_tracker_create(b200_tracker** out, int n_streams, int max_tr
         b200_tracker_destroy(t);
         return fail(B200_ECUDA, "tracker_create: host ring / streams: %s", cudaGetErrorString(e));
     }
-    // host offsets inside the pinned block mirror the device input block
     d.pw = cost::PairWeights{(float)conf->w_app, (float)conf->w_bbox, (float)conf->w_conf, (float)conf->alpha,
                              (float)conf->beta, 1e-6f};
     d.maha_thr = conf->maha_thr; d.cost_max = conf->cost_max; d.conf_update_min = conf->conf_update_min;
@@ -1516,9 +1494,6 @@ extern "C" int b200_tracker_create(b200_tracker** out, int n_streams, int max_tr
             per_sm = 1;
             cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, trk::front_kernel, trk::kFrontWarps * 32, t->front_smem);
             t->front_resident = sms * (per_sm > 0 ? per_sm : 1);
-            // experiment knobs: total CTAs of the front / update kernels (a smaller footprint leaves SM room to ROI Align)
-            if (const char* e = getenv("B200TRACK_FRONT_CTAS")) t->front_resident = atoi(e) > 0 ? atoi(e) : t->front_resident;
-            if (const char* e = getenv("B200TRACK_UPD_CTAS")) t->upd_grid = atoi(e) > 0 ? atoi(e) : t->upd_grid;
         }
     }
     *out = t;
@@ -1595,16 +1570,8 @@ extern "C" int b200_tracker_step(b200_tracker* t, const int32_t* n_det, const do
         // few streams: a cluster of CTAs per stream shares the updates, and the kernel is resident when the front one ends
         const bool few = d.S <= 8;
         const int cl = few ? trk::kBackCluster : 1;
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(d.S * cl); cfg.blockDim = dim3(trk::kThreads); cfg.dynamicSmemBytes = t->back_smem; cfg.stream = st;
-        cudaLaunchAttribute attr[2];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        attr[1].id = cudaLaunchAttributeClusterDimension;
-        attr[1].val.clusterDim.x = cl; attr[1].val.clusterDim.y = 1; attr[1].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = few ? 2 : 0;
-        (void)cudaLaunchKernelEx(&cfg, trk::back_kernel<true>, d, t->smem_matrix_floats);
+        launch_ex(trk::back_kernel<true>, dim3(d.S * cl), dim3(trk::kThreads), t->back_smem, st, few, few ? cl : 0, d,
+                  t->smem_matrix_floats);
         return check_launch("trk back_kernel");
     }
     trk::begin_kernel<<<dim3(d.S, 2), t->begin_threads, 0, st>>>(d);
@@ -1615,26 +1582,17 @@ extern "C" int b200_tracker_step(b200_tracker* t, const int32_t* n_det, const do
     // time its predecessor finishes.  With many streams the chain shares the GPU with ROI Align of the next
     // frame and early-resident CTAs would only take SM slots away from it.
     const bool pdl = d.S <= 8;
-    auto launch = [&](auto kern, dim3 grid, dim3 block, size_t smem, auto... args) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = pdl ? 1 : 0;
-        (void)cudaLaunchKernelEx(&cfg, kern, args...);     // errors surface in check_launch()
-    };
-    if (d.HIST <= 32) launch(trk::cost1_sparse32_kernel, dim3(t->cost1_grid), dim3(trk::kCost1Warps * 32), 0, d);
-    else launch(trk::cost1_sparse_kernel, dim3(t->cost1_grid), dim3(trk::kCost1Warps * 32), 0, d);
+    const dim3 c1_grid(t->cost1_grid), c1_block(trk::kCost1Warps * 32);
+    if (d.HIST <= 32) launch_ex(trk::cost1_sparse32_kernel, c1_grid, c1_block, 0, st, pdl, 0, d);
+    else launch_ex(trk::cost1_sparse_kernel, c1_grid, c1_block, 0, st, pdl, 0, d);
     if ((rc = check_launch("trk cost1_sparse_kernel"))) return rc;
-    launch(trk::assign_kernel<1>, dim3(d.S), dim3(t->ctl_threads), t->assign_smem, d, t->smem_matrix_floats);
+    launch_ex(trk::assign_kernel<1>, dim3(d.S), dim3(trk::kThreads), t->assign_smem, st, pdl, 0, d, t->smem_matrix_floats);
     if ((rc = check_launch("trk assign_kernel<1>"))) return rc;
-    launch(trk::cost2_kernel, dim3(cost_grid), dim3(cost::kThreads), csm, d);
+    launch_ex(trk::cost2_kernel, dim3(cost_grid), dim3(cost::kThreads), csm, st, pdl, 0, d);
     if ((rc = check_launch("trk cost2_kernel"))) return rc;
-    launch(trk::assign_kernel<2>, dim3(d.S), dim3(t->ctl_threads), t->assign_smem, d, t->smem_matrix_floats);
+    launch_ex(trk::assign_kernel<2>, dim3(d.S), dim3(trk::kThreads), t->assign_smem, st, pdl, 0, d, t->smem_matrix_floats);
     if ((rc = check_launch("trk assign_kernel<2>"))) return rc;
-    launch(trk::update_kernel, dim3(t->upd_grid), dim3(trk::kUpdWarps * 32), 0, d);
+    launch_ex(trk::update_kernel, dim3(t->upd_grid), dim3(trk::kUpdWarps * 32), 0, st, pdl, 0, d);
     if ((rc = check_launch("trk update_kernel"))) return rc;
     return B200_OK;
 }
@@ -1663,12 +1621,13 @@ extern "C" int b200_tracker_step_packed(b200_tracker* t, int64_t K, const void* 
     p.S = t->d.S; p.MD = t->d.MD; p.K = (int)K; p.box_stride = box_stride; p.conf_stride = conf_stride;
     p.det_half = det_dtype == B200_DTYPE_F16; p.emb_half = emb_dtype == B200_DTYPE_F16;
     p.boxes = boxes; p.confs = confs; p.embs = embs; p.stream_index = stream_index; p.active = active;
-    p.n_det = t->pk_ndet; p.p_boxes = t->pk_boxes; p.p_confs = t->pk_confs; p.p_embs = t->pk_embs;
+    const trk::StepInputs& in = t->pk;
+    p.n_det = in.n_det; p.p_boxes = in.boxes; p.p_confs = in.confs; p.p_embs = in.embs;
     p.inv = t->pk_inv; p.over = t->pk_over; p.track_of_det = track_of_det;
     trk::pack_kernel<<<p.S, trk::kPackThreads, 0, st>>>(p);
     int rc = check_launch("trk pack_kernel");
     if (rc) return rc;
-    if ((rc = b200_tracker_step(t, t->pk_ndet, t->pk_boxes, t->pk_confs, t->pk_embs, frame_id, result, stream))) return rc;
+    if ((rc = b200_tracker_step(t, in.n_det, in.boxes, in.confs, in.embs, frame_id, result, stream))) return rc;
     trk::finish_kernel<<<p.S, trk::kThreads, 0, st>>>(p, result, t->d.res_stride);
     return check_launch("trk finish_kernel");
 }
@@ -1692,33 +1651,21 @@ int step_host_submit(b200_tracker* t, const int32_t* n_det_host, const double* b
     const int slot = (int)(t->next_ticket % b200_tracker::kRing);
     if (t->ticket_of[slot] >= 0) B200_CUDA(cudaEventSynchronize(t->done[slot]));      // the DMA that last used this slot
     char* pin = static_cast<char*>(t->pinned) + (size_t)slot * t->slot_bytes;
-    char* dev_in = reinterpret_cast<char*>(t->in_ndet);
-    auto host_of = [&](const void* dev_ptr) { return pin + (reinterpret_cast<const char*>(dev_ptr) - dev_in); };
-    int* h_ndet = reinterpret_cast<int*>(host_of(t->in_ndet));
-    int* h_frame = reinterpret_cast<int*>(host_of(t->in_frame));
-    double* h_boxes = reinterpret_cast<double*>(host_of(t->in_boxes));
-    double* h_confs = reinterpret_cast<double*>(host_of(t->in_confs));
-    float* h_embs = reinterpret_cast<float*>(host_of(t->in_embs));
+    char* dslot = static_cast<char*>(t->ring_dev) + (size_t)slot * t->slot_bytes;
+    const trk::Slot hs(pin, d), ds(dslot, d);
+    const trk::StepInputs& h = hs.in;
+    const trk::StepInputs& dv = ds.in;
     bool dense = true;                               // every stream full: three large copies instead of 3 S small ones
     int n_max = 0;
     for (int s = 0; s < d.S; ++s) {
         const int n = n_det_host[s];
         B200_REQUIRE(n <= d.MD, "tracker_step_host: stream %d has %d detections, capacity %d", s, n, d.MD);
-        h_ndet[s] = n;
-        h_frame[s] = frame_id_host[s];
+        h.n_det[s] = n;
+        h.frame[s] = frame_id_host[s];
         if (n != d.MD) dense = false;
         if (n > n_max) n_max = n;
         if (n > 0) B200_REQUIRE(boxes_host && confs_host && embs_host, "tracker_step_host: null detection arrays");
     }
-    // device side of the slot: same layout as the pinned slot (inputs, then the result table)
-    char* dslot = static_cast<char*>(t->ring_dev) + (size_t)slot * t->slot_bytes;
-    auto dev_of = [&](const void* base_ptr) { return dslot + (reinterpret_cast<const char*>(base_ptr) - dev_in); };
-    int* d_ndet = reinterpret_cast<int*>(dev_of(t->in_ndet));
-    int* d_frame = reinterpret_cast<int*>(dev_of(t->in_frame));
-    double* d_boxes = reinterpret_cast<double*>(dev_of(t->in_boxes));
-    double* d_confs = reinterpret_cast<double*>(dev_of(t->in_confs));
-    float* d_embs = reinterpret_cast<float*>(dev_of(t->in_embs));
-    int* d_res = reinterpret_cast<int*>(dslot + ((t->in_bytes + 255) & ~(size_t)255));
     cudaStream_t up = inline_dma ? st : t->up_stream, down = inline_dma ? st : t->down_stream;
     if (direct) {
         const void* arrs[3] = {boxes_host, confs_host, embs_host};
@@ -1731,41 +1678,40 @@ int step_host_submit(b200_tracker* t, const int32_t* n_det_host, const double* b
                          "(cudaHostAlloc / cudaHostRegister / torch pin_memory)");
         }
         // the two small per-stream vectors go through the ring slot (the caller may reuse them at once)
-        B200_CUDA(cudaMemcpyAsync(d_ndet, h_ndet, sizeof(int) * d.S, cudaMemcpyHostToDevice, up));
-        B200_CUDA(cudaMemcpyAsync(d_frame, h_frame, sizeof(int) * d.S, cudaMemcpyHostToDevice, up));
+        B200_CUDA(cudaMemcpyAsync(dv.n_det, h.n_det, sizeof(int) * d.S, cudaMemcpyHostToDevice, up));
+        B200_CUDA(cudaMemcpyAsync(dv.frame, h.frame, sizeof(int) * d.S, cudaMemcpyHostToDevice, up));
         if (n_max > 0) {
-            B200_CUDA(cudaMemcpyAsync(d_boxes, boxes_host, sizeof(double) * 4 * (size_t)d.S * d.MD, cudaMemcpyHostToDevice, up));
-            B200_CUDA(cudaMemcpyAsync(d_confs, confs_host, sizeof(double) * (size_t)d.S * d.MD, cudaMemcpyHostToDevice, up));
-            B200_CUDA(cudaMemcpyAsync(d_embs, embs_host, sizeof(float) * 128 * (size_t)d.S * d.MD, cudaMemcpyHostToDevice, up));
+            B200_CUDA(cudaMemcpyAsync(dv.boxes, boxes_host, sizeof(double) * 4 * (size_t)d.S * d.MD, cudaMemcpyHostToDevice, up));
+            B200_CUDA(cudaMemcpyAsync(dv.confs, confs_host, sizeof(double) * (size_t)d.S * d.MD, cudaMemcpyHostToDevice, up));
+            B200_CUDA(cudaMemcpyAsync(dv.embs, embs_host, sizeof(float) * 128 * (size_t)d.S * d.MD, cudaMemcpyHostToDevice, up));
         }
     } else {
         if (dense) {
-            memcpy(h_boxes, boxes_host, sizeof(double) * 4 * (size_t)d.S * d.MD);
-            memcpy(h_confs, confs_host, sizeof(double) * (size_t)d.S * d.MD);
-            memcpy(h_embs, embs_host, sizeof(float) * 128 * (size_t)d.S * d.MD);
+            memcpy(h.boxes, boxes_host, sizeof(double) * 4 * (size_t)d.S * d.MD);
+            memcpy(h.confs, confs_host, sizeof(double) * (size_t)d.S * d.MD);
+            memcpy(h.embs, embs_host, sizeof(float) * 128 * (size_t)d.S * d.MD);
         } else {
             for (int s = 0; s < d.S; ++s) {
                 const int n = n_det_host[s];
                 if (n <= 0) continue;
-                memcpy(h_boxes + (size_t)s * d.MD * 4, boxes_host + (size_t)s * d.MD * 4, sizeof(double) * 4 * n);
-                memcpy(h_confs + (size_t)s * d.MD, confs_host + (size_t)s * d.MD, sizeof(double) * n);
-                memcpy(h_embs + (size_t)s * d.MD * 128, embs_host + (size_t)s * d.MD * 128, sizeof(float) * 128 * n);
+                memcpy(h.boxes + (size_t)s * d.MD * 4, boxes_host + (size_t)s * d.MD * 4, sizeof(double) * 4 * n);
+                memcpy(h.confs + (size_t)s * d.MD, confs_host + (size_t)s * d.MD, sizeof(double) * n);
+                memcpy(h.embs + (size_t)s * d.MD * 128, embs_host + (size_t)s * d.MD * 128, sizeof(float) * 128 * n);
             }
         }
-        B200_CUDA(cudaMemcpyAsync(dslot, pin, t->in_bytes, cudaMemcpyHostToDevice, up));
+        B200_CUDA(cudaMemcpyAsync(dslot, pin, hs.in_bytes, cudaMemcpyHostToDevice, up));
     }
     if (!inline_dma) {
         B200_CUDA(cudaEventRecord(t->up[slot], up));
         B200_CUDA(cudaStreamWaitEvent(st, t->up[slot], 0));        // the caller's stream runs the kernels
     }
-    const int rc = b200_tracker_step(t, d_ndet, d_boxes, d_confs, d_embs, d_frame, d_res, stream);
+    const int rc = b200_tracker_step(t, dv.n_det, dv.boxes, dv.confs, dv.embs, dv.frame, ds.result, stream);
     if (rc) return rc;
     if (!inline_dma) {
         B200_CUDA(cudaEventRecord(t->ran[slot], st));
         B200_CUDA(cudaStreamWaitEvent(down, t->ran[slot], 0));
     }
-    char* h_res = pin + ((t->in_bytes + 255) & ~(size_t)255);
-    B200_CUDA(cudaMemcpyAsync(h_res, d_res, t->res_bytes, cudaMemcpyDeviceToHost, down));
+    B200_CUDA(cudaMemcpyAsync(hs.result, ds.result, t->res_bytes, cudaMemcpyDeviceToHost, down));
     B200_CUDA(cudaEventRecord(t->done[slot], down));
     t->ticket_of[slot] = t->next_ticket;
     *ticket = t->next_ticket++;
@@ -1791,8 +1737,8 @@ extern "C" int b200_tracker_step_result(b200_tracker* t, int64_t ticket, int32_t
     B200_REQUIRE(ticket >= 0 && t->ticket_of[slot] == ticket, "tracker_step_result: ticket %lld is not in flight (at most %d steps may be pending)",
                  (long long)ticket, b200_tracker::kRing);
     B200_CUDA(cudaEventSynchronize(t->done[slot]));
-    const char* pin = static_cast<const char*>(t->pinned) + (size_t)slot * t->slot_bytes;
-    memcpy(result_host, pin + ((t->in_bytes + 255) & ~(size_t)255), t->res_bytes);
+    const trk::Slot hs(static_cast<char*>(t->pinned) + (size_t)slot * t->slot_bytes, t->d);
+    memcpy(result_host, hs.result, t->res_bytes);
     t->ticket_of[slot] = -1;
     return B200_OK;
 }
@@ -1816,14 +1762,15 @@ int stage_stream_inputs(b200_tracker* t, int s, int n_det, const double* boxes_h
     *d = t->d;
     B200_REQUIRE(n_det >= 0 && n_det <= d->MD, "tracker op: %d detections, capacity %d", n_det, d->MD);
     const size_t MD = d->MD;
+    const trk::StepInputs& in = t->in;
     if (n_det > 0) {
         B200_REQUIRE(boxes_host && confs_host && embs_host, "tracker op: null detection arrays");
-        B200_CUDA(cudaMemcpyAsync(t->in_boxes + (size_t)s * MD * 4, boxes_host, sizeof(double) * 4 * n_det, cudaMemcpyHostToDevice, st));
-        B200_CUDA(cudaMemcpyAsync(t->in_confs + (size_t)s * MD, confs_host, sizeof(double) * n_det, cudaMemcpyHostToDevice, st));
-        B200_CUDA(cudaMemcpyAsync(t->in_embs + (size_t)s * MD * 128, embs_host, sizeof(float) * 128 * n_det, cudaMemcpyHostToDevice, st));
+        B200_CUDA(cudaMemcpyAsync(in.boxes + (size_t)s * MD * 4, boxes_host, sizeof(double) * 4 * n_det, cudaMemcpyHostToDevice, st));
+        B200_CUDA(cudaMemcpyAsync(in.confs + (size_t)s * MD, confs_host, sizeof(double) * n_det, cudaMemcpyHostToDevice, st));
+        B200_CUDA(cudaMemcpyAsync(in.embs + (size_t)s * MD * 128, embs_host, sizeof(float) * 128 * n_det, cudaMemcpyHostToDevice, st));
     }
-    B200_CUDA(cudaMemcpyAsync(t->in_frame + s, &frame_id, sizeof(int), cudaMemcpyHostToDevice, st));
-    d->n_det = t->in_ndet; d->boxes = t->in_boxes; d->confs = t->in_confs; d->embs = t->in_embs; d->frame_id = t->in_frame;
+    B200_CUDA(cudaMemcpyAsync(in.frame + s, &frame_id, sizeof(int), cudaMemcpyHostToDevice, st));
+    d->n_det = in.n_det; d->boxes = in.boxes; d->confs = in.confs; d->embs = in.embs; d->frame_id = in.frame;
     d->result = t->dev_result;
     return B200_OK;
 }
@@ -1947,30 +1894,34 @@ extern "C" int b200_tracker_export(b200_tracker* t, int stream_idx, int32_t* ids
     B200_REQUIRE(stream_idx >= 0 && stream_idx < d.S, "tracker_export: stream %d out of range", stream_idx);
     cudaStream_t st = as_stream(stream);
     const size_t MT = d.MT, H = d.HIST;
-    Carver c;
-    const size_t o_ids = c.take<int>(MT), o_x = c.take<double>(MT * 8), o_P = c.take<double>(MT * 64),
-                 o_stage = c.take<uint8_t>(MT), o_ema = c.take<float>(MT * 128), o_bank = c.take<float>(MT * H * 128),
-                 o_bl = c.take<int>(MT), o_miss = c.take<int>(MT), o_age = c.take<int>(MT),
-                 o_lb = c.take<double>(MT * 4), o_lc = c.take<double>(MT), o_lk = c.take<double>(MT);
+    // staging buffer: the stream's live tracks packed in ascending track id
+    int *s_ids, *s_bl, *s_miss, *s_age;
+    double *s_x, *s_P, *s_lb, *s_lc, *s_lk;
+    uint8_t* s_stage;
+    float *s_ema, *s_bank;
+    auto carve = [&](trk::Carver& c) {
+        c.take(s_ids, MT); c.take(s_x, MT * 8); c.take(s_P, MT * 64); c.take(s_stage, MT); c.take(s_ema, MT * 128);
+        c.take(s_bank, MT * H * 128); c.take(s_bl, MT); c.take(s_miss, MT); c.take(s_age, MT); c.take(s_lb, MT * 4);
+        c.take(s_lc, MT); c.take(s_lk, MT);
+    };
+    trk::Carver size;
+    carve(size);
     char* buf = nullptr;
-    B200_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&buf), c.off, st));
-    trk::export_kernel<<<d.MT < 256 ? d.MT : 256, 128, 0, st>>>(
-        d, stream_idx, reinterpret_cast<int*>(buf + o_ids), reinterpret_cast<double*>(buf + o_x),
-        reinterpret_cast<double*>(buf + o_P), reinterpret_cast<uint8_t*>(buf + o_stage),
-        reinterpret_cast<float*>(buf + o_ema), reinterpret_cast<float*>(buf + o_bank), reinterpret_cast<int*>(buf + o_bl),
-        reinterpret_cast<int*>(buf + o_miss), reinterpret_cast<int*>(buf + o_age), reinterpret_cast<double*>(buf + o_lb),
-        reinterpret_cast<double*>(buf + o_lc), reinterpret_cast<double*>(buf + o_lk));
+    B200_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&buf), size.off, st));
+    trk::Carver c{buf};
+    carve(c);
+    trk::export_kernel<<<d.MT < 256 ? d.MT : 256, 128, 0, st>>>(d, stream_idx, s_ids, s_x, s_P, s_stage, s_ema, s_bank, s_bl,
+                                                                 s_miss, s_age, s_lb, s_lc, s_lk);
     int rc = check_launch("trk export_kernel");
     if (rc) return rc;
     int hdr[trk::kHdr];
     B200_CUDA(cudaMemcpyAsync(hdr, d.hdr + stream_idx * trk::kHdr, sizeof(hdr), cudaMemcpyDeviceToHost, st));
     B200_CUDA(cudaStreamSynchronize(st));
     const size_t n = hdr[trk::H_NLIVE];
-#define PULL(dst, off, T, per) if (dst && n) B200_CUDA(cudaMemcpyAsync(dst, buf + off, sizeof(T) * (per) * n, cudaMemcpyDeviceToHost, st))
-    PULL(ids, o_ids, int, 1); PULL(x, o_x, double, 8); PULL(P, o_P, double, 64); PULL(stage, o_stage, uint8_t, 1);
-    PULL(ema, o_ema, float, 128); PULL(bank, o_bank, float, H * 128); PULL(bank_len, o_bl, int, 1);
-    PULL(miss, o_miss, int, 1); PULL(age, o_age, int, 1); PULL(last_bbox, o_lb, double, 4);
-    PULL(last_conf, o_lc, double, 1); PULL(last_cost, o_lk, double, 1);
+#define PULL(dst, src, per) if (dst && n) B200_CUDA(cudaMemcpyAsync(dst, src, sizeof(*src) * (per) * n, cudaMemcpyDeviceToHost, st))
+    PULL(ids, s_ids, 1); PULL(x, s_x, 8); PULL(P, s_P, 64); PULL(stage, s_stage, 1); PULL(ema, s_ema, 128);
+    PULL(bank, s_bank, H * 128); PULL(bank_len, s_bl, 1); PULL(miss, s_miss, 1); PULL(age, s_age, 1);
+    PULL(last_bbox, s_lb, 4); PULL(last_conf, s_lc, 1); PULL(last_cost, s_lk, 1);
 #undef PULL
     if (next_id) *next_id = hdr[trk::H_NEXT];
     B200_CUDA(cudaStreamSynchronize(st));
@@ -1978,7 +1929,6 @@ extern "C" int b200_tracker_export(b200_tracker* t, int stream_idx, int32_t* ids
     return (int)n;
 }
 
-#ifdef B200_TRK_TIMING
 #ifdef B200_TRK_TIMING
 extern "C" int b200_debug_lsap_stats(unsigned long long* out4, int reset) {
     unsigned long long z[4] = {0, 0, 0, 0};
@@ -1990,7 +1940,6 @@ extern "C" int b200_debug_lsap_clk(long long* out8) {
     cudaMemcpyFromSymbol(out8, b200::lsap::g_lsap_clk, 8 * sizeof(long long));
     return 0;
 }
-#endif
 
 extern "C" int b200_debug_timing(long long* out32) {
     return cudaMemcpyFromSymbol(out32, b200::trk::g_timing, sizeof(long long) * 32) == cudaSuccess ? 0 : -2;

@@ -77,7 +77,7 @@ class MultiStreamTracker:
         self._h = ctypes.c_void_p()
         self._create(int(max_tracks), int(max_dets))
         self.n_live = np.zeros(self.S, dtype=np.int64)
-        self._n_live_stale = False                 # set by step_device: the host copy of the live counts is out of date
+        self._n_live_stale = False                 # set by device-side steps and step-by-step methods: n_live is out of date
         self._pending = []                         # StepHandles of step_async calls whose result has not been collected
         self._pending_births = np.zeros(self.S, dtype=np.int64)
 
@@ -100,7 +100,6 @@ class MultiStreamTracker:
             _lib.check(_lib.lib().b200_tracker_create(ctypes.byref(h), self.S, max_tracks, max_dets, ctypes.byref(cc)))
         self._h, self.max_tracks, self.max_dets = h, max_tracks, max_dets
         self.stride = _lib.lib().b200_tracker_result_stride(h)
-        self._res = np.zeros((self.S, self.stride), dtype=np.int32)
 
     def grow(self, max_tracks: Optional[int] = None, max_dets: Optional[int] = None):
         """Migrates every stream's state into a handle with larger capacities (export -> create -> import)."""
@@ -157,9 +156,10 @@ class MultiStreamTracker:
             rc = _lib.lib().b200_tracker_step_host(self._h, p(n_det), p(boxes), p(confs), p(embs), p(frame_ids), p(res),
                                                    _lib.stream_ptr(self.device))
         _lib.check(rc)
-        h = StepHandle(self, -1, np.zeros(self.S, np.int64))
-        h._finish(res)
-        return h.result()
+        err = self._read_result(res, current=True)
+        if err is not None:
+            raise err
+        return res
 
     def step_async(self, n_det, boxes, confs, embs, frame_ids, *, pinned: bool = False) -> "StepHandle":
         """``step`` without the wait: uploads the detections, queues the step and the download of the result table on the
@@ -204,20 +204,47 @@ class MultiStreamTracker:
             boxes = np.ascontiguousarray(boxes, dtype=np.float64).reshape(self.S, self.max_dets, 4)
             confs = np.ascontiguousarray(confs, dtype=np.float64).reshape(self.S, self.max_dets)
             embs = np.ascontiguousarray(embs, dtype=np.float32).reshape(self.S, self.max_dets, 128)
-        # capacity: live tracks are only known up to the last collected result; every pending step may have added
-        # all of its detections
+        self._reserve_tracks(n_det)
+        return n_det, boxes, confs, embs, frame_ids
+
+    def _reserve_tracks(self, n_det):
+        """Grows the handle (raises with ``auto_grow=False``) unless live tracks + ``n_det`` fit in ``max_tracks``, where
+        every pending step may have added all of its detections."""
+        if self._n_live_stale:                         # device-side calls may have created tracks the host has not counted
+            self.n_live_now()
         bound = self.n_live + self._pending_births + np.maximum(n_det, 0)
         while int(bound.max()) > self.max_tracks and self._pending:     # collect the oldest results until the bound fits
             self._pending[0]._collect()
             bound = self.n_live + self._pending_births + np.maximum(n_det, 0)
-        if int(bound.max()) > self.max_tracks and self._n_live_stale:
-            bound = self.n_live_now() + np.maximum(n_det, 0)
         if int(bound.max()) > self.max_tracks:         # the reference is unbounded: migrate to a larger handle
             if not self.auto_grow:
                 raise _lib.B200Error("tracker capacity: live tracks + detections could exceed max_tracks=%d; "
                                      "construct the tracker with a larger max_tracks" % self.max_tracks)
             self.grow(max_tracks=max(int(bound.max()), 2 * self.max_tracks))
-        return n_det, boxes, confs, embs, frame_ids
+
+    def _read_result(self, res: np.ndarray, current: bool) -> Optional[Exception]:
+        """Takes a collected result table (live counts, ``last_result``); returns the exception the step raises, or None."""
+        self.n_live[:] = res[:, R_NLIVE]
+        if current:                                    # nothing was queued after this step: the live counts are exact
+            self._n_live_stale = False
+        # A failing stream does not lose the others: the table (handle.table; last_result = the most recently collected
+        # one) is complete before anything is raised, and the failing stream's state is what the reference leaves behind
+        # when scipy raises (predict only).
+        self.last_result = res
+        bad = np.nonzero(res[:, R_STATUS])[0]
+        if not len(bad):
+            return None
+        st = int(res[bad[0], R_STATUS])
+        if st == _lib.ENUMERIC:
+            return ValueError("matrix contains invalid numeric entries (stream %d)" % bad[0])
+        if st == _lib.EINFEASIBLE:
+            return ValueError("cost matrix is infeasible (stream %d)" % bad[0])
+        if st == _lib.ECAPACITY:
+            return _lib.B200Error(
+                "tracker capacity exceeded on stream %d: births were dropped because live tracks + detections "
+                "exceeded max_tracks=%d (device-side steps do not grow the handle; call grow() or construct with a "
+                "larger max_tracks)" % (bad[0], self.max_tracks))
+        return _lib.B200Error("tracker step failed on stream %d with status %d" % (bad[0], st))
 
     def drain(self):
         """Waits for every pending ``step_async`` (their results stay available on their handles)."""
@@ -365,32 +392,8 @@ class StepHandle:
         except Exception as exc:                       # noqa: BLE001
             self._error = exc
             return
-        self._finish(res)
-
-    def _finish(self, res):
-        """Takes the step's result table: live counts, last_result, and the error ``result()`` will raise, if any."""
-        ms = self._ms
         self._res = self.table = res
-        ms._res = res
-        ms.n_live[:] = res[:, R_NLIVE]
-        # A failing stream does not lose the others: the table (handle.table; ms.last_result = the most recently collected
-        # one) is complete before anything is raised, and the failing stream's state is what the reference leaves behind
-        # when scipy raises (predict only).
-        ms.last_result = res
-        bad = np.nonzero(res[:, R_STATUS])[0]
-        if len(bad):
-            st = int(res[bad[0], R_STATUS])
-            if st == _lib.ENUMERIC:
-                self._error = ValueError("matrix contains invalid numeric entries (stream %d)" % bad[0])
-            elif st == _lib.EINFEASIBLE:
-                self._error = ValueError("cost matrix is infeasible (stream %d)" % bad[0])
-            elif st == _lib.ECAPACITY:
-                self._error = _lib.B200Error(
-                    "tracker capacity exceeded on stream %d: births were dropped because live tracks + detections "
-                    "exceeded max_tracks=%d (device-side steps do not grow the handle; call grow() or construct with a "
-                    "larger max_tracks)" % (bad[0], ms.max_tracks))
-            else:
-                self._error = _lib.B200Error("tracker step failed on stream %d with status %d" % (bad[0], st))
+        self._error = ms._read_result(res, current=False)
 
     def done(self) -> bool:
         return self._res is not None or self._error is not None
@@ -485,10 +488,7 @@ class Tracking:
     def update_arrays(self, boxes: np.ndarray, confs: np.ndarray, embs: np.ndarray, frame_id: int):
         """Array form of ``update``: boxes [N,4] float64 xyxy, confs [N], embs [N,128] float32."""
         N = boxes.shape[0]
-        if N > self._ms.max_dets:
-            if not self._ms.auto_grow:
-                raise ValueError("%d detections exceed max_dets=%d" % (N, self._ms.max_dets))
-            self._ms.grow(max_dets=max(N, 2 * self._ms.max_dets))
+        self._reserve_dets(N)
         MD = self._ms.max_dets
         if self._boxes.shape[1] != MD:                 # the handle has grown (here or in one of the step-by-step methods)
             self._boxes, self._confs = np.zeros((1, MD, 4), np.float64), np.zeros((1, MD), np.float64)
@@ -513,26 +513,25 @@ class Tracking:
         if embs.shape[1] != 128:
             raise ValueError(f"det_embs must be 128D, got sizes [{embs.shape[1]}]")
         N = boxes.shape[0]
-        if N > ms.max_dets:
-            if not ms.auto_grow:
-                raise ValueError("%d detections exceed max_dets=%d" % (N, ms.max_dets))
-            ms.grow(max_dets=max(N, 2 * ms.max_dets))
-        bound = int(ms.n_live_now()[0]) + N
-        if bound > ms.max_tracks:                    # the reference is unbounded: migrate to a larger handle
-            if not ms.auto_grow:
-                raise _lib.B200Error("tracker capacity: live tracks + detections could exceed max_tracks=%d; "
-                                     "construct the tracker with a larger max_tracks" % ms.max_tracks)
-            ms.grow(max_tracks=max(bound, 2 * ms.max_tracks))
+        self._reserve_dets(N)
+        ms._reserve_tracks([N])
         if self._frame_dev is None:
             self._frame_dev = torch.empty((1,), dtype=torch.int32, device=self.device)
         self._frame_dev.fill_(int(frame_id))
         table, _ = ms.step_detections(boxes, confs, embs, self._frame_dev)
         res = table.cpu().numpy()
         self._snap = None
-        h = StepHandle(ms, -1, np.zeros(ms.S, np.int64))
-        h._finish(res)                               # live count from the table: the handle's count is current again
-        ms._n_live_stale = False
-        return ms.decode(h.result()[0])
+        err = ms._read_result(res, current=True)
+        if err is not None:
+            raise err
+        return ms.decode(res[0])
+
+    def _reserve_dets(self, n: int):
+        """Grows the handle's ``max_dets`` to hold ``n`` detections (raises instead with ``auto_grow=False``)."""
+        if n > self._ms.max_dets:
+            if not self._ms.auto_grow:
+                raise ValueError("%d detections exceed max_dets=%d" % (n, self._ms.max_dets))
+            self._ms.grow(max_dets=max(n, 2 * self._ms.max_dets))
 
     # -- the reference's methods one by one (mainTracking.py:340-448), on the device state -----------
     def _dets(self, det_embs, det_boxes, det_confs):

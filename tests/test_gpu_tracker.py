@@ -380,6 +380,44 @@ def test_step_device_vs_oracle():
     assert ms.n_live_now().tolist() == [len(r.tracks) for r in refs]
 
 
+@pytest.mark.parametrize("path", ["step_device", "create_new_tracks"])
+def test_host_step_grows_after_device_side_births(path):
+    """Tracks created by device-side calls (step_device, create_new_tracks) are not in the host's live count.  A host step
+    whose births do not fit beside them must grow the handle first, not drop them: two groups of 8 detections fill a
+    16-track handle, then a host step brings 8 more, far from every track, and must match the unbounded oracle."""
+    cfg = dict(SHIPPED_CONF)
+    rng = np.random.default_rng(3)
+    objs = []
+    for g in range(3):                              # 400 px between groups: the Mahalanobis gate rejects every pair
+        e = rng.standard_normal((8, 128)).astype(np.float32)
+        e /= np.linalg.norm(e, axis=1, keepdims=True)
+        objs.append({"embs": list(e), "bboxes": [[100.0 + 150 * j, 100.0 + 400 * g, 140.0 + 150 * j, 140.0 + 400 * g]
+                                                  for j in range(8)],
+                     "confs": [0.9] * 8, "input_hw": (1280, 1280), "frame_id": g})
+    ref = tracker_ref.TrackerRef(cfg)
+    trk = Tracking(conf=cfg, max_tracks=16, max_dets=8)
+    if path == "step_device":
+        ms = trk._ms
+        d = lambda a, dt: torch.tensor(np.asarray(a), dtype=dt, device="cuda")  # noqa: E731
+        for o in objs[:2]:
+            ref.update(o)
+            ms.step_device(d([8], torch.int32), d([o["bboxes"]], torch.float64), d([o["confs"]], torch.float64),
+                           d([np.stack(o["embs"])], torch.float32), d([o["frame_id"]], torch.int32))
+        res = ms.step([8], [objs[2]["bboxes"]], [objs[2]["confs"]], [np.stack(objs[2]["embs"])], [2])
+        got = ms.decode(res[0])
+    else:
+        for o in objs[:2]:
+            ref.spawn(range(8), o["embs"], o["bboxes"], o["confs"], o["frame_id"])
+            trk.create_new_tracks(range(8), o["embs"], o["bboxes"], o["confs"], o["frame_id"])
+        got = trk.update(objs[2])
+    want = ref.update(objs[2])
+    assert len(ref.tracks) == 24 and trk._ms.max_tracks >= 24
+    assert got[0] == want[0] and got[1] == want[1] and got[2] == want[2]
+    ids, st = _oracle_state(ref)
+    _compare_state(trk, ids, st, path)
+    assert trk.next_id == ref.next_id
+
+
 def test_step_async_matches_step_and_defers_errors():
     """MultiStreamTracker.step_async: up to four steps queued ahead of their results; every result equals the oracle's,
     results come back in order, a NaN frame raises at .result() of THAT step only and the stream carries on."""
