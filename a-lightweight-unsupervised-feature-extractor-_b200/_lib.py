@@ -42,6 +42,19 @@ class tracker_conf(ctypes.Structure):
 
 _P, _I, _L, _F, _D = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_float, ctypes.c_double
 
+# b200_tracker_state: (field, element type, shape after the row dimension; "cap" / "hist_max" are the image's), in the
+# struct's order.  n_live and next_id are [n_rows]; every other field is [n_rows, cap, ...].
+STATE_LAYOUT = (
+    ("n_live", "int32", ()), ("next_id", "int32", ()), ("ids", "int32", ("cap",)), ("x", "float64", ("cap", 8)),
+    ("P", "float64", ("cap", 8, 8)), ("stage", "uint8", ("cap",)), ("ema", "float32", ("cap", 128)),
+    ("bank", "float32", ("cap", "hist_max", 128)), ("bank_len", "int32", ("cap",)), ("miss", "int32", ("cap",)),
+    ("age", "int32", ("cap",)), ("last_bbox", "float64", ("cap", 4)), ("last_conf", "float64", ("cap",)),
+    ("last_cost", "float64", ("cap",)))
+
+
+class tracker_state(ctypes.Structure):
+    _fields_ = [(n, _P) for n, _, _ in STATE_LAYOUT] + [(n, ctypes.c_int32) for n in ("n_rows", "cap", "hist_max")]
+
 SIGNATURES = {
     "b200_version": (ctypes.c_int, []),
     "b200_last_error": (ctypes.c_char_p, []),
@@ -82,6 +95,8 @@ SIGNATURES = {
     "b200_peer_gather_destroy": (None, [_P]),
     "b200_tracker_export": (_I, [_P, _I] + [_P] * 14),
     "b200_tracker_import": (_I, [_P, _I, _I] + [_P] * 12 + [_I, _P]),
+    "b200_tracker_export_device": (_I, [_P, _P, ctypes.POINTER(tracker_state), _P, _P]),
+    "b200_tracker_import_device": (_I, [_P, _P, ctypes.POINTER(tracker_state), _P, _P]),
 }
 
 

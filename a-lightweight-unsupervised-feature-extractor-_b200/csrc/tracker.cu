@@ -1146,34 +1146,77 @@ __global__ void __launch_bounds__(kThreads) op_queue_matches_kernel(Dev d, int s
     if (threadIdx.x == 0) { out[1] = 0; d.wcount[2] = n; }
 }
 
-// Packs one stream's live tracks, ascending track id, for b200_tracker_export.
-__global__ void export_kernel(Dev d, int s, int* ids, double* x, double* P, uint8_t* stage, float* ema, float* bank,
-                              int* bank_len, int* miss, int* age, double* last_bbox, double* last_conf,
-                              double* last_cost) {
-    const size_t sb = (size_t)s * d.MT;
-    const int nl = d.hdr[s * kHdr + H_NLIVE];
-    for (int p = blockIdx.x; p < nl; p += gridDim.x) {
-        const size_t slot = sb + d.order[sb + p];
-        const int t = threadIdx.x;
-        if (t == 0) {
-            ids[p] = d.tid[slot]; stage[p] = d.kf_stage[slot]; bank_len[p] = d.bank_len[slot];
-            miss[p] = d.miss[slot]; age[p] = d.age[slot]; last_conf[p] = d.last_conf[slot];
-            last_cost[p] = d.last_cost[slot];
+// ---- state images (b200_tracker_state): export / import of any set of streams ------------------------------------------
+// One warp per (image row, track): a full 64-stream group of 256 tracks is 16 384 warps.  About 94 % of the bytes are the
+// history bank (hist_max x 512 B per track), moved one 512-byte row per warp instruction in 16-byte vectors with
+// kRowsInFlight rows of loads issued before their stores.
+constexpr int kStateWarps = 8;
+constexpr int kRowsInFlight = 6;
+
+// Moves one track between slot `slot` of the handle and track `it` (row * cap + position) of an image.  EXPORT: slot ->
+// image, the bank ring unrolled oldest row first and rows past bank_len zeroed (what b200_tracker_export writes); import:
+// image -> slot, every bank row in order (the slot's ring then starts at row 0, as after b200_tracker_import).
+template <bool EXPORT>
+__device__ __forceinline__ void copy_track(const Dev& d, const b200_tracker_state& im, size_t slot, size_t it, int lane) {
+    auto mv = [&](auto* s_side, auto* i_side) { if (EXPORT) *i_side = *s_side; else *s_side = *i_side; };
+    const int H = d.HIST;
+    const int len = EXPORT ? d.bank_len[slot] : H, head = EXPORT ? d.bank_head[slot] : 0;
+    float4* sb = reinterpret_cast<float4*>(d.bank) + slot * H * 32 + lane;
+    float4* ib = reinterpret_cast<float4*>(im.bank) + it * H * 32 + lane;
+    for (int j0 = 0; j0 < H; j0 += kRowsInFlight) {
+        float4 v[kRowsInFlight];
+#pragma unroll
+        for (int u = 0; u < kRowsInFlight; ++u) {
+            const int j = j0 + u;
+            const int sr = head + j < H ? head + j : head + j - H;        // slot row of image row j
+            v[u] = j < len ? (EXPORT ? sb[(size_t)sr * 32] : ib[(size_t)j * 32]) : make_float4(0.f, 0.f, 0.f, 0.f);
         }
-        if (t < 8) x[(size_t)p * 8 + t] = d.kf_x[slot * 8 + t];
-        if (t < 4) last_bbox[(size_t)p * 4 + t] = d.last_bbox[slot * 4 + t];
-        if (t < 64) P[(size_t)p * 64 + t] = d.kf_P[slot * 64 + t];
-        if (t < cost::kD) ema[(size_t)p * cost::kD + t] = d.ema[slot * cost::kD + t];
-        const int len = d.bank_len[slot], head = d.bank_head[slot];
-        for (int i = t; i < d.HIST * cost::kD; i += blockDim.x) {
-            const int row = i / cost::kD, k = i % cost::kD;
-            bank[((size_t)p * d.HIST + row) * cost::kD + k] =
-                row < len ? d.bank[(slot * d.HIST + (head + row) % d.HIST) * cost::kD + k] : 0.0f;
-        }
+#pragma unroll
+        for (int u = 0; u < kRowsInFlight; ++u)
+            if (j0 + u < H) (EXPORT ? ib : sb)[(size_t)(j0 + u) * 32] = v[u];
+    }
+    // P and ema: 512 B each, one vector per lane; x (64 B) and last_bbox (32 B): lanes 0-5; the scalars: lanes 8-14
+    mv(reinterpret_cast<float4*>(d.kf_P) + slot * 32 + lane, reinterpret_cast<float4*>(im.P) + it * 32 + lane);
+    mv(reinterpret_cast<float4*>(d.ema) + slot * 32 + lane, reinterpret_cast<float4*>(im.ema) + it * 32 + lane);
+    if (lane < 4) mv(reinterpret_cast<float4*>(d.kf_x) + slot * 4 + lane, reinterpret_cast<float4*>(im.x) + it * 4 + lane);
+    else if (lane < 6) mv(reinterpret_cast<float4*>(d.last_bbox) + slot * 2 + lane - 4,
+                          reinterpret_cast<float4*>(im.last_bbox) + it * 2 + lane - 4);
+    switch (lane) {
+        case 8: mv(d.tid + slot, im.ids + it); break;
+        case 9: mv(d.kf_stage + slot, im.stage + it); break;
+        case 10: mv(d.bank_len + slot, im.bank_len + it); break;
+        case 11: mv(d.miss + slot, im.miss + it); break;
+        case 12: mv(d.age + slot, im.age + it); break;
+        case 13: mv(d.last_conf + slot, im.last_conf + it); break;
+        case 14: mv(d.last_cost + slot, im.last_cost + it); break;
+        default: break;
     }
 }
 
-__global__ void import_finish_kernel(Dev d, int s, int n, int next_id) {
+__device__ __forceinline__ int image_stream(const int* streams, int s0, int r) { return streams ? streams[r] : s0 + r; }
+
+// grid (ceil(cap / kStateWarps), n_rows).  Row r is stream streams[r] (streams == nullptr: s0 + r); b200_tracker_export
+// runs it as a one-row image over its staging buffer.
+__global__ void __launch_bounds__(kStateWarps * 32) export_state_kernel(Dev d, b200_tracker_state im, const int* streams,
+                                                                         int s0, int* status) {
+    const int r = blockIdx.y;
+    const int s = image_stream(streams, s0, r);
+    const bool in_range = s >= 0 && s < d.S;
+    const int nl = in_range ? d.hdr[s * kHdr + H_NLIVE] : 0;
+    const bool ok = in_range && nl <= im.cap;
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        if (status) status[r] = !in_range ? B200_EINVAL : ok ? B200_OK : B200_ECAPACITY;
+        if (ok) { im.n_live[r] = nl; im.next_id[r] = d.hdr[s * kHdr + H_NEXT]; }
+    }
+    const int p = blockIdx.x * kStateWarps + (threadIdx.x >> 5);
+    if (!ok || p >= nl) return;
+    const size_t sb = (size_t)s * d.MT;
+    copy_track<true>(d, im, sb + d.order[sb + p], (size_t)r * im.cap + p, threadIdx.x & 31);
+}
+
+// The slot layout an import leaves in stream s (all threads of the CTA): tracks in slots 0..n-1 in id order, their bank
+// rings at row 0, free list MT-1 ... n, header counts.
+__device__ void finish_import(const Dev& d, int s, int n, int next_id) {
     const size_t sb = (size_t)s * d.MT;
     for (int i = threadIdx.x; i < d.MT; i += blockDim.x) {
         if (i < n) { d.order[sb + i] = i; d.bank_head[sb + i] = 0; d.last_frame[sb + i] = 0; }
@@ -1184,6 +1227,53 @@ __global__ void import_finish_kernel(Dev d, int s, int n, int next_id) {
         d.hdr[s * kHdr + H_NEXT] = next_id;
         d.hdr[s * kHdr + H_NFREE] = d.MT - n;
     }
+}
+
+__global__ void import_finish_kernel(Dev d, int s, int n, int next_id) { finish_import(d, s, n, next_id); }
+
+// One CTA per image row, ahead of import_state_kernel: validates the row (every index it reads is checked first) and, if it
+// passes, rebuilds the stream's header, order and free list.  imp_row[s] = r names the row import_state_kernel copies into
+// stream s (-1: none); only entries of streams named by this image are read, and each is written here first.
+__global__ void __launch_bounds__(kThreads) import_check_kernel(Dev d, b200_tracker_state im, const int* streams,
+                                                                 int* imp_row, int* status) {
+    const int r = blockIdx.x;
+    const int s = image_stream(streams, 0, r);
+    if (s < 0 || s >= d.S) {
+        if (status && threadIdx.x == 0) status[r] = B200_EINVAL;
+        return;
+    }
+    bool dup = false;                                // another row naming the same stream: neither is applied
+    if (streams)
+        for (int q = threadIdx.x; q < im.n_rows; q += blockDim.x) dup |= q != r && streams[q] == s;
+    const int n = im.n_live[r], next_id = im.next_id[r];
+    int st = __syncthreads_or(dup) || n < 0 ? B200_EINVAL
+             : n > (im.cap < d.MT ? im.cap : d.MT) ? B200_ECAPACITY : B200_OK;
+    if (st == B200_OK) {
+        const size_t rb = (size_t)r * im.cap;
+        bool bad = false;
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            const int id = im.ids[rb + i], bl = im.bank_len[rb + i];
+            bad |= id < 0 || id >= next_id || (i > 0 && im.ids[rb + i - 1] >= id) || bl < 0 || bl > d.HIST ||
+                   im.stage[rb + i] > 2;
+        }
+        if (__syncthreads_or(bad)) st = B200_EINVAL;
+    }
+    if (st == B200_OK) finish_import(d, s, n, next_id);
+    if (threadIdx.x == 0) {
+        imp_row[s] = st == B200_OK ? r : -1;
+        if (status) status[r] = st;
+    }
+}
+
+// grid (ceil(cap / kStateWarps), n_rows): copies the rows import_check_kernel accepted into slots 0..n-1 of their streams.
+__global__ void __launch_bounds__(kStateWarps * 32) import_state_kernel(Dev d, b200_tracker_state im, const int* streams,
+                                                                         const int* imp_row) {
+    const int r = blockIdx.y;
+    const int s = image_stream(streams, 0, r);
+    if (s < 0 || s >= d.S || imp_row[s] != r) return;
+    const int p = blockIdx.x * kStateWarps + (threadIdx.x >> 5);
+    if (p >= im.n_live[r]) return;
+    copy_track<false>(d, im, (size_t)s * d.MT + p, (size_t)r * im.cap + p, threadIdx.x & 31);
 }
 
 __global__ void reset_kernel(Dev d) {
@@ -1344,6 +1434,7 @@ struct b200_tracker {
     // packed step queued on one stream never races with a host step or a step-by-step operation queued on another
     trk::StepInputs pk = {};
     int* pk_inv = nullptr; int* pk_over = nullptr;
+    int* imp_row = nullptr;         // [S] b200_tracker_import_device: the image row accepted for each stream
 #ifndef B200_TRK_BEGIN_THREADS
 #define B200_TRK_BEGIN_THREADS 256
 #endif
@@ -1396,6 +1487,7 @@ extern "C" int b200_tracker_create(b200_tracker** out, int n_streams, int max_tr
         c.take(t->dev_result, S * (size_t)d.res_stride);
         trk::take_inputs(c, t->pk, S, MD);
         c.take(t->pk_inv, S * MD); c.take(t->pk_over, S);
+        c.take(t->imp_row, S);
     };
     trk::Carver size;
     carve_arena(size);
@@ -1885,6 +1977,54 @@ extern "C" int b200_tracker_update_matched(b200_tracker* t, int stream_idx, cons
     return B200_OK;
 }
 
+namespace {
+
+// Host-side argument checks shared by the two image entry points: the image's own first, then against the handle.
+int check_image(const b200_tracker* t, const int32_t* streams, const b200_tracker_state* im, const char* fn) {
+    B200_REQUIRE(im, "%s: null image", fn);
+    B200_REQUIRE(im->cap >= 1, "%s: image cap %d must be >= 1", fn, im->cap);
+    B200_REQUIRE(im->n_rows >= 0 && im->n_rows <= 65535, "%s: image n_rows %d outside [0, 65535]", fn, im->n_rows);
+    if (im->n_rows > 0) {
+        B200_REQUIRE(im->n_live && im->next_id && im->ids && im->x && im->P && im->stage && im->ema && im->bank &&
+                     im->bank_len && im->miss && im->age && im->last_bbox && im->last_conf && im->last_cost,
+                     "%s: null image field", fn);
+        const uintptr_t vec = reinterpret_cast<uintptr_t>(im->x) | reinterpret_cast<uintptr_t>(im->P) |
+                              reinterpret_cast<uintptr_t>(im->ema) | reinterpret_cast<uintptr_t>(im->bank) |
+                              reinterpret_cast<uintptr_t>(im->last_bbox);
+        B200_REQUIRE((vec & 15) == 0, "%s: image x / P / ema / bank / last_bbox must be 16-byte aligned", fn);
+    }
+    B200_REQUIRE(t, "%s: null handle", fn);
+    B200_REQUIRE(im->hist_max == t->d.HIST, "%s: image hist_max %d, handle hist_max %d", fn, im->hist_max, t->d.HIST);
+    B200_REQUIRE(streams || im->n_rows == t->d.S, "%s: streams == NULL needs n_rows == n_streams (%d, %d)", fn,
+                 im->n_rows, t->d.S);
+    return B200_OK;
+}
+
+dim3 image_grid(const b200_tracker_state& im) {
+    return dim3((unsigned)((im.cap + trk::kStateWarps - 1) / trk::kStateWarps), (unsigned)im.n_rows);
+}
+
+}  // namespace
+
+extern "C" int b200_tracker_export_device(b200_tracker* t, const int32_t* streams, const b200_tracker_state* img,
+                                          int32_t* status, void* stream) {
+    int rc = check_image(t, streams, img, "tracker_export_device");
+    if (rc || img->n_rows == 0) return rc;
+    trk::export_state_kernel<<<image_grid(*img), trk::kStateWarps * 32, 0, as_stream(stream)>>>(t->d, *img, streams, 0, status);
+    return check_launch("trk export_state_kernel");
+}
+
+extern "C" int b200_tracker_import_device(b200_tracker* t, const int32_t* streams, const b200_tracker_state* img,
+                                          int32_t* status, void* stream) {
+    int rc = check_image(t, streams, img, "tracker_import_device");
+    if (rc || img->n_rows == 0) return rc;
+    cudaStream_t st = as_stream(stream);
+    trk::import_check_kernel<<<img->n_rows, trk::kThreads, 0, st>>>(t->d, *img, streams, t->imp_row, status);
+    if ((rc = check_launch("trk import_check_kernel"))) return rc;
+    trk::import_state_kernel<<<image_grid(*img), trk::kStateWarps * 32, 0, st>>>(t->d, *img, streams, t->imp_row);
+    return check_launch("trk import_state_kernel");
+}
+
 extern "C" int b200_tracker_export(b200_tracker* t, int stream_idx, int32_t* ids, double* x, double* P, uint8_t* stage,
                                    float* ema, float* bank, int32_t* bank_len, int32_t* miss, int32_t* age,
                                    double* last_bbox, double* last_conf, double* last_cost, int32_t* next_id,
@@ -1894,15 +2034,14 @@ extern "C" int b200_tracker_export(b200_tracker* t, int stream_idx, int32_t* ids
     B200_REQUIRE(stream_idx >= 0 && stream_idx < d.S, "tracker_export: stream %d out of range", stream_idx);
     cudaStream_t st = as_stream(stream);
     const size_t MT = d.MT, H = d.HIST;
-    // staging buffer: the stream's live tracks packed in ascending track id
-    int *s_ids, *s_bl, *s_miss, *s_age;
-    double *s_x, *s_P, *s_lb, *s_lc, *s_lk;
-    uint8_t* s_stage;
-    float *s_ema, *s_bank;
+    // staging buffer: a one-row image of the stream, cap = max_tracks
+    b200_tracker_state s{};
+    s.n_rows = 1; s.cap = d.MT; s.hist_max = d.HIST;
     auto carve = [&](trk::Carver& c) {
-        c.take(s_ids, MT); c.take(s_x, MT * 8); c.take(s_P, MT * 64); c.take(s_stage, MT); c.take(s_ema, MT * 128);
-        c.take(s_bank, MT * H * 128); c.take(s_bl, MT); c.take(s_miss, MT); c.take(s_age, MT); c.take(s_lb, MT * 4);
-        c.take(s_lc, MT); c.take(s_lk, MT);
+        c.take(s.n_live, 2); s.next_id = s.n_live + 1;
+        c.take(s.ids, MT); c.take(s.x, MT * 8); c.take(s.P, MT * 64); c.take(s.stage, MT); c.take(s.ema, MT * 128);
+        c.take(s.bank, MT * H * 128); c.take(s.bank_len, MT); c.take(s.miss, MT); c.take(s.age, MT); c.take(s.last_bbox, MT * 4);
+        c.take(s.last_conf, MT); c.take(s.last_cost, MT);
     };
     trk::Carver size;
     carve(size);
@@ -1910,20 +2049,19 @@ extern "C" int b200_tracker_export(b200_tracker* t, int stream_idx, int32_t* ids
     B200_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&buf), size.off, st));
     trk::Carver c{buf};
     carve(c);
-    trk::export_kernel<<<d.MT < 256 ? d.MT : 256, 128, 0, st>>>(d, stream_idx, s_ids, s_x, s_P, s_stage, s_ema, s_bank, s_bl,
-                                                                 s_miss, s_age, s_lb, s_lc, s_lk);
-    int rc = check_launch("trk export_kernel");
+    trk::export_state_kernel<<<image_grid(s), trk::kStateWarps * 32, 0, st>>>(d, s, nullptr, stream_idx, nullptr);
+    int rc = check_launch("trk export_state_kernel");
     if (rc) return rc;
-    int hdr[trk::kHdr];
-    B200_CUDA(cudaMemcpyAsync(hdr, d.hdr + stream_idx * trk::kHdr, sizeof(hdr), cudaMemcpyDeviceToHost, st));
+    int hdr[2];
+    B200_CUDA(cudaMemcpyAsync(hdr, s.n_live, sizeof(hdr), cudaMemcpyDeviceToHost, st));
     B200_CUDA(cudaStreamSynchronize(st));
-    const size_t n = hdr[trk::H_NLIVE];
+    const size_t n = hdr[0];
 #define PULL(dst, src, per) if (dst && n) B200_CUDA(cudaMemcpyAsync(dst, src, sizeof(*src) * (per) * n, cudaMemcpyDeviceToHost, st))
-    PULL(ids, s_ids, 1); PULL(x, s_x, 8); PULL(P, s_P, 64); PULL(stage, s_stage, 1); PULL(ema, s_ema, 128);
-    PULL(bank, s_bank, H * 128); PULL(bank_len, s_bl, 1); PULL(miss, s_miss, 1); PULL(age, s_age, 1);
-    PULL(last_bbox, s_lb, 4); PULL(last_conf, s_lc, 1); PULL(last_cost, s_lk, 1);
+    PULL(ids, s.ids, 1); PULL(x, s.x, 8); PULL(P, s.P, 64); PULL(stage, s.stage, 1); PULL(ema, s.ema, 128);
+    PULL(bank, s.bank, H * 128); PULL(bank_len, s.bank_len, 1); PULL(miss, s.miss, 1); PULL(age, s.age, 1);
+    PULL(last_bbox, s.last_bbox, 4); PULL(last_conf, s.last_conf, 1); PULL(last_cost, s.last_cost, 1);
 #undef PULL
-    if (next_id) *next_id = hdr[trk::H_NEXT];
+    if (next_id) *next_id = hdr[1];
     B200_CUDA(cudaStreamSynchronize(st));
     B200_CUDA(cudaFreeAsync(buf, st));
     return (int)n;

@@ -102,14 +102,122 @@ class MultiStreamTracker:
         self.stride = _lib.lib().b200_tracker_result_stride(h)
 
     def grow(self, max_tracks: Optional[int] = None, max_dets: Optional[int] = None):
-        """Migrates every stream's state into a handle with larger capacities (export -> create -> import)."""
+        """Migrates every stream's state into a handle with larger capacities, on the device: ``state_dict()`` -> a new
+        handle -> import.  If the larger handle cannot be created the tracker is left as it was.  Live counts do not
+        change.  A CUDA graph captured before a growth holds the old handle's buffers: capture it again."""
         self.drain()
-        snaps = [self.export(s) for s in range(self.S)]
-        old = self._h
+        sd = self.state_dict()
+        old = (self._h, self.max_tracks, self.max_dets, self.stride)
         self._create(max(self.max_tracks, int(max_tracks or 0)), max(self.max_dets, int(max_dets or 0)))
-        _lib.lib().b200_tracker_destroy(old)
-        for s, snap in enumerate(snaps):
-            self.import_state(s, snap)
+        try:
+            status = self._import(sd, None)            # reads the status back: the import has completed
+            bad = np.nonzero(status)[0]
+            if len(bad):
+                raise _lib.B200Error("grow: stream %d failed to migrate (status %d)" % (bad[0], status[bad[0]]))
+        except BaseException:
+            _lib.lib().b200_tracker_destroy(self._h)
+            self._h, self.max_tracks, self.max_dets, self.stride = old
+            raise
+        _lib.lib().b200_tracker_destroy(old[0])
+
+    # -- device-side state images (b200_tracker_state, layout _lib.STATE_LAYOUT) ----------------------------------
+    def _stream_index(self, streams, what, distinct):
+        """-> (host int64 indices, device int32 tensor, or None for every stream in order)."""
+        if streams is None:
+            return np.arange(self.S), None
+        idx = np.asarray(streams.cpu() if isinstance(streams, torch.Tensor) else streams, dtype=np.int64).reshape(-1)
+        if len(idx) and (idx.min() < 0 or idx.max() >= self.S):
+            raise ValueError("%s: stream index out of range [0, %d)" % (what, self.S))
+        if distinct and len(np.unique(idx)) != len(idx):
+            raise ValueError("%s: duplicate stream index" % what)
+        return idx, torch.as_tensor(idx, dtype=torch.int32).to(self.device)
+
+    def _new_image(self, rows: int, cap: int) -> Dict[str, torch.Tensor]:
+        dims = dict(cap=cap, hist_max=self.conf["hist_max"])
+        return {n: torch.zeros((rows,) + tuple(dims.get(k, k) for k in shape), dtype=getattr(torch, dt), device=self.device)
+                for n, dt, shape in _lib.STATE_LAYOUT}
+
+    @staticmethod
+    def _c_image(sd):
+        im = _lib.tracker_state()
+        for n, _, _ in _lib.STATE_LAYOUT:
+            setattr(im, n, sd[n].data_ptr())
+        im.n_rows, im.cap, im.hist_max = sd["n_live"].shape[0], sd["ids"].shape[1], sd["bank"].shape[2]
+        return im
+
+    def _import(self, sd, dev_idx, read_status=True):
+        """b200_tracker_import_device on the current stream; returns the per-row status (synchronises) or None."""
+        status = torch.empty(sd["n_live"].shape[0], dtype=torch.int32, device=self.device) if read_status else None
+        im = self._c_image(sd)
+        with torch.cuda.device(self.device):
+            rc = _lib.lib().b200_tracker_import_device(self._h, _lib.ptr(dev_idx), ctypes.byref(im), _lib.ptr(status),
+                                                       _lib.stream_ptr(self.device))
+        _lib.check(rc)
+        return status.cpu().numpy() if read_status else None
+
+    def state_dict(self, streams=None) -> Dict[str, torch.Tensor]:
+        """The state of ``streams`` (a list or tensor of stream indices; None = every stream, in order) as device tensors,
+        one row per stream: ``n_live`` / ``next_id`` [R] int32 and the live tracks of each row in ascending track id,
+        in ``export``'s layout with ``cap = max_tracks`` slots per row (``ids`` [R, cap], ``bank`` [R, cap, hist_max,
+        128], ...; slots past ``n_live`` are zero).  Asynchronous on the current stream, no read-back: ``torch.save``
+        it, ``load_state_dict`` it into another tracker, or capture it in a CUDA graph."""
+        self.drain()
+        idx, dev_idx = self._stream_index(streams, "state_dict", distinct=False)
+        sd = self._new_image(len(idx), self.max_tracks)
+        if len(idx):
+            im = self._c_image(sd)
+            with torch.cuda.device(self.device):
+                rc = _lib.lib().b200_tracker_export_device(self._h, _lib.ptr(dev_idx), ctypes.byref(im), None,
+                                                           _lib.stream_ptr(self.device))
+            _lib.check(rc)
+        return sd
+
+    def load_state_dict(self, sd: Dict[str, torch.Tensor], streams=None):
+        """Replaces the state of ``streams`` (distinct indices; None = every stream, in order) by the rows of ``sd``, an
+        image as ``state_dict`` returns it (any ``cap``, tensors on any device).  The image carries state, not
+        configuration: hyper-parameters stay this tracker's own, and ``hist_max`` must be equal (ValueError).  A row with
+        more than ``max_tracks`` tracks grows the handle (``auto_grow``) or raises B200Error before anything changes.  A
+        malformed row raises B200Error naming its stream; the other rows are applied."""
+        self.drain()
+        want = {n: (getattr(torch, dt), shape) for n, dt, shape in _lib.STATE_LAYOUT}
+        if set(sd) != set(want):
+            raise ValueError("load_state_dict: keys must be %s" % sorted(want))
+        sd = {n: torch.as_tensor(v) for n, v in sd.items()}
+        for n, (dt, _) in want.items():
+            if sd[n].dtype != dt:
+                raise TypeError("load_state_dict: %s must be %s, got %s" % (n, dt, sd[n].dtype))
+        if sd["ids"].dim() != 2 or sd["bank"].dim() != 4:
+            raise ValueError("load_state_dict: ids must be [R, cap] and bank [R, cap, hist_max, 128]")
+        R, cap, H = sd["ids"].shape[0], sd["ids"].shape[1], sd["bank"].shape[2]
+        if H != self.conf["hist_max"]:
+            raise ValueError("load_state_dict: image hist_max %d, tracker hist_max %d" % (H, self.conf["hist_max"]))
+        dims = dict(cap=cap, hist_max=H)
+        for n, (_, shape) in want.items():
+            if tuple(sd[n].shape) != (R,) + tuple(dims.get(k, k) for k in shape):
+                raise ValueError("load_state_dict: %s has shape %s, inconsistent with ids %s" % (n, tuple(sd[n].shape), (R, cap)))
+        if streams is None and R != self.S:
+            raise ValueError("load_state_dict: %d rows for %d streams (pass streams=)" % (R, self.S))
+        idx, dev_idx = self._stream_index(streams, "load_state_dict", distinct=True)
+        if len(idx) != R:
+            raise ValueError("load_state_dict: %d rows, %d stream indices" % (R, len(idx)))
+        if R == 0:
+            return
+        n = sd["n_live"].cpu().numpy().astype(np.int64)
+        if int(n.max()) > self.max_tracks:
+            if not self.auto_grow:
+                raise _lib.B200Error("load_state_dict: %d tracks exceed max_tracks=%d; construct the tracker with a "
+                                     "larger max_tracks" % (int(n.max()), self.max_tracks))
+            self.grow(max_tracks=max(int(n.max()), 2 * self.max_tracks))
+        sd = {k: v.to(self.device).contiguous() for k, v in sd.items()}
+        status = self._import(sd, dev_idx)
+        ok = status == 0
+        self.n_live[idx[ok]] = n[ok]
+        bad = np.nonzero(~ok)[0]
+        if len(bad):
+            r = bad[0]
+            raise _lib.B200Error("load_state_dict: stream %d not loaded: %s" % (
+                idx[r], {_lib.EINVAL: "malformed image row", _lib.ECAPACITY: "more tracks than slots"}.get(
+                    int(status[r]), "status %d" % status[r])))
 
     def import_state(self, stream: int, snap: Dict[str, np.ndarray]):
         """Inverse of ``export`` for one stream."""
@@ -136,11 +244,20 @@ class MultiStreamTracker:
         except Exception:
             pass
 
-    def reset(self):
-        """Back to the state of ``Tracking.__init__`` (mainTracking.py:45-96): no tracks, next id 0, every stream."""
-        with torch.cuda.device(self.device):
-            _lib.check(_lib.lib().b200_tracker_reset(self._h, _lib.stream_ptr(self.device)))
-        self.n_live[:] = 0
+    def reset(self, streams=None):
+        """Back to the state of ``Tracking.__init__`` (mainTracking.py:45-96): no tracks, next id 0.  None: every
+        stream; a list of distinct stream indices: only those (a camera's video ended and a new one starts in the same
+        stream), the others untouched.  Asynchronous on the current stream."""
+        if streams is None:
+            with torch.cuda.device(self.device):
+                _lib.check(_lib.lib().b200_tracker_reset(self._h, _lib.stream_ptr(self.device)))
+            self.n_live[:] = 0
+            return
+        self.drain()
+        idx, dev_idx = self._stream_index(streams, "reset", distinct=True)
+        if len(idx):
+            self._import(self._new_image(len(idx), 1), dev_idx, read_status=False)   # empty rows: cannot fail
+            self.n_live[idx] = 0
 
     # -- one frame-step for every stream, host arrays in, host result table out -------------------
     def step(self, n_det, boxes, confs, embs, frame_ids) -> np.ndarray:
@@ -489,10 +606,7 @@ class Tracking:
         """Array form of ``update``: boxes [N,4] float64 xyxy, confs [N], embs [N,128] float32."""
         N = boxes.shape[0]
         self._reserve_dets(N)
-        MD = self._ms.max_dets
-        if self._boxes.shape[1] != MD:                 # the handle has grown (here or in one of the step-by-step methods)
-            self._boxes, self._confs = np.zeros((1, MD, 4), np.float64), np.zeros((1, MD), np.float64)
-            self._embs = np.zeros((1, MD, 128), np.float32)
+        self._fit_buffers()
         self._boxes[0, :N] = boxes
         self._confs[0, :N] = confs
         self._embs[0, :N] = embs
@@ -525,6 +639,23 @@ class Tracking:
         if err is not None:
             raise err
         return ms.decode(res[0])
+
+    def _fit_buffers(self):
+        MD = self._ms.max_dets
+        if self._boxes.shape[1] != MD:                 # the handle has grown (here or in one of the step-by-step methods)
+            self._boxes, self._confs = np.zeros((1, MD, 4), np.float64), np.zeros((1, MD), np.float64)
+            self._embs = np.zeros((1, MD, 128), np.float32)
+
+    def state_dict(self) -> Dict[str, torch.Tensor]:
+        """The tracker's state as device tensors (``MultiStreamTracker.state_dict`` of its one stream): ``torch.save`` it
+        and ``load_state_dict`` it into a fresh ``Tracking`` to continue the video where it stopped."""
+        return self._ms.state_dict()
+
+    def load_state_dict(self, sd: Dict[str, torch.Tensor]):
+        """Restores a ``state_dict`` (one row).  Hyper-parameters stay this tracker's own; ``hist_max`` must match."""
+        self._snap = None
+        self._ms.load_state_dict(sd)
+        self._fit_buffers()
 
     def _reserve_dets(self, n: int):
         """Grows the handle's ``max_dets`` to hold ``n`` detections (raises instead with ``auto_grow=False``)."""

@@ -267,13 +267,51 @@ int  b200_tracker_export(b200_tracker* t, int stream_idx, int32_t* ids, double* 
                          int32_t* next_id, void* stream);
 
 /* Inverse of b200_tracker_export: replaces one stream's state by `n` tracks given in ascending track-id
- * order (host arrays, same layouts as export).  Used to migrate state into a handle with larger
- * capacities -- the reference's Tracking is unbounded -- and to restore a saved tracker. */
+ * order (host arrays, same layouts as export).  b200_tracker_import_device below does the same for any
+ * set of streams from device memory without a synchronisation. */
 int  b200_tracker_import(b200_tracker* t, int stream_idx, int n, const int32_t* ids, const double* x,
                          const double* P, const uint8_t* stage, const float* ema, const float* bank,
                          const int32_t* bank_len, const int32_t* miss, const int32_t* age,
                          const double* last_bbox, const double* last_conf, const double* last_cost,
                          int32_t next_id, void* stream);
+
+/* Device-side image of the state of any set of streams: the layout of b200_tracker_export with a leading row
+ * dimension (n_rows rows of cap track slots; a row's live tracks first, ascending track id).  Every pointer is a
+ * device pointer; x, P, ema, bank and last_bbox must be 16-byte aligned. */
+typedef struct b200_tracker_state {
+    int32_t* n_live;        /* [n_rows] */
+    int32_t* next_id;       /* [n_rows] */
+    int32_t* ids;           /* [n_rows, cap] */
+    double*  x;             /* [n_rows, cap, 8] */
+    double*  P;             /* [n_rows, cap, 8, 8] */
+    uint8_t* stage;         /* [n_rows, cap] (0..2) */
+    float*   ema;           /* [n_rows, cap, 128] */
+    float*   bank;          /* [n_rows, cap, hist_max, 128], oldest row first */
+    int32_t* bank_len;      /* [n_rows, cap] */
+    int32_t* miss;          /* [n_rows, cap] */
+    int32_t* age;           /* [n_rows, cap] */
+    double*  last_bbox;     /* [n_rows, cap, 4] */
+    double*  last_conf;     /* [n_rows, cap] */
+    double*  last_cost;     /* [n_rows, cap] */
+    int32_t  n_rows, cap, hist_max;
+} b200_tracker_state;
+
+/* Image row r <-> handle stream streams[r] (device int32 [n_rows]; NULL = rows 0..S-1, then n_rows must be S).
+ * status: device int32 [n_rows] or NULL, B200_OK or why the row was skipped.  Both calls are asynchronous on
+ * `stream`, allocate nothing and never synchronise (capturable in a CUDA graph).
+ * export: writes n_live, next_id and the live tracks of each row, exactly what b200_tracker_export writes (bank rows
+ *   past bank_len zeroed); slots >= n_live are not touched.  B200_EINVAL: stream index outside [0,S);
+ *   B200_ECAPACITY: more than cap live tracks (nothing of the row is written).
+ * import: replaces each row's stream by the image and leaves the slot layout b200_tracker_import leaves, so the next
+ *   step is bit-identical to one after a host import.  A row is validated before anything is written and skipped,
+ *   its stream untouched, on: stream index outside [0,S) or named by another row, n_live < 0, ids not strictly
+ *   ascending or outside [0, next_id), bank_len outside [0, hist_max], stage > 2 (B200_EINVAL);
+ *   n_live > min(cap, max_tracks) (B200_ECAPACITY).  The image carries state only: hyper-parameters are the
+ *   handle's. */
+int  b200_tracker_export_device(b200_tracker* t, const int32_t* streams, const b200_tracker_state* img,
+                                int32_t* status, void* stream);
+int  b200_tracker_import_device(b200_tracker* t, const int32_t* streams, const b200_tracker_state* img,
+                                int32_t* status, void* stream);
 
 /* ---- result tables of all GPUs in one place, over NVLink peer memory (SURVEY.md section 8e) --------------------
  * The reference runs one inference process and hands every frame's matches to one consumer queue
