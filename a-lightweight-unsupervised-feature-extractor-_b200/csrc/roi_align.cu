@@ -22,16 +22,31 @@
 // the same operation order as torchvision and without FMA contraction so that cell
 // selection agrees with the CPU op.
 //
-// Kernels, by launch size (launch_tile):
-//   roi_align_tile_kernel    fewer than 16 384 tiles: steps 1-4 fused, one tile per warp (single-stream latency);
-//   roi_prep_kernel          large launches: step 1 once per ROI instead of once per channel tile, then
-//   roi_align_multi_kernel     NCHW / half / 7x7: the tile body with a warp walking eight tiles (next ROI record
-//                              loaded during the current tile, bulk-store wait deferred), or
-//   roi_align_pipe_kernel      channels-last float32: software pipeline over tiles with two footprint buffers
-//                              (16-byte cp.async.cg copies of tile n+1 while tile n accumulates);
-//   roi_align_generic_kernel other output sizes: one thread per output element.
+// Forward kernels (roi_align_dispatch -> launch_tile), for output sizes 10x10 and 7x7:
+//   roi_align_tile_kernel      fewer than 16 384 tiles or fewer than four channel tiles: steps 1-4 fused, one tile
+//                              per warp (single-stream latency);
+//   roi_prep_kernel            all other launches: step 1 once per ROI instead of once per channel tile, then the
+//                              first of these that applies:
+//   roi_align_tma_kernel         float32 NCHW map (tma_applies): the footprint arrives as TMA tensor boxes, a warp
+//                                walks 2-16 tiles with the next tile's boxes in flight;
+//   roi_align_pipe_kernel        channels-last map whose alignment allows it (launch_pipe): software pipeline over
+//                                tiles with two footprint buffers (16-byte cp.async.cg copies of tile n+1 while
+//                                tile n accumulates);
+//   roi_align_multi_kernel       everything else (half NCHW maps, alignments the two above cannot take): the tile body
+//                                with a warp walking eight tiles (next ROI record loaded during the current tile,
+//                                bulk-store wait deferred);
+//   roi_align_generic_kernel   other output sizes: one thread per output element.
 // Output is NCHW like the reference's, or channels-last on request (b200_roi_align_fwd_ex): lane = channel then
 // stores whole lines straight from the accumulators.
+//
+// Backward kernels (roi_align_bwd_dispatch -> launch_bwd; see "ROI Align backward" below), same output sizes:
+//   roi_align_bwd_tile_kernel  small launches as above: tables built per warp, scalar red.global.add per cell;
+//   roi_prep_kernel            all other launches, then
+//   roi_align_bwd_tma_kernel     float32 NCHW grad_in (tma_applies, 16-byte grad_out chunks): TMA reduce-add of
+//                                each tile's gradient boxes, followed by roi_align_bwd_tile_kernel for the tiles
+//                                roi_prep_kernel did not stage;
+//   roi_align_bwd_tile_kernel    otherwise (channels-last grad_in, alignment), with the prep records;
+//   roi_align_bwd_generic_kernel  other output sizes: one thread per grad_out element.
 #include <cuda.h>
 #include <cuda_fp16.h>
 
@@ -41,10 +56,11 @@
 namespace b200 {
 namespace {
 
-#ifndef B200_ROI_WARPS
-#define B200_ROI_WARPS 2
-#endif
-constexpr int kWarpsPerCta = B200_ROI_WARPS;
+// Launch shape of the tile, multi-tile and backward tile kernels.  This value, the CTAs per SM below and the tiles per
+// warp of the walking kernels were chosen by the sweeps in profiles/r01_roi_ncu_summary.md, r02_roi_ncu_summary.md and
+// r02_roi_variant_sweep_*.txt.
+constexpr int kWarpsPerCta = 2;
+constexpr int kMinCtasPerSm = 6;  // register cap of the tile / multi-tile / pipelined kernels: 5 and 7 are slower
 constexpr int kFootCap = 8;     // max footprint rows / cols on the staged path (<= 64 cells x 32 ch = 8 KB)
 constexpr int kCellCap = kFootCap * kFootCap;
 
@@ -134,10 +150,6 @@ __device__ __forceinline__ void axis_footprint(float start, float bin, int P, in
     *n = t1.hi - t0.lo + 1;
 }
 
-__device__ __forceinline__ void cp_async4(void* smem_dst, const void* gsrc) {
-    const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(d), "l"(gsrc) : "memory");
-}
 __device__ __forceinline__ void cp_async4_s(unsigned smem_addr, const void* gsrc) {     // shared-space address
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(smem_addr), "l"(gsrc) : "memory");
 }
@@ -152,29 +164,13 @@ __device__ __forceinline__ void cp_async_wait_all() {
 }
 
 // One bulk async copy shared -> global issued by a single lane (TMA engine, SASS UBLKCP).  The
-// source tile may be overwritten only after bulk_store_wait_read() on the issuing lane.
-// B200_ROI_L2_HINT: 0 = none; 1 = the output tiles (written once, never read by this library) leave with an L2 evict-first
-// policy; 2 = the footprint loads too.  ROI Align streams ~1 GB per 64-stream step through a 126 MB L2; without a hint
-// it evicts the tracker's banks and Kalman state between two association steps.
-#ifndef B200_ROI_L2_HINT
-#define B200_ROI_L2_HINT 0
-#endif
-__device__ __forceinline__ unsigned long long l2_evict_first_policy() {
-    unsigned long long pol;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;\n" : "=l"(pol));
-    return pol;
-}
+// source tile may be overwritten only after bulk_store_wait_read() on the issuing lane.  (An L2 evict-first hint on
+// these stores, and on the footprint loads, was measured neutral or slower: profiles/r02_l2_hint_sweep.txt.)
 __device__ __forceinline__ void bulk_store_issue(void* gdst, const void* ssrc, unsigned bytes) {
     const unsigned s = (unsigned)__cvta_generic_to_shared(ssrc);
-#if B200_ROI_L2_HINT >= 1
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;\n" ::"l"(gdst), "r"(s),
-                 "r"(bytes), "l"(l2_evict_first_policy())
-                 : "memory");
-#else
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;\n" ::"l"(gdst), "r"(s),
                  "r"(bytes)
                  : "memory");
-#endif
     asm volatile("cp.async.bulk.commit_group;\n" ::: "memory");
 }
 __device__ __forceinline__ void bulk_store_wait_read() {
@@ -307,9 +303,11 @@ roi_prep_kernel(const float* __restrict__ rois, long long K, int B, int H, int W
     }
 }
 
-#ifndef B200_ROI_MIN_CTAS
-#define B200_ROI_MIN_CTAS 6
-#endif
+// Slot of a launch's span in timing builds (B200_TRK_TIMING): the step index mod 8.  Only the B200_SPAN_* arguments
+// call it, so product builds do not evaluate it.
+[[maybe_unused]] __device__ __forceinline__ int span_slot(const float* rois, long long K) {
+    return (int)((reinterpret_cast<uintptr_t>(rois) / (size_t)(K * 20)) & 7);
+}
 
 // One (ROI k, channels c0 .. c0+cn) tile, start to finish, by one warp.  sMain: L::kMainFloats floats (V staging /
 // big tables, later the output tile), sTab: L::kTabFloats floats; both private to the warp.
@@ -526,7 +524,7 @@ __device__ __forceinline__ void process_tile(const T* __restrict__ feat, int B, 
 }
 
 template <int PH, int PW, bool NHWC, typename T, bool PREP, bool OCL>
-__global__ void __launch_bounds__(kWarpsPerCta * 32, (B200_ROI_MIN_CTAS * 2 + kWarpsPerCta - 1) / kWarpsPerCta)
+__global__ void __launch_bounds__(kWarpsPerCta * 32, (kMinCtasPerSm * 2 + kWarpsPerCta - 1) / kWarpsPerCta)
 roi_align_tile_kernel(const T* __restrict__ feat, int B, int C, int H, int W,
                       const float* __restrict__ rois, long long K, float scale, int sr, int aligned,
                       T* __restrict__ out, int ctiles, const RoiPrep* __restrict__ prep,
@@ -537,15 +535,14 @@ roi_align_tile_kernel(const T* __restrict__ feat, int B, int C, int H, int W,
     // Warps are independent: no block-wide barriers anywhere below.
     const long long wi = (long long)blockIdx.x * kWarpsPerCta + warp;
     if (wi >= K * ctiles) return;
-    const int span_slot = (int)((reinterpret_cast<uintptr_t>(rois) / (size_t)(K * 20)) & 7);   // debug: step index mod 8
-    B200_SPAN_BEGIN(span_slot);
+    B200_SPAN_BEGIN(span_slot(rois, K));
     float* sMain = smem + (size_t)warp * L::kFloatsPerWarp;
     const unsigned wi32 = (unsigned)wi;       // the launcher keeps the tile count below 2^31
     const long long k = wi32 / (unsigned)ctiles;
     const int c0 = (int)(wi32 % (unsigned)ctiles) * 32;
     process_tile<PH, PW, NHWC, T, PREP, OCL>(feat, B, C, H, W, rois, scale, sr, aligned, out, k, c0, min(32, C - c0),
                                              prep, prep_tabs, sMain, sMain + L::kMainFloats, lane);
-    B200_SPAN_END(span_slot);
+    B200_SPAN_END(span_slot(rois, K));
 }
 
 // Large launches that cannot use the pipelined kernel below (NCHW maps, half storage, 7x7): the tile kernel with a
@@ -553,11 +550,9 @@ roi_align_tile_kernel(const T* __restrict__ feat, int B, int C, int H, int W,
 // tile and the wait for the output tile's bulk store moves behind the next tile's address arithmetic, which
 // takes two of the three exposed round trips off the critical path; tiles are handed out in groups the size of
 // the resident warp set as in the pipelined kernel.
-#ifndef B200_ROI_MULTI_TILES
-#define B200_ROI_MULTI_TILES 8
-#endif
+constexpr int kMultiTilesPerWarp = 8;
 template <int PH, int PW, bool NHWC, typename T, bool OCL>
-__global__ void __launch_bounds__(kWarpsPerCta * 32, (B200_ROI_MIN_CTAS * 2 + kWarpsPerCta - 1) / kWarpsPerCta)
+__global__ void __launch_bounds__(kWarpsPerCta * 32, (kMinCtasPerSm * 2 + kWarpsPerCta - 1) / kWarpsPerCta)
 roi_align_multi_kernel(const T* __restrict__ feat, int B, int C, int H, int W, const float* __restrict__ rois,
                        long long K, float scale, int sr, int aligned, T* __restrict__ out, int ctiles,
                        const RoiPrep* __restrict__ prep, const float* __restrict__ prep_tabs, int group_warps,
@@ -571,8 +566,7 @@ roi_align_multi_kernel(const T* __restrict__ feat, int B, int C, int H, int W, c
     const unsigned total = (unsigned)min((long long)(grp + 1) * window, K * ctiles);
     if (t >= total) return;
     asm volatile("griddepcontrol.wait;" ::: "memory");      // roi_prep_kernel's records and tables are complete and visible
-    const int span_slot = (int)((reinterpret_cast<uintptr_t>(rois) / (size_t)(K * 20)) & 7);   // debug: step index mod 8
-    B200_SPAN_BEGIN(span_slot);
+    B200_SPAN_BEGIN(span_slot(rois, K));
     float* sMain = smem + (size_t)warp * L::kFloatsPerWarp;
     unsigned k = t / (unsigned)ctiles;
     int4 h0 = reinterpret_cast<const int4*>(prep + k)[0], h1 = reinterpret_cast<const int4*>(prep + k)[1];
@@ -595,7 +589,7 @@ roi_align_multi_kernel(const T* __restrict__ feat, int B, int C, int H, int W, c
         t = tn; k = kn; h0 = n0; h1 = n1;
     }
     if (pending && lane == 0) bulk_store_wait_read();
-    B200_SPAN_END(span_slot);
+    B200_SPAN_END(span_slot(rois, K));
 }
 
 // ---- software-pipelined persistent kernel: large float32 launches -------------------------------------
@@ -611,10 +605,7 @@ roi_align_multi_kernel(const T* __restrict__ feat, int B, int C, int H, int W, c
 // instead of 232 us on the bench launch.)  Tiles whose footprint does not fit a buffer flush the pipeline
 // and go through process_tile() with the warp's whole shared-memory region.
 constexpr int kPipeWarps = 2;
-#ifndef B200_ROI_PIPE_TILES
-#define B200_ROI_PIPE_TILES 8
-#endif
-constexpr int kPipeTilesPerWarp = B200_ROI_PIPE_TILES;
+constexpr int kPipeTilesPerWarp = 8;
 
 template <int PH, int PW>
 struct PipeSmem {
@@ -670,7 +661,7 @@ __device__ __forceinline__ bool pipe_can_stage(const int4 rec1, bool vec16, int 
 }
 
 template <int PH, int PW, bool OCL, typename T>
-__global__ void __launch_bounds__(kPipeWarps * 32, (B200_ROI_MIN_CTAS * 2 + kPipeWarps - 1) / kPipeWarps)
+__global__ void __launch_bounds__(kPipeWarps * 32, (kMinCtasPerSm * 2 + kPipeWarps - 1) / kPipeWarps)
 roi_align_pipe_kernel(const T* __restrict__ feat, int B, int C, int H, int W, const float* __restrict__ rois,
                       long long K, float scale, int sr, int aligned, T* __restrict__ out, int ctiles,
                       const RoiPrep* __restrict__ prep, const float* __restrict__ prep_tabs, int group_warps,
@@ -694,8 +685,7 @@ roi_align_pipe_kernel(const T* __restrict__ feat, int B, int C, int H, int W, co
     const unsigned total = (unsigned)min((long long)(grp + 1) * window, K * ctiles);
     if (t >= total) return;
     asm volatile("griddepcontrol.wait;" ::: "memory");      // roi_prep_kernel's records and tables are complete and visible
-    const int span_slot = (int)((reinterpret_cast<uintptr_t>(rois) / (size_t)(K * 20)) & 7);   // debug: step index mod 8
-    B200_SPAN_BEGIN(span_slot);
+    B200_SPAN_BEGIN(span_slot(rois, K));
 
     // current tile (a*), next tile (n*): ROI index, first channel, prep record
     unsigned ka = t / (unsigned)ctiles;
@@ -816,7 +806,7 @@ roi_align_pipe_kernel(const T* __restrict__ feat, int B, int C, int H, int W, co
         tn = tm; kn = km; cnx = cm; n0 = m0; n1 = m1;
         par ^= 1;
     }
-    B200_SPAN_END(span_slot);
+    B200_SPAN_END(span_slot(rois, K));
 }
 
 
@@ -853,22 +843,9 @@ struct TmaMaps {                                           // the same map with 
     CUtensorMap m[3];
 };
 __device__ __forceinline__ int tma_box_rows(int rows) { return rows <= 1 ? 1 : rows <= 3 ? 3 : 5; }
-#ifndef B200_ROI_TMA_WARPS
-#define B200_ROI_TMA_WARPS 2
-#endif
-#ifndef B200_ROI_TMA_CTAS
-#define B200_ROI_TMA_CTAS 3
-#endif
-#ifndef B200_ROI_TMA_TILES
-#define B200_ROI_TMA_TILES 16
-#endif
-#ifndef B200_ROI_TMA_REGS
-#define B200_ROI_TMA_REGS 216
-#endif
-#ifndef B200_ROI_TMA_MAX_CTAS
-#define B200_ROI_TMA_MAX_CTAS 0
-#endif
-constexpr int kTmaWarps = B200_ROI_TMA_WARPS;
+// CTA shape and register cap of the TMA kernels (profiles/r02_roi_variant_sweep_*.txt, r02_roi_ncu_summary.md)
+constexpr int kTmaWarps = 2;
+constexpr int kTmaRegs = 216;
 
 template <int PH, int PW>
 struct TmaSmem {
@@ -897,13 +874,8 @@ __device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
         "DONE_%=:\n\t}\n" ::"r"(bar), "r"(parity) : "memory");
 }
 __device__ __forceinline__ void tma_box_4d(unsigned dst, const CUtensorMap* tm, int x, int y, int c, int b, unsigned bar) {
-#if B200_ROI_L2_HINT >= 2
-    asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%2, %3, %4, %5}], [%6], %7;\n"
-                 ::"r"(dst), "l"(tm), "r"(x), "r"(y), "r"(c), "r"(b), "r"(bar), "l"(l2_evict_first_policy()) : "memory");
-#else
     asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];\n"
                  ::"r"(dst), "l"(tm), "r"(x), "r"(y), "r"(c), "r"(b), "r"(bar) : "memory");
-#endif
 }
 __device__ __forceinline__ void bulk_load(unsigned dst, const void* src, unsigned bytes, unsigned bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];\n"
@@ -929,7 +901,7 @@ __device__ __forceinline__ int bcast0(int v) { return __shfl_sync(0xffffffffu, v
 // the whole (converged) warp; the operands are broadcast from lane 0 first so that they are provably warp-uniform and
 // go to the TMA instructions through uniform registers directly (with per-lane values ptxas wraps every UTMALDG /
 // UBLKCP in an ELECT / R2UR.BROADCAST loop, which showed up as 11 % of all stall samples).
-template <int PH, int PW, typename T>
+template <int PH, int PW>
 __device__ __forceinline__ void tma_issue(const TmaMaps* tm, const int4 h0, const int4 h1, unsigned k, int c0,
                                           const float* __restrict__ prep_tabs, unsigned sv, unsigned stab, unsigned bar) {
     using S = TmaSmem<PH, PW>;
@@ -941,15 +913,9 @@ __device__ __forceinline__ void tma_issue(const TmaMaps* tm, const int4 h0, cons
     const int r0 = FY > kTmaRows ? kTmaRows : tma_box_rows(FY);                 // rows of the first box
     const int r1 = FY > kTmaRows ? tma_box_rows(FY - kTmaRows) : 0;            // rows of the box below it
     if (elect_one()) {
-#ifdef B200_ROI_TMA_NOLOAD                       // timing experiment only (results are wrong): no footprint traffic
-        mbar_expect_tx(baru, (unsigned)S::kTabBytes);
-        bulk_load(stabu, prep_tabs + (size_t)ku * S::L::kTabFloats, S::kTabBytes, baru);
-        if (false) {
-#else
         mbar_expect_tx(baru, (unsigned)(S::kTabBytes + (any ? (r0 + r1) * kTmaRowBytes : 0)));
         bulk_load(stabu, prep_tabs + (size_t)ku * S::L::kTabFloats, S::kTabBytes, baru);
         if (any) {
-#endif
             tma_box_4d(svu, &tm->m[r0 >> 1], xmin, ymin, cu, b, baru);
             if (r1) tma_box_4d(svu + kTmaRows * kTmaRowBytes, &tm->m[r1 >> 1], xmin, ymin + kTmaRows, cu, b, baru);
         }
@@ -962,10 +928,9 @@ __device__ __forceinline__ void tma_issue(const TmaMaps* tm, const int4 h0, cons
 // footprint as zeros, never as map data); then, column-outer like separable_accumulate: for every column that
 // carries weight (one uniform test per column and box, not per row), ty[ph] = sum_r Wy[r][ph] * V[r][x] and
 // acc[ph][pw] += Wx[x][pw] * ty[ph].
-template <int PH, int PW, typename T>
+template <int PH, int PW>
 __device__ __forceinline__ void tma_accumulate(float (&acc)[PH][PW], const unsigned char* sV, const float* sWy,
                                                const float* sWx, int FY, int FX, int xmask, int lane) {
-    static_assert(sizeof(T) == 4, "float32 maps only");
     constexpr int PHP = (PH + 3) & ~3, PWP = (PW + 3) & ~3;
     const int nrb = FY > kTmaRows ? 2 : 1, ncb = FX > 4 ? 2 : 1;
     for (int rb = 0; rb < nrb; ++rb) {
@@ -1020,10 +985,10 @@ __device__ __forceinline__ void tma_accumulate(float (&acc)[PH][PW], const unsig
     }
 }
 
-template <int PH, int PW, typename T, bool OCL>
-__global__ void __maxnreg__(B200_ROI_TMA_REGS)
-roi_align_tma_kernel(const __grid_constant__ TmaMaps tmap, const T* __restrict__ feat, int B, int C, int H, int W,
-                     const float* __restrict__ rois, long long K, float scale, int sr, int aligned, T* __restrict__ out,
+template <int PH, int PW, bool OCL>
+__global__ void __maxnreg__(kTmaRegs)
+roi_align_tma_kernel(const __grid_constant__ TmaMaps tmap, const float* __restrict__ feat, int B, int C, int H, int W,
+                     const float* __restrict__ rois, long long K, float scale, int sr, int aligned, float* __restrict__ out,
                      int ctiles, const RoiPrep* __restrict__ prep, const float* __restrict__ prep_tabs, int group_warps,
                      int tiles_per_warp) {
     using L = TileSmem<PH, PW>;
@@ -1041,8 +1006,7 @@ roi_align_tma_kernel(const __grid_constant__ TmaMaps tmap, const T* __restrict__
     const unsigned total = (unsigned)min((long long)(grp + 1) * window, K * ctiles);
     if (t >= total) return;
     asm volatile("griddepcontrol.wait;" ::: "memory");      // roi_prep_kernel's records and tables are complete and visible
-    const int span_slot = (int)((reinterpret_cast<uintptr_t>(rois) / (size_t)(K * 20)) & 7);   // debug: step index mod 8
-    B200_SPAN_BEGIN(span_slot);
+    B200_SPAN_BEGIN(span_slot(rois, K));
     if (lane == 0) {
         mbar_init(sbar, 1);
         mbar_init(sbar + 8, 1);
@@ -1070,8 +1034,8 @@ roi_align_tma_kernel(const __grid_constant__ TmaMaps tmap, const T* __restrict__
     // V offset of a tile with `nb` boxes in slot p: slot 0 grows up from the start, slot 1 down from the end
     auto v_off = [&](int p, int nr) { return p ? (unsigned)(kTmaVBytes - nr * kTmaRowBytes) : 0u; };
     if (a1.y) {
-        tma_issue<PH, PW, T>(&tmap, a0, a1, ka, ca, prep_tabs, sbase + v_off(0, tma_tile_rows(a0, a1)),
-                             sbase + S::kOffTab, sbar);
+        tma_issue<PH, PW>(&tmap, a0, a1, ka, ca, prep_tabs, sbase + v_off(0, tma_tile_rows(a0, a1)),
+                          sbase + S::kOffTab, sbar);
         cur_issued = true;
     }
     for (;;) {
@@ -1082,8 +1046,8 @@ roi_align_tma_kernel(const __grid_constant__ TmaMaps tmap, const T* __restrict__
         // the next tile's footprint is requested now if it fits beside the current one, else once that is consumed
         bool next_issued = false;
         if (have_next && n1.y && nba + nbn <= kTmaVRows) {
-            tma_issue<PH, PW, T>(&tmap, n0, n1, kn, cnx, prep_tabs, sbase + v_off(par ^ 1, nbn),
-                                 sbase + S::kOffTab + (par ^ 1) * S::kTabBytes, sbar + 8 * (par ^ 1));
+            tma_issue<PH, PW>(&tmap, n0, n1, kn, cnx, prep_tabs, sbase + v_off(par ^ 1, nbn),
+                              sbase + S::kOffTab + (par ^ 1) * S::kTabBytes, sbar + 8 * (par ^ 1));
             next_issued = true;
         }
         // record of the tile after next: requested after the accumulation (register pressure), see roi_align_pipe_kernel
@@ -1101,8 +1065,8 @@ roi_align_tma_kernel(const __grid_constant__ TmaMaps tmap, const T* __restrict__
         };
         if (a1.y) {
             if (!cur_issued) {         // only when the previous iteration could not fit it beside its own tile
-                tma_issue<PH, PW, T>(&tmap, a0, a1, ka, ca, prep_tabs, sbase + v_off(par, nba),
-                                     sbase + S::kOffTab + par * S::kTabBytes, sbar + 8 * par);
+                tma_issue<PH, PW>(&tmap, a0, a1, ka, ca, prep_tabs, sbase + v_off(par, nba),
+                                  sbase + S::kOffTab + par * S::kTabBytes, sbar + 8 * par);
             }
             mbar_wait(sbar + 8 * par, (phase >> par) & 1u);
             phase ^= 1u << par;
@@ -1113,52 +1077,39 @@ roi_align_tma_kernel(const __grid_constant__ TmaMaps tmap, const T* __restrict__
             for (int a = 0; a < PH; ++a)
 #pragma unroll
                 for (int bq = 0; bq < PW; ++bq) acc[a][bq] = 0.0f;
-            if (nba) tma_accumulate<PH, PW, T>(acc, base + v_off(par, nba), sWy, sWy + kFootCap * PHP, FY, FX, a1.z, lane);
+            if (nba) tma_accumulate<PH, PW>(acc, base + v_off(par, nba), sWy, sWy + kFootCap * PHP, FY, FX, a1.z, lane);
             load_after_next();
             __syncwarp();              // V and the tables of this slot are dead
             if (have_next && n1.y && !next_issued && nbn <= kTmaVRows) {
-                tma_issue<PH, PW, T>(&tmap, n0, n1, kn, cnx, prep_tabs, sbase + v_off(par ^ 1, nbn),
-                                     sbase + S::kOffTab + (par ^ 1) * S::kTabBytes, sbar + 8 * (par ^ 1));
+                tma_issue<PH, PW>(&tmap, n0, n1, kn, cnx, prep_tabs, sbase + v_off(par ^ 1, nbn),
+                                  sbase + S::kOffTab + (par ^ 1) * S::kTabBytes, sbar + 8 * (par ^ 1));
                 next_issued = true;
             }
             if (OCL) {                 // channels-last result: full-line stores straight from the accumulators
-                T* gl = out + (size_t)ka * NB * C + ca + lane;
+                float* gl = out + (size_t)ka * NB * C + ca + lane;
                 if (lane < cn) {
 #pragma unroll
                     for (int a = 0; a < PH; ++a)
 #pragma unroll
-                        for (int bq = 0; bq < PW; ++bq) gl[(size_t)(a * PW + bq) * C] = from_f<T>(acc[a][bq]);
+                        for (int bq = 0; bq < PW; ++bq) gl[(size_t)(a * PW + bq) * C] = acc[a][bq];
                 }
             } else {
                 if (pending && lane == 0) bulk_store_wait_read();
                 pending = false;
                 __syncwarp();
-                if (sizeof(T) == 4) {
-                    float* myrow = sOut + lane * NB;
-                    if ((NB & 3) == 0) {
+                float* myrow = sOut + lane * NB;
+                if ((NB & 3) == 0) {
 #pragma unroll
-                        for (int q = 0; q < NB / 4; ++q)
-                            reinterpret_cast<float4*>(myrow)[q] =
-                                make_float4(acc[(4 * q) / PW][(4 * q) % PW], acc[(4 * q + 1) / PW][(4 * q + 1) % PW],
-                                            acc[(4 * q + 2) / PW][(4 * q + 2) % PW], acc[(4 * q + 3) / PW][(4 * q + 3) % PW]);
-                    } else {
-#pragma unroll
-                        for (int i = 0; i < NB; ++i) myrow[i] = acc[i / PW][i % PW];
-                    }
+                    for (int q = 0; q < NB / 4; ++q)
+                        reinterpret_cast<float4*>(myrow)[q] =
+                            make_float4(acc[(4 * q) / PW][(4 * q) % PW], acc[(4 * q + 1) / PW][(4 * q + 1) % PW],
+                                        acc[(4 * q + 2) / PW][(4 * q + 2) % PW], acc[(4 * q + 3) / PW][(4 * q + 3) % PW]);
                 } else {
-                    __half* myrow = reinterpret_cast<__half*>(sOut) + lane * NB;
-                    if ((NB & 1) == 0) {
 #pragma unroll
-                        for (int q = 0; q < NB / 2; ++q)
-                            reinterpret_cast<__half2*>(myrow)[q] = __floats2half2_rn(acc[(2 * q) / PW][(2 * q) % PW],
-                                                                                     acc[(2 * q + 1) / PW][(2 * q + 1) % PW]);
-                    } else {
-#pragma unroll
-                        for (int i = 0; i < NB; ++i) myrow[i] = __float2half_rn(acc[i / PW][i % PW]);
-                    }
+                    for (int i = 0; i < NB; ++i) myrow[i] = acc[i / PW][i % PW];
                 }
-                T* gdst = out + ((size_t)ka * C + ca) * NB;
-                const unsigned bytes = (unsigned)cn * NB * (unsigned)sizeof(T);
+                float* gdst = out + ((size_t)ka * C + ca) * NB;
+                const unsigned bytes = (unsigned)cn * NB * 4u;
                 if (((reinterpret_cast<uintptr_t>(gdst) & 15) == 0) && (bytes & 15u) == 0) {
                     asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");
                     __syncwarp();
@@ -1166,22 +1117,21 @@ roi_align_tma_kernel(const __grid_constant__ TmaMaps tmap, const T* __restrict__
                     pending = true;
                 } else {
                     __syncwarp();
-                    const T* tile = reinterpret_cast<const T*>(sOut);
-                    for (int i = lane; i < cn * NB; i += 32) gdst[i] = tile[i];
+                    for (int i = lane; i < cn * NB; i += 32) gdst[i] = sOut[i];
                     __syncwarp();
                 }
             }
         } else {
             // footprint larger than the staged path: everything through the generic tile body, the output tile as scratch
-            process_tile<PH, PW, false, T, true, OCL, true>(feat, B, C, H, W, rois, scale, sr, aligned, out, (long long)ka, ca,
-                                                            cn, prep, prep_tabs, sOut,
-                                                            reinterpret_cast<float*>(base + S::kOffTab + par * S::kTabBytes),
-                                                            lane, a0, a1, &pending);
+            process_tile<PH, PW, false, float, true, OCL, true>(feat, B, C, H, W, rois, scale, sr, aligned, out, (long long)ka,
+                                                                ca, cn, prep, prep_tabs, sOut,
+                                                                reinterpret_cast<float*>(base + S::kOffTab + par * S::kTabBytes),
+                                                                lane, a0, a1, &pending);
             load_after_next();
             __syncwarp();
             if (have_next && n1.y && !next_issued && nbn <= kTmaVRows) {
-                tma_issue<PH, PW, T>(&tmap, n0, n1, kn, cnx, prep_tabs, sbase + v_off(par ^ 1, nbn),
-                                     sbase + S::kOffTab + (par ^ 1) * S::kTabBytes, sbar + 8 * (par ^ 1));
+                tma_issue<PH, PW>(&tmap, n0, n1, kn, cnx, prep_tabs, sbase + v_off(par ^ 1, nbn),
+                                  sbase + S::kOffTab + (par ^ 1) * S::kTabBytes, sbar + 8 * (par ^ 1));
                 next_issued = true;
             }
         }
@@ -1192,7 +1142,7 @@ roi_align_tma_kernel(const __grid_constant__ TmaMaps tmap, const T* __restrict__
         par ^= 1;
     }
     if (pending && lane == 0) bulk_store_wait_read();
-    B200_SPAN_END(span_slot);
+    B200_SPAN_END(span_slot(rois, K));
 }
 
 // Any output size / any parameters: one thread per output element, direct sampling.
@@ -1248,19 +1198,40 @@ inline int device_ordinal() {
     return dev;
 }
 
-// Warps of `kern` the current device holds at once (and the shared-memory opt-in, once per device).
-template <typename Kern>
-int resident_warps_of(Kern kern, int (&cache)[kMaxDevices], int warps_per_cta, int smem_bytes, int* out) {
+// Warps of Kern the current device holds at once (and the shared-memory opt-in, once per device).
+template <auto Kern>
+int resident_warps_of(int warps_per_cta, int smem_bytes, int* out) {
+    static int cache[kMaxDevices];
     const int dev = device_ordinal();
     if (!cache[dev]) {
         int sms = 0, per_sm = 0;
         B200_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-        B200_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
-        B200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, warps_per_cta * 32, smem_bytes));
+        B200_CUDA(cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+        B200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, Kern, warps_per_cta * 32, smem_bytes));
         cache[dev] = sms * (per_sm > 0 ? per_sm : 1) * warps_per_cta;
     }
     *out = cache[dev];
     return B200_OK;
+}
+
+// Warps a launch of the walking kernels (multi-tile, pipelined, TMA) needs: they are taken in groups of `resident`
+// (what the device holds at once), each group covering a window of resident * tiles_per_warp consecutive tiles; the
+// last window may need fewer warps than a group.
+long long walker_warps(long long tiles, int resident, int tiles_per_warp) {
+    const long long window = (long long)resident * tiles_per_warp;
+    const long long groups = (tiles + window - 1) / window;
+    const long long last = tiles - (groups - 1) * window;                 // tiles in the last window
+    return (groups - 1) * resident + (last < resident ? last : resident);
+}
+
+// Tiles per warp of the TMA kernels, both directions: 16 amortise a warp's start-up (mbarrier init, first un-overlapped
+// load) best, but a warp that walks 16 tiles lives ~60 us; a launch of only a few waves (8 streams of BASELINE config 5:
+// 16 384 tiles) would then hold every SM slot from start to end and the association kernels of the other stream could
+// not start beside it.  Keep at least four waves of warps, and never fewer than 2 tiles per warp.
+constexpr int kTmaMaxTilesPerWarp = 16;
+int tma_tiles_per_warp(long long tiles, int resident) {
+    const long long tpw = tiles / ((long long)resident * 4);
+    return (int)(tpw < 2 ? 2 : tpw > kTmaMaxTilesPerWarp ? kTmaMaxTilesPerWarp : tpw);
 }
 
 // cuTensorMapEncodeTiled through the runtime's driver entry point (no link-time dependency on libcuda).
@@ -1280,6 +1251,61 @@ EncodeTiledFn encode_tiled_fn() {
     return reinterpret_cast<EncodeTiledFn>(fn);
 }
 
+// The TMA kernels apply to float32 NCHW tensors whose rows are a multiple of 16 bytes (the tensor map's stride rule) with
+// a 16-byte aligned base and dimensions inside the descriptor's limits.  (Half maps would need a 16-column window: not
+// built, they stay on the multi-tile kernel.)
+bool tma_applies(const float* map, int C, int H, int W) {
+    if (((size_t)W * 4) % 16 || (reinterpret_cast<uintptr_t>(map) & 15)) return false;
+    if ((unsigned long long)C * H * W * 4 >= (1ull << 40)) return false;
+    return encode_tiled_fn() != nullptr;
+}
+constexpr int kTmaXAlign = 4;                    // cells per 16 bytes of a float32 map row
+
+// The three tensor maps of the TMA kernels over a float32 [B,C,H,W] tensor: boxes of kTmaCols cells x 1 / 3 / 5 rows x
+// 32 channels.  False if the driver refuses one.
+bool encode_box_maps(const float* map, int B, int C, int H, int W, TmaMaps* out) {
+    EncodeTiledFn encode = encode_tiled_fn();
+    if (!encode) return false;
+    const cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)C, (cuuint64_t)B};
+    const cuuint64_t strides[3] = {(cuuint64_t)W * 4, (cuuint64_t)H * W * 4, (cuuint64_t)C * H * W * 4};
+    const cuuint32_t estr[4] = {1u, 1u, 1u, 1u};
+    for (int i = 0; i < 3; ++i) {
+        const cuuint32_t box[4] = {(cuuint32_t)kTmaCols, (cuuint32_t)(2 * i + 1), 32u, 1u};
+        const CUresult r = encode(&out->m[i], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(map), dims, strides,
+                                  box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                                  CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) return false;
+    }
+    return true;
+}
+
+// Below this many tiles one fused kernel is faster (the prep kernel costs a dependent launch); above it the
+// per-ROI work is done once by roi_prep_kernel and shared by the ROI's channel tiles.
+constexpr long long kPrepMinTiles = 16384;
+
+// The two-kernel path of both directions: roi_prep_kernel fills stream-ordered scratch (K records + K tables), then
+// `consume(prep, tabs)` launches the kernels that read it, then the scratch is freed behind them.  Returns the first
+// error, else what `consume` returns.
+template <int PH, int PW, typename Consume>
+int with_prep(const float* rois, long long K, int B, int H, int W, float scale, int sr, int aligned, int xalign,
+              cudaStream_t st, Consume consume) {
+    using L = TileSmem<PH, PW>;
+    cudaMemPool_t pool = nullptr;
+    int rc = scratch_pool(&pool);
+    if (rc) return rc;
+    char* ws = nullptr;
+    const size_t rec = (size_t)K * sizeof(RoiPrep), tab = (size_t)K * L::kTabFloats * sizeof(float);
+    B200_CUDA(cudaMallocFromPoolAsync(reinterpret_cast<void**>(&ws), rec + tab, pool, st));
+    RoiPrep* prep = reinterpret_cast<RoiPrep*>(ws);
+    float* tabs = reinterpret_cast<float*>(ws + rec);
+    roi_prep_kernel<PH, PW><<<(unsigned)((K + 3) / 4), 128, 0, st>>>(rois, K, B, H, W, scale, sr, aligned, prep, tabs,
+                                                                     xalign);
+    rc = check_launch("roi_prep_kernel");
+    if (rc == B200_OK) rc = consume(prep, tabs);
+    B200_CUDA(cudaFreeAsync(ws, st));
+    return rc;
+}
+
 // The tile kernels that follow roi_prep_kernel in the stream are launched as its programmatic dependents (launch_ex with
 // pdl): they become resident while the prep kernel still runs and wait for it with griddepcontrol.wait before they read a
 // record (-1.8 us per launch).  Measured A/B on the overlapped 64-stream step (profiles/r02_roi_pdl_ab.txt): channels-last
@@ -1287,71 +1313,27 @@ EncodeTiledFn encode_tiled_fn() {
 // chain's first kernel, released by the same event a few microseconds later, would otherwise get first -- so the TMA
 // kernel stays an ordinary launch.
 
-// Launches the TMA-staged kernel when it applies: NCHW map whose rows are a multiple of 16 bytes (the tensor map's
-// stride rule), 16-byte aligned base, dimensions inside the descriptor's limits.  Returns 1 when it does not.
-// The TMA-staged kernel applies to float32 NCHW maps whose rows are a multiple of 16 bytes (the tensor map's stride
-// rule) with a 16-byte aligned base and dimensions inside the descriptor's limits.  (Half maps would need a
-// 16-column window: not built, they stay on the multi-tile kernel.)
-template <typename T>
-bool tma_applies(const T* feat, int C, int H, int W) {
-    if (sizeof(T) != 4) return false;
-    if (((size_t)W * sizeof(T)) % 16 || (reinterpret_cast<uintptr_t>(feat) & 15)) return false;
-    if ((unsigned long long)C * H * W * sizeof(T) >= (1ull << 40)) return false;
-    return encode_tiled_fn() != nullptr;
-}
-constexpr int kTmaXAlign = 4;                    // cells per 16 bytes of a float32 map row
-
-template <int PH, int PW, bool OCL, typename T>
-int launch_tma(const T* feat, int B, int C, int H, int W, const float* rois, long long K, float scale, int sr, int aligned,
-               T* out, int ctiles, const RoiPrep* prep, const float* tabs, long long tiles, cudaStream_t st) {
-    using S = TmaSmem<PH, PW>;
-    constexpr int kEs = (int)sizeof(T);
-    if (reinterpret_cast<uintptr_t>(tabs) & 15) return 1;
-    EncodeTiledFn encode = encode_tiled_fn();
-    if (!encode) return 1;
+// Launches the TMA-staged kernel (the caller has checked tma_applies); returns 1 when it cannot.
+template <int PH, int PW, bool OCL>
+int launch_tma(const float* feat, int B, int C, int H, int W, const float* rois, long long K, float scale, int sr,
+               int aligned, float* out, int ctiles, const RoiPrep* prep, const float* tabs, long long tiles,
+               cudaStream_t st) {
+    constexpr int smem_bytes = TmaSmem<PH, PW>::kBytesPerCta;
     TmaMaps tmap;
-    const cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)C, (cuuint64_t)B};
-    const cuuint64_t strides[3] = {(cuuint64_t)W * kEs, (cuuint64_t)H * W * kEs, (cuuint64_t)C * H * W * kEs};
-    const cuuint32_t estr[4] = {1u, 1u, 1u, 1u};
-    for (int i = 0; i < 3; ++i) {                // boxes of 1, 3 and 5 rows
-        const cuuint32_t box[4] = {(cuuint32_t)kTmaCols, (cuuint32_t)(2 * i + 1), 32u, 1u};
-        const CUresult r = encode(&tmap.m[i], kEs == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4,
-                                  const_cast<T*>(feat), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                                  CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return 1;
-    }
-    static int cache[kMaxDevices];               // per instantiation and device
-    auto kern = roi_align_tma_kernel<PH, PW, T, OCL>;
+    if ((reinterpret_cast<uintptr_t>(tabs) & 15) || !encode_box_maps(feat, B, C, H, W, &tmap)) return 1;
+    constexpr auto kern = roi_align_tma_kernel<PH, PW, OCL>;
     int resident = 0;
-    // B200_ROI_TMA_MAX_CTAS > 0 caps the CTAs an SM holds by asking for more dynamic shared memory than the kernel uses, so
-    // that registers and shared memory stay free for kernels of other streams (the association chain).
-    int smem_bytes = S::kBytesPerCta;
-    if (B200_ROI_TMA_MAX_CTAS > 0 && smem_bytes < 233472 / (B200_ROI_TMA_MAX_CTAS + 1) + 256)
-        smem_bytes = 233472 / (B200_ROI_TMA_MAX_CTAS + 1) + 256;
-    const int rc = resident_warps_of(kern, cache, kTmaWarps, smem_bytes, &resident);
+    const int rc = resident_warps_of<kern>(kTmaWarps, smem_bytes, &resident);
     if (rc) return rc;
-    // Tiles per warp: 16 amortise a warp's start-up (mbarrier init, first un-overlapped load) best, but a warp that walks
-    // 16 tiles lives ~60 us; a launch of only a few waves (8 streams of BASELINE config 5: 16 384 tiles) would then hold
-    // every SM slot from start to end and the association kernels of the other stream could not start beside it.  Keep
-    // at least four waves of warps, and never fewer than 2 tiles per warp.
-    long long tpw = tiles / ((long long)resident * 4);
-    tpw = tpw < 2 ? 2 : tpw > B200_ROI_TMA_TILES ? B200_ROI_TMA_TILES : tpw;
-    const long long window = (long long)resident * tpw;
-    const long long groups = (tiles + window - 1) / window;
-    const long long last = tiles - (groups - 1) * window;
-    const long long warps = (groups - 1) * resident + (last < resident ? last : resident);
+    const int tpw = tma_tiles_per_warp(tiles, resident);
+    const long long warps = walker_warps(tiles, resident, tpw);
     launch_ex(kern, dim3((unsigned)((warps + kTmaWarps - 1) / kTmaWarps)), dim3(kTmaWarps * 32), (size_t)smem_bytes, st, false, 0,
-              tmap, feat, B, C, H, W, rois, K, scale, sr, aligned, out, ctiles, prep, tabs, resident, (int)tpw);
+              tmap, feat, B, C, H, W, rois, K, scale, sr, aligned, out, ctiles, prep, tabs, resident, tpw);
     return check_launch("roi_align_tma_kernel");
 }
 
-// Below this many tiles one fused kernel is faster (the prep kernel costs a dependent launch); above it the
-// per-ROI work is done once by roi_prep_kernel and shared by the ROI's channel tiles.
-constexpr long long kPrepMinTiles = 16384;
-
-// Launches the pipelined kernel when it applies (channels-last float32 map, PH*PW a multiple of 4, 16-byte
-// aligned output);
-// returns 1 when it does not.
+// Launches the pipelined kernel when it applies (channels-last map; NCHW output needs 16-byte rows of a lane's result
+// and a 16-byte aligned base; half maps need 16-byte copies); returns 1 when it does not.
 template <int PH, int PW, bool NHWC, bool OCL, typename T>
 int launch_pipe(const T* feat, int B, int C, int H, int W, const float* rois, long long K, float scale, int sr,
                 int aligned, T* out, int ctiles, const RoiPrep* prep, const float* tabs, long long tiles,
@@ -1363,15 +1345,11 @@ int launch_pipe(const T* feat, int B, int C, int H, int W, const float* rois, lo
         using P = PipeSmem<PH, PW>;
         if (!OCL && ((reinterpret_cast<uintptr_t>(out) & 15) || (sizeof(T) == 2 && (C & 1)))) return 1;
         if (sizeof(T) == 2 && ((C & 7) || (reinterpret_cast<uintptr_t>(feat) & 15))) return 1;   // half: 16-byte copies only
-        static int cache[kMaxDevices];       // warps the device holds at once (per instantiation and device)
-        auto kern = roi_align_pipe_kernel<PH, PW, OCL, T>;
+        constexpr auto kern = roi_align_pipe_kernel<PH, PW, OCL, T>;
         int resident_warps = 0;
-        const int rcw = resident_warps_of(kern, cache, kPipeWarps, P::kBytesPerCta, &resident_warps);
+        const int rcw = resident_warps_of<kern>(kPipeWarps, P::kBytesPerCta, &resident_warps);
         if (rcw) return rcw;
-        const long long window = (long long)resident_warps * kPipeTilesPerWarp;
-        const long long groups = (tiles + window - 1) / window;
-        const long long last = tiles - (groups - 1) * window;                 // tiles in the last window
-        const long long warps = (groups - 1) * resident_warps + (last < resident_warps ? last : resident_warps);
+        const long long warps = walker_warps(tiles, resident_warps, kPipeTilesPerWarp);
         launch_ex(kern, dim3((unsigned)((warps + kPipeWarps - 1) / kPipeWarps)), dim3(kPipeWarps * 32), (size_t)P::kBytesPerCta, st,
                   true, 0, feat, B, C, H, W, rois, K, scale, sr, aligned, out, ctiles, prep, tabs, resident_warps,
                   (int)kPipeTilesPerWarp);
@@ -1401,43 +1379,70 @@ int launch_tile(const T* feat, int B, int C, int H, int W, const float* rois, lo
                                                                             aligned, out, ctiles, nullptr, nullptr);
         return check_launch("roi_align_tile_kernel");
     }
-    cudaMemPool_t pool = nullptr;
-    int rc = scratch_pool(&pool);
-    if (rc) return rc;
-    char* ws = nullptr;                      // stream-ordered scratch: K records + K tables
-    const size_t rec = (size_t)K * sizeof(RoiPrep), tab = (size_t)K * L::kTabFloats * sizeof(float);
-    B200_CUDA(cudaMallocFromPoolAsync(reinterpret_cast<void**>(&ws), rec + tab, pool, st));
-    RoiPrep* prep = reinterpret_cast<RoiPrep*>(ws);
-    float* tabs = reinterpret_cast<float*>(ws + rec);
+    constexpr bool kTmaLayout = !NHWC && std::is_same_v<T, float>;
     bool use_tma = false;
-    if constexpr (!NHWC && sizeof(T) == 4) use_tma = tma_applies(feat, C, H, W);
-    roi_prep_kernel<PH, PW><<<(unsigned)((K + 3) / 4), 128, 0, st>>>(rois, K, B, H, W, scale, sr, aligned, prep, tabs,
-                                                                     use_tma ? kTmaXAlign : 1);
-    rc = check_launch("roi_prep_kernel");
-    if (rc == B200_OK) {
-        rc = 1;
-        if constexpr (!NHWC && sizeof(T) == 4)
+    if constexpr (kTmaLayout) use_tma = tma_applies(feat, C, H, W);
+    return with_prep<PH, PW>(rois, K, B, H, W, scale, sr, aligned, use_tma ? kTmaXAlign : 1, st,
+                             [&](const RoiPrep* prep, const float* tabs) {
+        int rc = 1;
+        if constexpr (kTmaLayout)
             if (use_tma) rc = launch_tma<PH, PW, OCL>(feat, B, C, H, W, rois, K, scale, sr, aligned, out, ctiles, prep, tabs, warps, st);
         if (rc == 1) rc = launch_pipe<PH, PW, NHWC, OCL>(feat, B, C, H, W, rois, K, scale, sr, aligned, out, ctiles, prep, tabs, warps, st);
         if (rc == 1) {                       // no TMA / pipelined kernel for this layout / type / size / alignment
-            static int cache[kMaxDevices];   // per instantiation and device
-            auto multi = roi_align_multi_kernel<PH, PW, NHWC, T, OCL>;
+            constexpr auto multi = roi_align_multi_kernel<PH, PW, NHWC, T, OCL>;
             int resident_warps = 0;
-            rc = resident_warps_of(multi, cache, kWarpsPerCta, L::kBytesPerCta, &resident_warps);
+            rc = resident_warps_of<multi>(kWarpsPerCta, L::kBytesPerCta, &resident_warps);
             if (rc == B200_OK) {
-                const long long window = (long long)resident_warps * B200_ROI_MULTI_TILES;
-                const long long groups = (warps + window - 1) / window;
-                const long long last = warps - (groups - 1) * window;
-                const long long nw = (groups - 1) * resident_warps + (last < resident_warps ? last : resident_warps);
+                const long long nw = walker_warps(warps, resident_warps, kMultiTilesPerWarp);
                 launch_ex(multi, dim3((unsigned)((nw + kWarpsPerCta - 1) / kWarpsPerCta)), dim3(kWarpsPerCta * 32),
                           (size_t)L::kBytesPerCta, st, true, 0, feat, B, C, H, W, rois, K, scale, sr, aligned, out, ctiles, prep,
-                          tabs, resident_warps, (int)B200_ROI_MULTI_TILES);
+                          tabs, resident_warps, kMultiTilesPerWarp);
                 rc = check_launch("roi_align_multi_kernel");
             }
         }
-    }
-    B200_CUDA(cudaFreeAsync(ws, st));
-    return rc;
+        return rc;
+    });
+}
+
+// ---- dispatch shared by both directions -----------------------------------------------------------------------
+template <int V> using IntC = std::integral_constant<int, V>;
+template <bool V> using BoolC = std::integral_constant<bool, V>;
+
+// Output sizes with tile kernels (10x10, 7x7) go to tiled(IntC<PH>, IntC<PW>, BoolC<a>, BoolC<b>), where a and b are the
+// two layout flags the launchers take as template parameters; every other size goes to generic().
+template <typename Tiled, typename Generic>
+int dispatch_size(int PH, int PW, bool a, bool b, Tiled tiled, Generic generic) {
+    auto layouts = [&](auto ph, auto pw) {
+        if (a) return b ? tiled(ph, pw, BoolC<true>(), BoolC<true>()) : tiled(ph, pw, BoolC<true>(), BoolC<false>());
+        return b ? tiled(ph, pw, BoolC<false>(), BoolC<true>()) : tiled(ph, pw, BoolC<false>(), BoolC<false>());
+    };
+    if (PH == 10 && PW == 10) return layouts(IntC<10>(), IntC<10>());
+    if (PH == 7 && PW == 7) return layouts(IntC<7>(), IntC<7>());
+    return generic();
+}
+
+// Shape and pointer checks of both directions; `op` starts every message, `map` names the [B,C,H,W] tensor.  Pointers
+// are not looked at when there are no ROIs.
+int check_shapes(const char* op, const char* map, int B, int C, int H, int W, int PH, int PW, int64_t K, bool null_ptr) {
+    B200_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, "%s: bad %s shape [%d,%d,%d,%d]", op, map, B, C, H, W);
+    B200_REQUIRE(PH > 0 && PW > 0, "%s: bad output size (%d,%d)", op, PH, PW);
+    B200_REQUIRE(K >= 0, "%s: negative ROI count", op);
+    B200_REQUIRE(K == 0 || !null_ptr, "%s: null pointer", op);
+    return B200_OK;
+}
+
+// Grid of the generic kernels: one thread per element, at most 32 CTAs of 256 threads per SM (grid-stride loop).
+unsigned generic_blocks(long long total) {
+    const long long want = (total + 255) / 256;
+    return (unsigned)(want < (long long)kSMs * 32 ? want : (long long)kSMs * 32);
+}
+
+// Calls fn(float()) or fn(__half()) for a B200_DTYPE_* of the map / gradient; EINVAL for any other.
+template <typename Fn>
+int with_dtype(int dtype, const char* op, Fn fn) {
+    if (dtype == B200_DTYPE_F32) return fn(float());
+    if (dtype == B200_DTYPE_F16) return fn(__half());
+    return fail(B200_EINVAL, "%s: bad dtype %d", op, dtype);
 }
 
 template <typename T>
@@ -1447,38 +1452,23 @@ int roi_align_dispatch(const T* feat, int layout, int B, int C, int H, int W, co
     B200_REQUIRE(layout == B200_LAYOUT_NCHW || layout == B200_LAYOUT_NHWC, "roi_align: bad layout %d", layout);
     B200_REQUIRE(out_layout == B200_LAYOUT_NCHW || out_layout == B200_LAYOUT_NHWC, "roi_align: bad output layout %d",
                  out_layout);
-    B200_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, "roi_align: bad feature shape [%d,%d,%d,%d]", B, C, H, W);
-    B200_REQUIRE(PH > 0 && PW > 0, "roi_align: bad output size (%d,%d)", PH, PW);
-    B200_REQUIRE(K >= 0, "roi_align: negative ROI count");
+    if (const int rc = check_shapes("roi_align", "feature", B, C, H, W, PH, PW, K, !feat || !rois || !out)) return rc;
     if (K == 0) return B200_OK;
-    B200_REQUIRE(feat && rois && out, "roi_align: null pointer");
     cudaStream_t st = as_stream(stream);
     const bool nhwc = layout == B200_LAYOUT_NHWC, ocl = out_layout == B200_LAYOUT_NHWC;
-#define B200_TILE(ph, pw)                                                                                            \
-    if (PH == ph && PW == pw) {                                                                                      \
-        if (ocl)                                                                                                     \
-            return nhwc ? launch_tile<ph, pw, true, true, T>(feat, B, C, H, W, rois, K, spatial_scale, sampling_ratio, \
-                                                             aligned, out, st)                                       \
-                        : launch_tile<ph, pw, false, true, T>(feat, B, C, H, W, rois, K, spatial_scale,              \
-                                                              sampling_ratio, aligned, out, st);                     \
-        return nhwc ? launch_tile<ph, pw, true, false, T>(feat, B, C, H, W, rois, K, spatial_scale, sampling_ratio,    \
-                                                          aligned, out, st)                                          \
-                    : launch_tile<ph, pw, false, false, T>(feat, B, C, H, W, rois, K, spatial_scale,                 \
-                                                           sampling_ratio, aligned, out, st);                        \
-    }
-    B200_TILE(10, 10)
-    B200_TILE(7, 7)
-#undef B200_TILE
-    const long long total = (long long)K * C * PH * PW;
-    const long long want = (total + 255) / 256;
-    const unsigned blocks = (unsigned)(want < (long long)kSMs * 32 ? want : (long long)kSMs * 32);
-    if (nhwc)
-        roi_align_generic_kernel<true, T><<<blocks, 256, 0, st>>>(feat, B, C, H, W, rois, total, PH, PW,
-                                                                  spatial_scale, sampling_ratio, aligned, out, ocl);
-    else
-        roi_align_generic_kernel<false, T><<<blocks, 256, 0, st>>>(feat, B, C, H, W, rois, total, PH, PW,
-                                                                   spatial_scale, sampling_ratio, aligned, out, ocl);
-    return check_launch("roi_align_generic_kernel");
+    return dispatch_size(
+        PH, PW, nhwc, ocl,
+        [&](auto ph, auto pw, auto map_cl, auto out_cl) {
+            return launch_tile<ph, pw, map_cl, out_cl, T>(feat, B, C, H, W, rois, K, spatial_scale, sampling_ratio, aligned,
+                                                          out, st);
+        },
+        [&] {
+            const long long total = (long long)K * C * PH * PW;
+            const auto kern = nhwc ? roi_align_generic_kernel<true, T> : roi_align_generic_kernel<false, T>;
+            kern<<<generic_blocks(total), 256, 0, st>>>(feat, B, C, H, W, rois, total, PH, PW, spatial_scale, sampling_ratio,
+                                                        aligned, out, ocl);
+            return check_launch("roi_align_generic_kernel");
+        });
 }
 
 // ---- ROI Align backward (torchvision's _roi_align_backward) ---------------------------------------------------
@@ -1675,10 +1665,7 @@ struct BwdTmaSmem {
     static constexpr int kBytesPerWarp = (kOffBar + 16 + 127) & ~127;
     static_assert(kTabBytes % 16 == 0, "bulk-copy alignment");
 };
-#ifndef B200_ROI_BWD_TMA_WARPS
-#define B200_ROI_BWD_TMA_WARPS 2
-#endif
-constexpr int kBwdTmaWarps = B200_ROI_BWD_TMA_WARPS;
+constexpr int kBwdTmaWarps = 2;
 
 __device__ __forceinline__ void tma_reduce_add_4d(const CUtensorMap* tm, unsigned src, int x, int y, int c, int b) {
     asm volatile("cp.reduce.async.bulk.tensor.4d.global.shared::cta.add.tile.bulk_group [%0, {%1, %2, %3, %4}], [%5];\n"
@@ -1806,46 +1793,27 @@ int launch_bwd_tile(const T* go, const float* rois, long long K, float scale, in
     return check_launch("roi_align_bwd_tile_kernel");
 }
 
-// Launches the TMA kernel when it applies; returns 1 when it does not.
+// Launches the TMA kernel (the caller has checked tma_applies); returns 1 when it cannot.
 template <int PH, int PW, typename T, bool GCL>
 int launch_bwd_tma(const T* go, long long K, float* gi, int B, int C, int H, int W, int ctiles, const RoiPrep* prep,
                    const float* tabs, long long tiles, cudaStream_t st) {
-    using S = BwdTmaSmem<PH, PW, T>;
-    if (reinterpret_cast<uintptr_t>(tabs) & 15) return 1;
-    EncodeTiledFn encode = encode_tiled_fn();
-    if (!encode) return 1;
+    constexpr int smem_bytes = BwdTmaSmem<PH, PW, T>::kBytesPerWarp * kBwdTmaWarps;
     TmaMaps tmap;
-    const cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)C, (cuuint64_t)B};
-    const cuuint64_t strides[3] = {(cuuint64_t)W * 4, (cuuint64_t)H * W * 4, (cuuint64_t)C * H * W * 4};
-    const cuuint32_t estr[4] = {1u, 1u, 1u, 1u};
-    for (int i = 0; i < 3; ++i) {                // boxes of 1, 3 and 5 rows, as launch_tma's
-        const cuuint32_t box[4] = {(cuuint32_t)kTmaCols, (cuuint32_t)(2 * i + 1), 32u, 1u};
-        const CUresult r = encode(&tmap.m[i], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, gi, dims, strides, box, estr,
-                                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return 1;
-    }
-    static int cache[kMaxDevices];               // per instantiation and device
-    auto kern = roi_align_bwd_tma_kernel<PH, PW, T, GCL>;
-    constexpr int smem_bytes = S::kBytesPerWarp * kBwdTmaWarps;
+    if ((reinterpret_cast<uintptr_t>(tabs) & 15) || !encode_box_maps(gi, B, C, H, W, &tmap)) return 1;
+    constexpr auto kern = roi_align_bwd_tma_kernel<PH, PW, T, GCL>;
     int resident = 0;
-    const int rc = resident_warps_of(kern, cache, kBwdTmaWarps, smem_bytes, &resident);
+    const int rc = resident_warps_of<kern>(kBwdTmaWarps, smem_bytes, &resident);
     if (rc) return rc;
-    long long tpw = tiles / ((long long)resident * 4);            // at least four waves of warps, 2 .. 16 tiles each
-    tpw = tpw < 2 ? 2 : tpw > 16 ? 16 : tpw;
-    const long long window = (long long)resident * tpw;
-    const long long groups = (tiles + window - 1) / window;
-    const long long last = tiles - (groups - 1) * window;
-    const long long warps = (groups - 1) * resident + (last < resident ? last : resident);
+    const int tpw = tma_tiles_per_warp(tiles, resident);
+    const long long warps = walker_warps(tiles, resident, tpw);
     kern<<<(unsigned)((warps + kBwdTmaWarps - 1) / kBwdTmaWarps), kBwdTmaWarps * 32, smem_bytes, st>>>(
-        tmap, go, K, C, ctiles, prep, tabs, resident, (int)tpw);
+        tmap, go, K, C, ctiles, prep, tabs, resident, tpw);
     return check_launch("roi_align_bwd_tma_kernel");
 }
 
 template <int PH, int PW, typename T, bool GCL, bool ICL>
 int launch_bwd(const T* go, const float* rois, long long K, float scale, int sr, int aligned, float* gi, int B, int C, int H,
                int W, cudaStream_t st) {
-    using L = TileSmem<PH, PW>;
     const int ctiles = (C + 31) / 32;
     const long long tiles = K * ctiles;
     if ((tiles + kWarpsPerCta - 1) / kWarpsPerCta > 0x7fffffffLL || tiles >= (1LL << 32))
@@ -1853,22 +1821,12 @@ int launch_bwd(const T* go, const float* rois, long long K, float scale, int sr,
     if (tiles < kPrepMinTiles || ctiles < 4)
         return launch_bwd_tile<PH, PW, T, GCL, ICL, 0>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, ctiles, nullptr,
                                                        nullptr, st);
-    cudaMemPool_t pool = nullptr;
-    int rc = scratch_pool(&pool);
-    if (rc) return rc;
-    char* ws = nullptr;                          // stream-ordered scratch: K records + K tables
-    const size_t rec = (size_t)K * sizeof(RoiPrep), tab = (size_t)K * L::kTabFloats * sizeof(float);
-    B200_CUDA(cudaMallocFromPoolAsync(reinterpret_cast<void**>(&ws), rec + tab, pool, st));
-    RoiPrep* prep = reinterpret_cast<RoiPrep*>(ws);
-    float* tabs = reinterpret_cast<float*>(ws + rec);
     // the TMA kernel also bulk-loads NCHW grad_out chunks [cn][PH*PW]: each must be whole 16-byte units at a 16-byte boundary
     const bool use_tma = !ICL && tma_applies(gi, C, H, W) &&
                          (GCL || (((size_t)C * PH * PW * sizeof(T)) & 15) == 0 && (reinterpret_cast<uintptr_t>(go) & 15) == 0);
-    roi_prep_kernel<PH, PW><<<(unsigned)((K + 3) / 4), 128, 0, st>>>(rois, K, B, H, W, scale, sr, aligned, prep, tabs,
-                                                                     use_tma ? kTmaXAlign : 1);
-    rc = check_launch("roi_prep_kernel");
-    if (rc == B200_OK) {
-        rc = 1;
+    return with_prep<PH, PW>(rois, K, B, H, W, scale, sr, aligned, use_tma ? kTmaXAlign : 1, st,
+                             [&](const RoiPrep* prep, const float* tabs) {
+        int rc = 1;
         if constexpr (!ICL) {
             if (use_tma) {
                 rc = launch_bwd_tma<PH, PW, T, GCL>(go, K, gi, B, C, H, W, ctiles, prep, tabs, tiles, st);
@@ -1881,9 +1839,8 @@ int launch_bwd(const T* go, const float* rois, long long K, float scale, int sr,
         if (rc == 1)
             rc = launch_bwd_tile<PH, PW, T, GCL, ICL, 1>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, ctiles, prep,
                                                          tabs, st);
-    }
-    B200_CUDA(cudaFreeAsync(ws, st));
-    return rc;
+        return rc;
+    });
 }
 
 template <typename T>
@@ -1892,34 +1849,21 @@ int roi_align_bwd_dispatch(const T* go, int go_layout, const float* rois, int64_
     B200_REQUIRE(layout == B200_LAYOUT_NCHW || layout == B200_LAYOUT_NHWC, "roi_align_backward: bad layout %d", layout);
     B200_REQUIRE(go_layout == B200_LAYOUT_NCHW || go_layout == B200_LAYOUT_NHWC,
                  "roi_align_backward: bad grad_out layout %d", go_layout);
-    B200_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, "roi_align_backward: bad input shape [%d,%d,%d,%d]", B, C, H, W);
-    B200_REQUIRE(PH > 0 && PW > 0, "roi_align_backward: bad output size (%d,%d)", PH, PW);
-    B200_REQUIRE(K >= 0, "roi_align_backward: negative ROI count");
+    if (const int rc = check_shapes("roi_align_backward", "input", B, C, H, W, PH, PW, K, !go || !rois || !gi)) return rc;
     if (K == 0) return B200_OK;
-    B200_REQUIRE(go && rois && gi, "roi_align_backward: null pointer");
     cudaStream_t st = as_stream(stream);
     const bool gcl = go_layout == B200_LAYOUT_NHWC, icl = layout == B200_LAYOUT_NHWC;
-#define B200_BWD(ph, pw)                                                                                                 \
-    if (PH == ph && PW == pw) {                                                                                          \
-        if (gcl)                                                                                                         \
-            return icl ? launch_bwd<ph, pw, T, true, true>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, st)          \
-                       : launch_bwd<ph, pw, T, true, false>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, st);        \
-        return icl ? launch_bwd<ph, pw, T, false, true>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, st)             \
-                   : launch_bwd<ph, pw, T, false, false>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, st);           \
-    }
-    B200_BWD(10, 10)
-    B200_BWD(7, 7)
-#undef B200_BWD
-    const long long total = (long long)K * C * PH * PW;
-    const long long want = (total + 255) / 256;
-    const unsigned blocks = (unsigned)(want < (long long)kSMs * 32 ? want : (long long)kSMs * 32);
-    if (gcl)
-        roi_align_bwd_generic_kernel<true, T><<<blocks, 256, 0, st>>>(go, rois, total, PH, PW, scale, sr, aligned, gi,
-                                                                      icl, B, C, H, W);
-    else
-        roi_align_bwd_generic_kernel<false, T><<<blocks, 256, 0, st>>>(go, rois, total, PH, PW, scale, sr, aligned, gi,
-                                                                       icl, B, C, H, W);
-    return check_launch("roi_align_bwd_generic_kernel");
+    return dispatch_size(
+        PH, PW, gcl, icl,
+        [&](auto ph, auto pw, auto go_cl, auto gi_cl) {
+            return launch_bwd<ph, pw, T, go_cl, gi_cl>(go, rois, K, scale, sr, aligned, gi, B, C, H, W, st);
+        },
+        [&] {
+            const long long total = (long long)K * C * PH * PW;
+            const auto kern = gcl ? roi_align_bwd_generic_kernel<true, T> : roi_align_bwd_generic_kernel<false, T>;
+            kern<<<generic_blocks(total), 256, 0, st>>>(go, rois, total, PH, PW, scale, sr, aligned, gi, icl, B, C, H, W);
+            return check_launch("roi_align_bwd_generic_kernel");
+        });
 }
 
 // ---- box preparation in front of ROI Align (tracking.py:209-213, trainingCard.py:38-69) as one launch -----------
@@ -1991,27 +1935,21 @@ extern "C" int b200_roi_align_fwd_f16(const void* feat, int layout, int B, int C
 extern "C" int b200_roi_align_fwd_ex(const void* feat, int dtype, int layout, int B, int C, int H, int W,
                                      const float* rois, int64_t K, int PH, int PW, float spatial_scale,
                                      int sampling_ratio, int aligned, void* out, int out_layout, void* stream) {
-    if (dtype == B200_DTYPE_F32)
-        return b200::roi_align_dispatch<float>(static_cast<const float*>(feat), layout, B, C, H, W, rois, K, PH, PW,
-                                               spatial_scale, sampling_ratio, aligned, static_cast<float*>(out),
-                                               out_layout, stream);
-    if (dtype == B200_DTYPE_F16)
-        return b200::roi_align_dispatch<__half>(static_cast<const __half*>(feat), layout, B, C, H, W, rois, K, PH, PW,
-                                                spatial_scale, sampling_ratio, aligned, static_cast<__half*>(out),
-                                                out_layout, stream);
-    return b200::fail(B200_EINVAL, "roi_align: bad dtype %d", dtype);
+    return b200::with_dtype(dtype, "roi_align", [&](auto zero) {
+        using T = decltype(zero);
+        return b200::roi_align_dispatch<T>(static_cast<const T*>(feat), layout, B, C, H, W, rois, K, PH, PW, spatial_scale,
+                                           sampling_ratio, aligned, static_cast<T*>(out), out_layout, stream);
+    });
 }
 
 extern "C" int b200_roi_align_bwd_ex(const void* grad_out, int dtype, int grad_out_layout, const float* rois, int64_t K,
                                      int PH, int PW, float spatial_scale, int sampling_ratio, int aligned, float* grad_in,
                                      int layout, int B, int C, int H, int W, void* stream) {
-    if (dtype == B200_DTYPE_F32)
-        return b200::roi_align_bwd_dispatch<float>(static_cast<const float*>(grad_out), grad_out_layout, rois, K, PH, PW,
-                                                   spatial_scale, sampling_ratio, aligned, grad_in, layout, B, C, H, W, stream);
-    if (dtype == B200_DTYPE_F16)
-        return b200::roi_align_bwd_dispatch<__half>(static_cast<const __half*>(grad_out), grad_out_layout, rois, K, PH, PW,
-                                                    spatial_scale, sampling_ratio, aligned, grad_in, layout, B, C, H, W, stream);
-    return b200::fail(B200_EINVAL, "roi_align_backward: bad dtype %d", dtype);
+    return b200::with_dtype(dtype, "roi_align_backward", [&](auto zero) {
+        using T = decltype(zero);
+        return b200::roi_align_bwd_dispatch<T>(static_cast<const T*>(grad_out), grad_out_layout, rois, K, PH, PW,
+                                               spatial_scale, sampling_ratio, aligned, grad_in, layout, B, C, H, W, stream);
+    });
 }
 
 B200_SPAN_GETTER(b200_debug_spans_roi)
