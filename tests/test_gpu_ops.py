@@ -161,16 +161,24 @@ def test_app_cost_vs_oracle(M, N, T):
         assert_close(got.cpu().numpy(), want, rtol=1e-5, atol=2e-6, what="C_app")
 
 
-@pytest.mark.parametrize("kernel,M,N,T", [("2", 260, 130, 30), ("2", 300, 64, 9), ("2", 512, 512, 30), ("2", 70, 64, 32),
-                                          ("2", 257, 1000, 32), ("1", 512, 512, 30), ("1", 260, 130, 30)])
-def test_app_cost_tensor_core_kernels_vs_oracle(kernel, M, N, T, monkeypatch):
-    """Both tcgen05 forms of the dense appearance cost, each forced with B200TRACK_TC_KERNEL: 1 = a CTA per (bank tile,
-    detection tile) pair, 2 = a CTA keeps its bank tile resident and walks the detection tiles (two TMEM accumulators, the
-    tensor core one tile ahead of the epilogue).  Ragged tiles in both directions, empty / short / full banks, the EMA
-    fallback, top-k beyond five and the max-similarity variant."""
-    monkeypatch.setenv("B200TRACK_TC_KERNEL", kernel)
-    if kernel == "2" and (M * 32 + 127) // 128 % 2 == 0 and N > 64:
-        monkeypatch.setenv("B200TRACK_TC_CLUSTER", "2")       # CTA pairs sharing the detection tiles (half-tile multicast)
+# nseg = the number of segments each bank tile's walk is split into on 148 SMs: clamp(148 // m_tiles, 1, n_tiles) with
+# m_tiles = ceil(M / 4) bank tiles and n_tiles = ceil(N / 64) detection tiles.  Every shape has M * N >= 64 * 64.
+@pytest.mark.parametrize("M,N,T", [(260, 130, 30),     # nseg 2: segments of 2 and 1 steps (ragged last segment)
+                                   (300, 64, 9),       # nseg 1: 75 bank tiles, one step
+                                   (512, 512, 30),     # nseg 1: BASELINE config 4, 8 steps
+                                   (70, 64, 32),       # nseg 1: 18 bank tiles but a single detection tile
+                                   (257, 1000, 32),    # nseg 2: 8 steps each
+                                   (392, 512, 30),     # nseg 1: 98 bank tiles, 8 steps
+                                   (16, 260, 30),      # nseg 5 = n_tiles < 148 // 4: segments of exactly one step
+                                   (100, 900, 30),     # nseg 5: segments of exactly three steps
+                                   (40, 2000, 32),     # nseg 14: segments of 3 and 2 steps, ragged last tile
+                                   (64, 4096, 30)])    # nseg 9 < n_tiles = 64: segments of 8 and 7 steps
+def test_app_cost_tensor_core_kernels_vs_oracle(M, N, T):
+    """The tcgen05 dense appearance cost (a CTA per bank tile and segment keeps its bank image resident and walks the
+    segment's detection tiles: two TMEM accumulators, the tensor core one tile ahead of the epilogue) on every case of
+    its launch: one segment, several, ragged, of one step and of enough steps that both buffers and both accumulators
+    are reused.  Ragged tiles in both directions, empty / short / full banks, the EMA fallback, top-k beyond five and
+    the max-similarity variant.  Each call is the two tensor-core launches (prep + walk), not the float32 kernel."""
     rng = np.random.default_rng(3 * M + 11 * N + T)
     lens = rng.integers(0, T + 1, M)
     lens[0], lens[1], lens[2], lens[M - 1] = T, 0, 1, T
@@ -178,13 +186,16 @@ def test_app_cost_tensor_core_kernels_vs_oracle(kernel, M, N, T, monkeypatch):
     ema = rng.standard_normal((M, 128)).astype(np.float32)
     det = rng.standard_normal((N, 128)).astype(np.float32) * 0.3
     banks = [[bank[i, t] for t in range(lens[i])] for i in range(M)]
+    lib = alufe_b200._lib.lib()
     for topk, mean, fb in [(5, True, True), (5, True, False), (1, False, True), (9, True, True)]:
         want = cost_ref.app_cost_topk(banks, list(det), topk=topk, use_topk_mean=mean,
                                       fallback_embs=list(ema) if fb else None)
+        launches = lib.b200_launch_count()
         got = cost.app_cost_topk(torch.from_numpy(bank).cuda(), torch.from_numpy(lens.astype(np.int32)).cuda(),
                                  torch.from_numpy(det).cuda(), topk=topk, use_topk_mean=mean,
                                  fallback=torch.from_numpy(ema).cuda() if fb else None)
-        assert_close(got.cpu().numpy(), want, rtol=1e-5, atol=2e-6, what="C_app kernel %s topk %d" % (kernel, topk))
+        assert lib.b200_launch_count() - launches == 2
+        assert_close(got.cpu().numpy(), want, rtol=1e-5, atol=2e-6, what="C_app topk %d" % topk)
 
 
 def test_app_cost_c4_size_properties():
