@@ -26,10 +26,9 @@ __device__ long long g_lsap_clk[8];                 // SM-clock stamps inside so
 #endif
 
 constexpr int kMaxThreads = 256;
-#ifndef B200_LSAP_WARP_MAX_COLS
-#define B200_LSAP_WARP_MAX_COLS 128
-#endif
-constexpr int kWarpSolverMaxCols = B200_LSAP_WARP_MAX_COLS;   // wider problems use the multi-warp register solver
+// Widest problem of the single-warp solver; wider ones use the multi-warp register solver.  One warp wins up to 128
+// columns and loses from 256 on (the 64 / 128 / 256 / 512-column timings in the comment of solve_block).
+constexpr int kWarpSolverMaxCols = 128;
 
 struct Work {              // all arrays in shared memory, sized for R rows / Cc columns
     double* u;             // [R]

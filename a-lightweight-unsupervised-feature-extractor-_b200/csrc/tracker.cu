@@ -373,11 +373,10 @@ struct RowMin {
 //   per survivor: lanes split the 128 dimensions (one coalesced 512 B read per bank row, eight rows in
 //   flight), a shuffle reduction gives <bank_t, det>, lane t keeps the similarity of row t, then k rounds
 //   of warp-max give the top-k mean.  No shared memory and few registers, so every row of a 64-stream
-//   group is resident at once and the kernel can share SMs with ROI Align.
-#ifndef B200_COST1_WARPS
-#define B200_COST1_WARPS 4
-#endif
-constexpr int kCost1Warps = B200_COST1_WARPS;
+//   group is resident at once and the kernel can share SMs with ROI Align.  Four warps per CTA: with two or one,
+//   neither the six-kernel chain alone nor the overlapped step changed (profiles/r02_chain_cta_sweep.txt, builds
+//   c1w2 / c1w1).
+constexpr int kCost1Warps = 4;
 
 __device__ __forceinline__ unsigned fkey(float f) {                 // order-preserving float -> uint
     const unsigned b = __float_as_uint(f);
@@ -948,10 +947,9 @@ __global__ void __launch_bounds__(kThreads) assign_kernel(Dev d, int smem_matrix
 // back_kernel (one CTA of 256 threads per stream): stage-1 assignment and bookkeeping, the ReID-only cost of the
 // stream's long-lost rows (usually none), stage-2 assignment, births, purge, result table, and finally the Kalman / EMA
 // / bank updates of the stream's own matches.  Streams are independent, so nothing inside waits for another CTA.
-#ifndef B200_TRK_FRONT_WARPS
-#define B200_TRK_FRONT_WARPS 4
-#endif
-constexpr int kFrontWarps = B200_TRK_FRONT_WARPS;
+// Four warps per front CTA: two or one do not shorten the overlapped 64-stream step (profiles/r02_footprint_sweep.txt,
+// builds fw2 / fw1).
+constexpr int kFrontWarps = 4;
 
 __global__ void __launch_bounds__(kFrontWarps * 32, 2) front_kernel(Dev d) {
     Span span((d.frame_id[0] & 7) * 6 + 0);
@@ -1000,10 +998,8 @@ __global__ void __launch_bounds__(kFrontWarps * 32, 2) front_kernel(Dev d) {
 // of the cluster runs the serial part (assignments, births, purge, result table) while the others wait at the cluster
 // barrier, then all CTAs of the cluster share the stream's Kalman / EMA / bank updates -- 12.5 -> 6 us for 64 matches,
 // 23 -> 6 us for 128 (profiles/r02_fused_timeline.txt).  Without the cluster attribute the cluster is the CTA itself.
-#ifndef B200_TRK_BACK_CLUSTER
-#define B200_TRK_BACK_CLUSTER 4
-#endif
-constexpr int kBackCluster = B200_TRK_BACK_CLUSTER;
+// Clusters of 2 and of 8 CTAs were measured against 4 and neither was faster (commit 7145e8b; no profile recorded).
+constexpr int kBackCluster = 4;
 
 __device__ __forceinline__ unsigned cluster_ctarank() {
     unsigned r;
@@ -1155,7 +1151,7 @@ constexpr int kRowsInFlight = 6;
 
 // Moves one track between slot `slot` of the handle and track `it` (row * cap + position) of an image.  EXPORT: slot ->
 // image, the bank ring unrolled oldest row first and rows past bank_len zeroed (what b200_tracker_export writes); import:
-// image -> slot, every bank row in order (the slot's ring then starts at row 0, as after b200_tracker_import).
+// image -> slot, every bank row in order (the slot's ring then starts at row 0).
 template <bool EXPORT>
 __device__ __forceinline__ void copy_track(const Dev& d, const b200_tracker_state& im, size_t slot, size_t it, int lane) {
     auto mv = [&](auto* s_side, auto* i_side) { if (EXPORT) *i_side = *s_side; else *s_side = *i_side; };
@@ -1229,15 +1225,14 @@ __device__ void finish_import(const Dev& d, int s, int n, int next_id) {
     }
 }
 
-__global__ void import_finish_kernel(Dev d, int s, int n, int next_id) { finish_import(d, s, n, next_id); }
-
 // One CTA per image row, ahead of import_state_kernel: validates the row (every index it reads is checked first) and, if it
 // passes, rebuilds the stream's header, order and free list.  imp_row[s] = r names the row import_state_kernel copies into
-// stream s (-1: none); only entries of streams named by this image are read, and each is written here first.
-__global__ void __launch_bounds__(kThreads) import_check_kernel(Dev d, b200_tracker_state im, const int* streams,
+// stream s (-1: none); only entries of streams named by this image are read, and each is written here first.  Streams as
+// in export_state_kernel; b200_tracker_import runs both kernels on a one-row image of its host arrays.
+__global__ void __launch_bounds__(kThreads) import_check_kernel(Dev d, b200_tracker_state im, const int* streams, int s0,
                                                                  int* imp_row, int* status) {
     const int r = blockIdx.x;
-    const int s = image_stream(streams, 0, r);
+    const int s = image_stream(streams, s0, r);
     if (s < 0 || s >= d.S) {
         if (status && threadIdx.x == 0) status[r] = B200_EINVAL;
         return;
@@ -1267,9 +1262,9 @@ __global__ void __launch_bounds__(kThreads) import_check_kernel(Dev d, b200_trac
 
 // grid (ceil(cap / kStateWarps), n_rows): copies the rows import_check_kernel accepted into slots 0..n-1 of their streams.
 __global__ void __launch_bounds__(kStateWarps * 32) import_state_kernel(Dev d, b200_tracker_state im, const int* streams,
-                                                                         const int* imp_row) {
+                                                                         int s0, const int* imp_row) {
     const int r = blockIdx.y;
-    const int s = image_stream(streams, 0, r);
+    const int s = image_stream(streams, s0, r);
     if (s < 0 || s >= d.S || imp_row[s] != r) return;
     const int p = blockIdx.x * kStateWarps + (threadIdx.x >> 5);
     if (p >= im.n_live[r]) return;
@@ -1434,11 +1429,7 @@ struct b200_tracker {
     // packed step queued on one stream never races with a host step or a step-by-step operation queued on another
     trk::StepInputs pk = {};
     int* pk_inv = nullptr; int* pk_over = nullptr;
-    int* imp_row = nullptr;         // [S] b200_tracker_import_device: the image row accepted for each stream
-#ifndef B200_TRK_BEGIN_THREADS
-#define B200_TRK_BEGIN_THREADS 256
-#endif
-    int begin_threads = B200_TRK_BEGIN_THREADS;   // CTA width of begin_kernel
+    int* imp_row = nullptr;         // [S] import_check_kernel: the image row accepted for each stream
     int cost_grid = 0, cost1_grid = 0, upd_grid = 0;   // persistent CTAs of the cost kernels (resident CTAs per SM x SMs)
     size_t assign_smem = 0;
     int smem_matrix_floats = 0;
@@ -1666,7 +1657,7 @@ extern "C" int b200_tracker_step(b200_tracker* t, const int32_t* n_det, const do
                   t->smem_matrix_floats);
         return check_launch("trk back_kernel");
     }
-    trk::begin_kernel<<<dim3(d.S, 2), t->begin_threads, 0, st>>>(d);
+    trk::begin_kernel<<<dim3(d.S, 2), trk::kThreads, 0, st>>>(d);
     rc = check_launch("trk begin_kernel");
     if (rc) return rc;
     // With a handful of streams the step is a chain of short, latency-bound kernels: launch the dependent ones
@@ -2004,6 +1995,25 @@ dim3 image_grid(const b200_tracker_state& im) {
     return dim3((unsigned)((im.cap + trk::kStateWarps - 1) / trk::kStateWarps), (unsigned)im.n_rows);
 }
 
+// The staging buffer of b200_tracker_export / b200_tracker_import, allocated in stream order on `st`: a one-row image of
+// `cap` slots.  n_live, next_id and the row's status share the first range.
+cudaError_t alloc_row_image(b200_tracker_state& s, size_t cap, int hist_max, cudaStream_t st, char*& buf) {
+    const size_t H = hist_max;
+    s.n_rows = 1; s.cap = (int)cap; s.hist_max = hist_max;
+    auto carve = [&](trk::Carver& c) {
+        c.take(s.n_live, 3); s.next_id = s.n_live + 1;
+        c.take(s.ids, cap); c.take(s.x, cap * 8); c.take(s.P, cap * 64); c.take(s.stage, cap); c.take(s.ema, cap * 128);
+        c.take(s.bank, cap * H * 128); c.take(s.bank_len, cap); c.take(s.miss, cap); c.take(s.age, cap);
+        c.take(s.last_bbox, cap * 4); c.take(s.last_conf, cap); c.take(s.last_cost, cap);
+    };
+    trk::Carver size;
+    carve(size);
+    const cudaError_t e = cudaMallocAsync(reinterpret_cast<void**>(&buf), size.off, st);
+    trk::Carver c{buf};
+    carve(c);
+    return e;
+}
+
 }  // namespace
 
 extern "C" int b200_tracker_export_device(b200_tracker* t, const int32_t* streams, const b200_tracker_state* img,
@@ -2019,9 +2029,9 @@ extern "C" int b200_tracker_import_device(b200_tracker* t, const int32_t* stream
     int rc = check_image(t, streams, img, "tracker_import_device");
     if (rc || img->n_rows == 0) return rc;
     cudaStream_t st = as_stream(stream);
-    trk::import_check_kernel<<<img->n_rows, trk::kThreads, 0, st>>>(t->d, *img, streams, t->imp_row, status);
+    trk::import_check_kernel<<<img->n_rows, trk::kThreads, 0, st>>>(t->d, *img, streams, 0, t->imp_row, status);
     if ((rc = check_launch("trk import_check_kernel"))) return rc;
-    trk::import_state_kernel<<<image_grid(*img), trk::kStateWarps * 32, 0, st>>>(t->d, *img, streams, t->imp_row);
+    trk::import_state_kernel<<<image_grid(*img), trk::kStateWarps * 32, 0, st>>>(t->d, *img, streams, 0, t->imp_row);
     return check_launch("trk import_state_kernel");
 }
 
@@ -2033,22 +2043,10 @@ extern "C" int b200_tracker_export(b200_tracker* t, int stream_idx, int32_t* ids
     const trk::Dev& d = t->d;
     B200_REQUIRE(stream_idx >= 0 && stream_idx < d.S, "tracker_export: stream %d out of range", stream_idx);
     cudaStream_t st = as_stream(stream);
-    const size_t MT = d.MT, H = d.HIST;
-    // staging buffer: a one-row image of the stream, cap = max_tracks
+    const size_t H = d.HIST;
     b200_tracker_state s{};
-    s.n_rows = 1; s.cap = d.MT; s.hist_max = d.HIST;
-    auto carve = [&](trk::Carver& c) {
-        c.take(s.n_live, 2); s.next_id = s.n_live + 1;
-        c.take(s.ids, MT); c.take(s.x, MT * 8); c.take(s.P, MT * 64); c.take(s.stage, MT); c.take(s.ema, MT * 128);
-        c.take(s.bank, MT * H * 128); c.take(s.bank_len, MT); c.take(s.miss, MT); c.take(s.age, MT); c.take(s.last_bbox, MT * 4);
-        c.take(s.last_conf, MT); c.take(s.last_cost, MT);
-    };
-    trk::Carver size;
-    carve(size);
     char* buf = nullptr;
-    B200_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&buf), size.off, st));
-    trk::Carver c{buf};
-    carve(c);
+    B200_CUDA(alloc_row_image(s, d.MT, d.HIST, st, buf));
     trk::export_state_kernel<<<image_grid(s), trk::kStateWarps * 32, 0, st>>>(d, s, nullptr, stream_idx, nullptr);
     int rc = check_launch("trk export_state_kernel");
     if (rc) return rc;
@@ -2093,22 +2091,35 @@ extern "C" int b200_tracker_import(b200_tracker* t, int stream_idx, int n, const
     const trk::Dev& d = t->d;
     B200_REQUIRE(stream_idx >= 0 && stream_idx < d.S, "tracker_import: stream %d out of range", stream_idx);
     B200_REQUIRE(n >= 0 && n <= d.MT, "tracker_import: %d tracks exceed max_tracks %d", n, d.MT);
+    B200_REQUIRE(n == 0 || (ids && x && P && stage && ema && bank && bank_len && miss && age && last_bbox && last_conf &&
+                            last_cost), "tracker_import: null array");
     cudaStream_t st = as_stream(stream);
-    const size_t sb = (size_t)stream_idx * d.MT, H = d.HIST;
-    if (n > 0) {
-        B200_REQUIRE(ids && x && P && stage && ema && bank && bank_len && miss && age && last_bbox && last_conf && last_cost,
-                     "tracker_import: null array");
-#define PUSH(dst, src, T, per) B200_CUDA(cudaMemcpyAsync(dst + sb * (per), src, sizeof(T) * (per) * n, cudaMemcpyHostToDevice, st))
-        PUSH(d.tid, ids, int, 1); PUSH(d.kf_x, x, double, 8); PUSH(d.kf_P, P, double, 64); PUSH(d.kf_stage, stage, uint8_t, 1);
-        PUSH(d.ema, ema, float, 128); PUSH(d.bank, bank, float, H * 128); PUSH(d.bank_len, bank_len, int, 1);
-        PUSH(d.miss, miss, int, 1); PUSH(d.age, age, int, 1); PUSH(d.last_bbox, last_bbox, double, 4);
-        PUSH(d.last_conf, last_conf, double, 1); PUSH(d.last_cost, last_cost, double, 1);
-#undef PUSH
-    }
-    trk::import_finish_kernel<<<1, 256, 0, st>>>(d, stream_idx, n, next_id);
-    int rc = check_launch("trk import_finish_kernel");
+    const size_t H = d.HIST;
+    b200_tracker_state s{};
+    char* buf = nullptr;
+    B200_CUDA(alloc_row_image(s, n > 0 ? n : 1, d.HIST, st, buf));
+    const int hdr[2] = {n, next_id};
+    cudaError_t e = cudaMemcpyAsync(s.n_live, hdr, sizeof(hdr), cudaMemcpyHostToDevice, st);
+    auto push = [&](auto* dst, const auto* src, size_t per) {
+        if (e == cudaSuccess && n > 0) e = cudaMemcpyAsync(dst, src, sizeof(*dst) * per * n, cudaMemcpyHostToDevice, st);
+    };
+    push(s.ids, ids, 1); push(s.x, x, 8); push(s.P, P, 64); push(s.stage, stage, 1); push(s.ema, ema, 128);
+    push(s.bank, bank, H * 128); push(s.bank_len, bank_len, 1); push(s.miss, miss, 1); push(s.age, age, 1);
+    push(s.last_bbox, last_bbox, 4); push(s.last_conf, last_conf, 1); push(s.last_cost, last_cost, 1);
+    B200_CUDA(e);
+    int* status = s.n_live + 2;
+    trk::import_check_kernel<<<1, trk::kThreads, 0, st>>>(d, s, nullptr, stream_idx, t->imp_row, status);
+    int rc = check_launch("trk import_check_kernel");
     if (rc) return rc;
+    trk::import_state_kernel<<<image_grid(s), trk::kStateWarps * 32, 0, st>>>(d, s, nullptr, stream_idx, t->imp_row);
+    if ((rc = check_launch("trk import_state_kernel"))) return rc;
+    int row_status = B200_OK;
+    B200_CUDA(cudaMemcpyAsync(&row_status, status, sizeof(row_status), cudaMemcpyDeviceToHost, st));
     B200_CUDA(cudaStreamSynchronize(st));          // the host arrays may be released after return
+    B200_CUDA(cudaFreeAsync(buf, st));
+    // n fits the image and max_tracks (checked above), so the only status left is B200_EINVAL: the stream is untouched.
+    B200_REQUIRE(row_status == B200_OK, "tracker_import: stream %d: malformed state (ids not ascending or outside "
+                 "[0, next_id), bank_len outside [0, hist_max] or stage > 2)", stream_idx);
     return B200_OK;
 }
 

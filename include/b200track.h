@@ -267,8 +267,10 @@ int  b200_tracker_export(b200_tracker* t, int stream_idx, int32_t* ids, double* 
                          int32_t* next_id, void* stream);
 
 /* Inverse of b200_tracker_export: replaces one stream's state by `n` tracks given in ascending track-id
- * order (host arrays, same layouts as export).  b200_tracker_import_device below does the same for any
- * set of streams from device memory without a synchronisation. */
+ * order (host arrays, same layouts as export).  The arrays go through b200_tracker_import_device below as a
+ * one-row image, with its checks: a malformed row returns B200_EINVAL and leaves the stream untouched.
+ * b200_tracker_import_device does the same for any set of streams from device memory without a
+ * synchronisation. */
 int  b200_tracker_import(b200_tracker* t, int stream_idx, int n, const int32_t* ids, const double* x,
                          const double* P, const uint8_t* stage, const float* ema, const float* bank,
                          const int32_t* bank_len, const int32_t* miss, const int32_t* age,

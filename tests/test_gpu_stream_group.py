@@ -43,7 +43,7 @@ if mp.parent_process() is None:
     from test_gpu_tracker import _oracle_state, _compare_state
     from test_gpu_tracker_state import _row
 
-FRONT_WARPS = 4                 # warps per front_kernel CTA (B200_TRK_FRONT_WARPS)
+FRONT_WARPS = 4                 # warps per front_kernel CTA (kFrontWarps in tracker.cu)
 
 
 @pytest.fixture(scope="module")

@@ -145,6 +145,57 @@ def test_grow_matches_the_host_round_trip_and_the_oracle():
         _same(x, y, "stream %d" % s)
 
 
+def test_import_state_loads_like_load_state_dict_and_refuses_malformed_snapshots():
+    """import_state (host arrays, b200_tracker_import) goes through the device import: a valid snapshot lands exactly as
+    load_state_dict of the same row does, and a snapshot the row check rejects raises and leaves the stream as it was."""
+    S, H = 3, CFG["hist_max"]
+    frames = _streams(S, 170, 30)
+    src = MultiStreamTracker(S, CFG, max_tracks=64, max_dets=MD)
+    a = MultiStreamTracker(S, CFG, max_tracks=64, max_dets=MD)
+    b = MultiStreamTracker(S, CFG, max_tracks=64, max_dets=MD)
+    for f in range(20):
+        _step(src, frames, f)
+        if f < 8:
+            _step(a, frames, f)
+            _step(b, frames, f)
+    snap = src.export(2)
+    assert len(snap["ids"]) >= 2 and (snap["bank_len"] == H).any()      # 20 frames at hist_max 5: full, wrapped rings
+    a.import_state(1, snap)
+    b.load_state_dict(src.state_dict([2]), streams=[1])
+    assert a.n_live[1] == b.n_live[1] == len(snap["ids"])
+    _same(a.export(1), snap, "imported")
+    for s, (x, y) in enumerate(zip(_exports(a), _exports(b))):
+        _same(x, y, "stream %d" % s)
+    moved = [frames[0], frames[2], frames[1]]
+    for f in range(20, 30):
+        got_a, want = _step(a, moved, f), _step(src, frames, f)
+        assert got_a == _step(b, moved, f) and got_a[1] == want[2], "frame %d" % f
+
+    before, n_before = a.export(0), int(a.n_live[0])
+
+    def bad(**edit):
+        out = {k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in snap.items()}
+        for k, (i, v) in edit.items():
+            out[k][i] = v
+        return out
+
+    ids, next_id = snap["ids"], snap["next_id"]
+    cases = {"unsorted ids": bad(ids=(slice(0, 2), ids[1::-1])), "negative id": bad(ids=(0, -1)),
+             "id not below next_id": bad(ids=(-1, next_id)), "bank_len above hist_max": bad(bank_len=(0, H + 1)),
+             "negative bank_len": bad(bank_len=(0, -1)), "stage above 2": bad(stage=(1, 3))}
+    for what, snap_bad in cases.items():
+        with pytest.raises(ValueError, match="malformed state"):
+            a.import_state(0, snap_bad)
+        _same(a.export(0), before, what)
+        assert a.n_live[0] == n_before, what
+
+    empty = MultiStreamTracker(1, CFG, max_tracks=8, max_dets=MD).export(0)     # no tracks: a one-slot image
+    empty["next_id"] = 7
+    a.import_state(2, empty)
+    _same(a.export(2), empty, "empty")
+    assert a.n_live[2] == 0
+
+
 def test_grow_keeps_the_old_handle_when_creation_fails():
     ms = MultiStreamTracker(2, CFG, max_tracks=16, max_dets=MD)
     frames = _streams(2, 70, 8)
