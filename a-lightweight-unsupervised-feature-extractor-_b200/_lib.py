@@ -8,8 +8,7 @@ import os
 import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# B200TRACK_LIB: load another build of the same library (the timing build of tools/build_timing.sh, a parent commit's
-# build to compare against); unset = the product
+# B200TRACK_LIB: load another build of the same library (e.g. another commit's, to compare against); unset = the product
 LIB_PATH = os.environ.get("B200TRACK_LIB") or os.path.join(_HERE, "libb200track.so")
 CSRC = os.path.join(_HERE, "csrc")
 

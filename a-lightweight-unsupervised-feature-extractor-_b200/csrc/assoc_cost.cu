@@ -1,6 +1,4 @@
 // Cost operators of the C ABI: build_C_app_topk and bbox/conf/total cost.  Math in assoc_cost.cuh.
-#include <stdlib.h>
-
 #include "assoc_cost.cuh"
 
 namespace b200 {
@@ -61,13 +59,10 @@ extern "C" int b200_app_cost_topk_f32(const float* bank, const int32_t* bank_len
     B200_REQUIRE(bank && bank_len && det && C_app, "app_cost: null pointer");
     B200_REQUIRE(ldc >= N, "app_cost: ldc < N");
     B200_REQUIRE(M <= 65535, "app_cost: M too large");
-    // large launches are a real GEMM: bf16x3-split tensor-core kernel (app_cost_tc.cu); B200TRACK_NO_TC=1 keeps the
-    // float32 FFMA kernel (used by the tests to compare the two)
-    static const bool no_tc = getenv("B200TRACK_NO_TC") != nullptr;
-    if (!no_tc) {
-        const int rc = app_cost_tc(bank, bank_len, fallback, det, M, N, T, topk, use_topk_mean, C_app, ldc, as_stream(stream));
-        if (rc != 1) return rc;
-    }
+    // large launches are a real GEMM: bf16x3-split tensor-core kernel (app_cost_tc.cu); problems under 64 x 64 and
+    // banks deeper than its 32 rows keep the float32 FFMA kernel below
+    const int rc = app_cost_tc(bank, bank_len, fallback, det, M, N, T, topk, use_topk_mean, C_app, ldc, as_stream(stream));
+    if (rc != 1) return rc;
     static bool configured[64];
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 0;

@@ -79,30 +79,4 @@ __device__ __forceinline__ int warp_max(int v) {
     return v;
 }
 
-
-#ifdef B200_TRK_TIMING          // debug builds only: global-timer spans of every kernel (see tools/timeline_probe.py)
-static __device__ unsigned long long g_span[128];     // per translation unit: [2*k] = min start, [2*k+1] = max end
-__device__ __forceinline__ unsigned long long gtime() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-#define B200_SPAN_BEGIN(k) do { if (threadIdx.x == 0) atomicMin(&::b200::g_span[2 * (k)], ::b200::gtime()); } while (0)
-#define B200_SPAN_END(k) do { if (threadIdx.x == 0) atomicMax(&::b200::g_span[2 * (k) + 1], ::b200::gtime()); } while (0)
-#define B200_SPAN_GETTER(name)                                                                          \
-    extern "C" int name(unsigned long long* out64, int reset) {                                         \
-        if (out64 && cudaMemcpyFromSymbol(out64, ::b200::g_span, sizeof(unsigned long long) * 128) != cudaSuccess) return -2; \
-        if (reset) {                                                                                    \
-            unsigned long long init[128];                                                                \
-            for (int i = 0; i < 128; ++i) init[i] = (i & 1) ? 0ull : ~0ull;                              \
-            if (cudaMemcpyToSymbol(::b200::g_span, init, sizeof(init)) != cudaSuccess) return -2;       \
-        }                                                                                               \
-        return 0;                                                                                       \
-    }
-#else
-#define B200_SPAN_GETTER(name)
-#define B200_SPAN_BEGIN(k) do { } while (0)
-#define B200_SPAN_END(k) do { } while (0)
-#endif
-
 }  // namespace b200

@@ -15,16 +15,6 @@
 namespace b200 {
 namespace lsap {
 
-#ifdef B200_TRK_TIMING             // debug builds: [0] searches skipped by the known-first-step rule, [1] full searches,
-__device__ unsigned long long g_lsap_stats[4];      // [2] Dijkstra steps of the full searches (per translation unit)
-__device__ long long g_lsap_clk[8];                 // SM-clock stamps inside solve_block (CTA 0)
-#define LSAP_STAT(i, n) do { if ((threadIdx.x & 31) == 0 && blockIdx.x == 0) g_lsap_stats[i] += (n); } while (0)
-#define LSAP_CLK(k) do { if (threadIdx.x == 0 && blockIdx.x == 0) g_lsap_clk[k] = clock64(); } while (0)
-#else
-#define LSAP_STAT(i, n) do { } while (0)
-#define LSAP_CLK(k) do { } while (0)
-#endif
-
 constexpr int kMaxThreads = 256;
 // Widest problem of the single-warp solver; wider ones use the multi-warp register solver.  One warp wins up to 128
 // columns and loses from 256 on (the 64 / 128 / 256 / 512-column timings in the comment of solve_block).
@@ -307,9 +297,7 @@ __device__ inline int solve_warp(const float* cost, int R, int Cc, int ld, doubl
         unsigned scanned = 0;                            // bit q: own column q scanned in this search
         int i = cur, n_todo = Cc, sink = -1;
         double minv = 0.0;
-        LSAP_STAT(1, 1);
         while (sink < 0) {
-            LSAP_STAT(2, 1);
             const double ui = u_s[i];
             const float* crow = cost + (size_t)i * ld;
             unsigned long long bk = ~0ull;
@@ -438,9 +426,7 @@ __device__ inline int solve_regs(const float* cost, int R, int Cc, int ld, const
         unsigned scanned = 0;
         int i = cur, n_todo = Cc, sink = -1;
         double minv = 0.0;
-        if (tid == 0) LSAP_STAT(1, 1);
         while (sink < 0) {
-            if (tid == 0) LSAP_STAT(2, 1);
             const double ui = w.u[i];
             const float* crow = cost + (size_t)i * ld;
             unsigned long long bk = ~0ull;
@@ -600,7 +586,6 @@ __device__ __noinline__ inline int solve_block(const float* cost, int R, int Cc,
     const float kNegInf = -__int_as_float(0x7f800000);
     int* first_col = w.seen_rows;                         // [R] column of the row's unique minimum, or -1
     float* first_val = reinterpret_cast<float*>(w.dist);  // [R] that minimum
-    LSAP_CLK(0);
     const int lpr = (pre_col && !stage_or_null) ? 0 : (Cc + 31) / 32;
     if (lpr == 0) {
         for (int i = tid; i < R; i += nthr) {
@@ -643,7 +628,6 @@ __device__ __noinline__ inline int solve_block(const float* cost, int R, int Cc,
         }
     }
     bad = __syncthreads_or(bad);
-    LSAP_CLK(1);
     if (bad) return B200_ENUMERIC;
     if (stage_or_null) { cost = stage_or_null; ld = Cc; }
     __shared__ int s_status;
@@ -663,7 +647,6 @@ __device__ __noinline__ inline int solve_block(const float* cost, int R, int Cc,
         if (tid == 0) s_status = rc;
     }
     __syncthreads();
-    LSAP_CLK(2);
     return s_status;
 }
 

@@ -303,12 +303,6 @@ roi_prep_kernel(const float* __restrict__ rois, long long K, int B, int H, int W
     }
 }
 
-// Slot of a launch's span in timing builds (B200_TRK_TIMING): the step index mod 8.  Only the B200_SPAN_* arguments
-// call it, so product builds do not evaluate it.
-[[maybe_unused]] __device__ __forceinline__ int span_slot(const float* rois, long long K) {
-    return (int)((reinterpret_cast<uintptr_t>(rois) / (size_t)(K * 20)) & 7);
-}
-
 // One (ROI k, channels c0 .. c0+cn) tile, start to finish, by one warp.  sMain: L::kMainFloats floats (V staging /
 // big tables, later the output tile), sTab: L::kTabFloats floats; both private to the warp.
 // MULTI (a warp that walks several tiles, roi_align_multi_kernel): the ROI's record arrives in registers (rec0 /
@@ -535,14 +529,12 @@ roi_align_tile_kernel(const T* __restrict__ feat, int B, int C, int H, int W,
     // Warps are independent: no block-wide barriers anywhere below.
     const long long wi = (long long)blockIdx.x * kWarpsPerCta + warp;
     if (wi >= K * ctiles) return;
-    B200_SPAN_BEGIN(span_slot(rois, K));
     float* sMain = smem + (size_t)warp * L::kFloatsPerWarp;
     const unsigned wi32 = (unsigned)wi;       // the launcher keeps the tile count below 2^31
     const long long k = wi32 / (unsigned)ctiles;
     const int c0 = (int)(wi32 % (unsigned)ctiles) * 32;
     process_tile<PH, PW, NHWC, T, PREP, OCL>(feat, B, C, H, W, rois, scale, sr, aligned, out, k, c0, min(32, C - c0),
                                              prep, prep_tabs, sMain, sMain + L::kMainFloats, lane);
-    B200_SPAN_END(span_slot(rois, K));
 }
 
 // Large launches that cannot use the pipelined kernel below (NCHW maps, half storage, 7x7): the tile kernel with a
@@ -566,7 +558,6 @@ roi_align_multi_kernel(const T* __restrict__ feat, int B, int C, int H, int W, c
     const unsigned total = (unsigned)min((long long)(grp + 1) * window, K * ctiles);
     if (t >= total) return;
     asm volatile("griddepcontrol.wait;" ::: "memory");      // roi_prep_kernel's records and tables are complete and visible
-    B200_SPAN_BEGIN(span_slot(rois, K));
     float* sMain = smem + (size_t)warp * L::kFloatsPerWarp;
     unsigned k = t / (unsigned)ctiles;
     int4 h0 = reinterpret_cast<const int4*>(prep + k)[0], h1 = reinterpret_cast<const int4*>(prep + k)[1];
@@ -589,7 +580,6 @@ roi_align_multi_kernel(const T* __restrict__ feat, int B, int C, int H, int W, c
         t = tn; k = kn; h0 = n0; h1 = n1;
     }
     if (pending && lane == 0) bulk_store_wait_read();
-    B200_SPAN_END(span_slot(rois, K));
 }
 
 // ---- software-pipelined persistent kernel: large float32 launches -------------------------------------
@@ -685,7 +675,6 @@ roi_align_pipe_kernel(const T* __restrict__ feat, int B, int C, int H, int W, co
     const unsigned total = (unsigned)min((long long)(grp + 1) * window, K * ctiles);
     if (t >= total) return;
     asm volatile("griddepcontrol.wait;" ::: "memory");      // roi_prep_kernel's records and tables are complete and visible
-    B200_SPAN_BEGIN(span_slot(rois, K));
 
     // current tile (a*), next tile (n*): ROI index, first channel, prep record
     unsigned ka = t / (unsigned)ctiles;
@@ -806,7 +795,6 @@ roi_align_pipe_kernel(const T* __restrict__ feat, int B, int C, int H, int W, co
         tn = tm; kn = km; cnx = cm; n0 = m0; n1 = m1;
         par ^= 1;
     }
-    B200_SPAN_END(span_slot(rois, K));
 }
 
 
@@ -1006,7 +994,6 @@ roi_align_tma_kernel(const __grid_constant__ TmaMaps tmap, const float* __restri
     const unsigned total = (unsigned)min((long long)(grp + 1) * window, K * ctiles);
     if (t >= total) return;
     asm volatile("griddepcontrol.wait;" ::: "memory");      // roi_prep_kernel's records and tables are complete and visible
-    B200_SPAN_BEGIN(span_slot(rois, K));
     if (lane == 0) {
         mbar_init(sbar, 1);
         mbar_init(sbar + 8, 1);
@@ -1142,7 +1129,6 @@ roi_align_tma_kernel(const __grid_constant__ TmaMaps tmap, const float* __restri
         par ^= 1;
     }
     if (pending && lane == 0) bulk_store_wait_read();
-    B200_SPAN_END(span_slot(rois, K));
 }
 
 // Any output size / any parameters: one thread per output element, direct sampling.
@@ -1951,5 +1937,3 @@ extern "C" int b200_roi_align_bwd_ex(const void* grad_out, int dtype, int grad_o
                                                spatial_scale, sampling_ratio, aligned, grad_in, layout, B, C, H, W, stream);
     });
 }
-
-B200_SPAN_GETTER(b200_debug_spans_roi)

@@ -27,22 +27,6 @@
 namespace b200 {
 namespace trk {
 
-struct Span {                     // RAII global-timer span of one kernel (debug builds only)
-    int k;
-    __device__ explicit Span(int kk) : k(kk) { B200_SPAN_BEGIN(k); }
-    __device__ ~Span() { B200_SPAN_END(k); }
-};
-
-#ifdef B200_TRK_TIMING          // debug builds only: SM-clock stamps at phase boundaries of stream 0
-__device__ long long g_timing[32];
-#define TRK_STAMP(k) do { __syncthreads(); if (threadIdx.x == 0 && blockIdx.x == 0) g_timing[k] = clock64(); } while (0)
-// global-timer stamps of the fused step's phases (CTA 0 of stream 0), slots 16..31 of the same array
-#define TRK_GSTAMP(k) do { __syncthreads(); if (threadIdx.x == 0 && blockIdx.x == 0 && blockIdx.y == 0) g_timing[16 + (k)] = (long long)::b200::gtime(); } while (0)
-#else
-#define TRK_STAMP(k) do { } while (0)
-#define TRK_GSTAMP(k) do { } while (0)
-#endif
-
 // Programmatic dependent launch (used for small stream counts, see b200_tracker_step): let the next kernel of
 // the step become resident while this one runs, then wait until the previous kernel has completed and its
 // writes are visible.  Both instructions are no-ops for a kernel launched without the attribute.
@@ -252,7 +236,6 @@ __device__ inline void predict_slot(const Dev& d, size_t slot) {
 
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kThreads) begin_kernel(Dev d) {
-    Span span((d.frame_id[0] & 7) * 6 + 0);
     __shared__ int scratch[kThreads / 32];
     const int s = blockIdx.x, tid = threadIdx.x;
     int* cnt = d.cnt + s * kHdr;
@@ -325,7 +308,6 @@ __device__ inline void cost2_item(const Dev& d, int s, int r, int j0, float* sme
 }
 
 __global__ void __launch_bounds__(cost::kThreads) cost2_kernel(Dev d) {
-    Span span((d.frame_id[0] & 7) * 6 + 3);
     TRK_PDL_PROLOGUE();
     extern __shared__ __align__(16) float smem[];
     __shared__ int s_idx[cost::kTileN];
@@ -384,7 +366,6 @@ __device__ __forceinline__ unsigned fkey(float f) {                 // order-pre
 }
 
 __global__ void __launch_bounds__(kCost1Warps * 32) cost1_sparse_kernel(Dev d) {
-    Span span((d.frame_id[0] & 7) * 6 + 1);
     TRK_PDL_PROLOGUE();
     const int total = d.wcount[0];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -607,7 +588,6 @@ __device__ __forceinline__ void cost1_row32(const Dev& d, int s, int r, size_t s
 }
 
 __global__ void __launch_bounds__(kCost1Warps * 32, 2) cost1_sparse32_kernel(Dev d) {
-    Span span((d.frame_id[0] & 7) * 6 + 1);
     TRK_PDL_PROLOGUE();
     const int total = d.wcount[0];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -743,7 +723,6 @@ __device__ __forceinline__ void update_entries(const Dev& d, int first, int tota
 }
 
 __global__ void __launch_bounds__(kUpdWarps * 32) update_kernel(Dev d) {
-    Span span((d.frame_id[0] & 7) * 6 + 5);
     TRK_PDL_PROLOGUE();
     __shared__ double scratch[kUpdWarps * 4 * 96];
     const int warp = threadIdx.x >> 5;
@@ -839,7 +818,6 @@ __device__ inline bool assign_body(const Dev& d, int s, unsigned char* smem_raw,
     int* m_col = d.tmp + sb;                        // column (local det index) of each match
     int n_match = 0, n_ut = 0, n_left = N;
     bool failed = false;                            // uniform across the CTA
-    if (STAGE == 1) TRK_STAMP(0);
 
     if (M > 0 && N > 0) {
         const bool tall = M > N;
@@ -855,7 +833,6 @@ __device__ inline bool assign_body(const Dev& d, int s, unsigned char* smem_raw,
                                          pre ? d.row_fv + sb : nullptr);
         if (tid == 0) s_rc = rc;
         __syncthreads();
-        if (STAGE == 1) TRK_STAMP(1);
         if (s_rc != B200_OK) {                      // NaN / infeasible: scipy would raise
             failed = true;
             if (tid == 0) { cnt[C_STATUS] = s_rc; if (STAGE == 1) cnt[C_MODE] = MODE_FAILED; }
@@ -902,7 +879,6 @@ __device__ inline bool assign_body(const Dev& d, int s, unsigned char* smem_raw,
                                [&](int pos, int j) { d.ud1[db + pos] = j; }, scratch);
         if (tid == 0) { cnt[C_NU] = n_left; cnt[C_NMATCH] = n_match; cnt[C_NUT] = n_ut; }
         if (!INLINE) enqueue_cost_work(d.work2, d.wcount + 1, s, n_left > 0 ? cnt[C_M2] : 0, n_left, scratch);
-        TRK_STAMP(5);
         __syncthreads();
         return false;
     }
@@ -931,7 +907,6 @@ __device__ inline bool assign_body(const Dev& d, int s, unsigned char* smem_raw,
 
 template <int STAGE>
 __global__ void __launch_bounds__(kThreads) assign_kernel(Dev d, int smem_matrix_floats) {
-    Span span((d.frame_id[0] & 7) * 6 + (STAGE == 1 ? 2 : 4));
     TRK_PDL_PROLOGUE();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     assign_body<STAGE, false, false>(d, blockIdx.x, smem_raw, smem_matrix_floats);
@@ -952,11 +927,9 @@ __global__ void __launch_bounds__(kThreads) assign_kernel(Dev d, int smem_matrix
 constexpr int kFrontWarps = 4;
 
 __global__ void __launch_bounds__(kFrontWarps * 32, 2) front_kernel(Dev d) {
-    Span span((d.frame_id[0] & 7) * 6 + 0);
     extern __shared__ __align__(16) int s_rows[];              // rows_main [MT] | rows_reid [MT]
     __shared__ int scratch[kThreads / 32];
     const int s = blockIdx.y, g = blockIdx.x, G = gridDim.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    TRK_GSTAMP(0);
     int* cnt = d.cnt + s * kHdr;
     const size_t sb = (size_t)s * d.MT;
     const int n = d.n_det[s], nl = d.hdr[s * kHdr + H_NLIVE];
@@ -978,20 +951,17 @@ __global__ void __launch_bounds__(kFrontWarps * 32, 2) front_kernel(Dev d) {
             cnt[C_NMATCH] = 0; cnt[C_NUT] = 0; cnt[C_STATUS] = 0;
         }
     }
-    TRK_GSTAMP(1);
     prep_detections(d, s, n, g, G);
     // ---- predict_all (:340-345): thread per track, the tracks of the rows this CTA owns (r = g, g + G, ...) ----
     const int own1 = M1 > g ? (M1 - g + G - 1) / G : 0, own2 = M2 > g ? (M2 - g + G - 1) / G : 0;
     for (int i = tid; i < own1 + own2; i += blockDim.x)
         predict_slot(d, sb + (i < own1 ? rm[g + i * G] : rr[g + (i - own1) * G]));
     __syncthreads();
-    TRK_GSTAMP(2);
     // ---- stage-1 cost of the owned rows, one warp per row ----
     for (int i = warp; i < own1; i += kFrontWarps) {
         const int r = g + i * G;
         cost1_row32<true>(d, s, r, sb + rm[r], n, lane);
     }
-    TRK_GSTAMP(3);
 }
 
 // Launched as thread-block clusters of kBackCluster CTAs per stream when the handle has few streams (latency mode): CTA 0
@@ -1020,17 +990,14 @@ __device__ __forceinline__ void cluster_sync_all() {       // release / acquire 
 // fits beside resident ROI Align CTAs, which the 238-register form does not.
 template <bool UPDATES>
 __global__ void __launch_bounds__(kThreads, UPDATES ? 1 : 2) back_kernel(Dev d, int smem_matrix_floats) {
-    Span span((d.frame_id[0] & 7) * 6 + 2);
     TRK_PDL_PROLOGUE();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ int s_idx[cost::kTileN];
     const unsigned rank = cluster_ctarank(), nrank = cluster_nctarank();
     const int s = blockIdx.x / nrank, tid = threadIdx.x;
     const int* cnt = d.cnt + s * kHdr;
-    TRK_GSTAMP(4);
     if (rank == 0) {
         if (!assign_body<1, true, UPDATES>(d, s, smem_raw, smem_matrix_floats)) {
-            TRK_GSTAMP(5);
             // ReID-only cost (:552-558) of this stream's long-lost rows against the leftover detections
             const int M2 = cnt[C_M2], NU = cnt[C_NU];
             if (M2 > 0 && NU > 0) {
@@ -1040,10 +1007,8 @@ __global__ void __launch_bounds__(kThreads, UPDATES ? 1 : 2) back_kernel(Dev d, 
             }
             __syncthreads();
         }
-        TRK_GSTAMP(6);
         assign_body<2, true, UPDATES>(d, s, smem_raw, smem_matrix_floats);
         __syncthreads();
-        TRK_GSTAMP(7);
     }
     if (!UPDATES) return;
     if (nrank > 1) cluster_sync_all();
@@ -1053,7 +1018,6 @@ __global__ void __launch_bounds__(kThreads, UPDATES ? 1 : 2) back_kernel(Dev d, 
     const int warp = tid >> 5;
     update_entries(d, (int)((size_t)s * d.MT), total, (int)rank * (kThreads / 32) + warp, (int)nrank * (kThreads / 32),
                    reinterpret_cast<double*>(smem_raw) + (size_t)warp * 4 * 96);
-    TRK_GSTAMP(8);
 }
 
 
@@ -2065,23 +2029,6 @@ extern "C" int b200_tracker_export(b200_tracker* t, int stream_idx, int32_t* ids
     return (int)n;
 }
 
-#ifdef B200_TRK_TIMING
-extern "C" int b200_debug_lsap_stats(unsigned long long* out4, int reset) {
-    unsigned long long z[4] = {0, 0, 0, 0};
-    if (out4) cudaMemcpyFromSymbol(out4, b200::lsap::g_lsap_stats, sizeof(z));
-    if (reset) cudaMemcpyToSymbol(b200::lsap::g_lsap_stats, z, sizeof(z));
-    return 0;
-}
-extern "C" int b200_debug_lsap_clk(long long* out8) {
-    cudaMemcpyFromSymbol(out8, b200::lsap::g_lsap_clk, 8 * sizeof(long long));
-    return 0;
-}
-
-extern "C" int b200_debug_timing(long long* out32) {
-    return cudaMemcpyFromSymbol(out32, b200::trk::g_timing, sizeof(long long) * 32) == cudaSuccess ? 0 : -2;
-}
-#endif
-
 extern "C" int b200_tracker_import(b200_tracker* t, int stream_idx, int n, const int32_t* ids, const double* x,
                                    const double* P, const uint8_t* stage, const float* ema, const float* bank,
                                    const int32_t* bank_len, const int32_t* miss, const int32_t* age,
@@ -2122,5 +2069,3 @@ extern "C" int b200_tracker_import(b200_tracker* t, int stream_idx, int n, const
                  "[0, next_id), bank_len outside [0, hist_max] or stage > 2)", stream_idx);
     return B200_OK;
 }
-
-B200_SPAN_GETTER(b200_debug_spans_trk)

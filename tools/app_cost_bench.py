@@ -1,7 +1,6 @@
-"""Dense appearance cost (north_star kernel 2): M tracks x 30 bank rows x 128 against N detections, the tensor-core
-kernels (default) or the float32 FFMA kernel (B200TRACK_NO_TC=1), CUDA events around whole calls with L2 flushed in
-front of each + max error against a float64 reference.  One JSON line per shape, each with the device name, power limit
-and library read in the same run.
+"""Dense appearance cost (north_star kernel 2): M tracks x 30 bank rows x 128 against N detections through the public
+call, CUDA events around whole calls with L2 flushed in front of each + max error against a float64 reference.  One
+JSON line per shape, each with the device name, power limit and library read in the same run.
 
 usage: python tools/app_cost_bench.py [MxN ...]        (default: 512x512, BASELINE config 4)"""
 import json, os, subprocess, sys
@@ -18,9 +17,9 @@ q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,
                    capture_output=True, text=True).stdout.strip().split(",")
 info = {"device": torch.cuda.get_device_name(0), "power_limit_w": float(q[1]) if len(q) > 1 else None,
         "lib": os.path.basename(_lib.LIB_PATH)}
-tc = not os.environ.get("B200TRACK_NO_TC")
 flush = torch.empty(64 * 1024 * 1024, device="cuda")
 for M, N in shapes:
+    tc = M * N >= 64 * 64                       # smaller problems run the float32 FFMA kernel (app_cost_tc.cu)
     g = torch.Generator(device="cuda").manual_seed(0)
     bank = torch.nn.functional.normalize(torch.randn((M, T, 128), device="cuda", generator=g), dim=2)
     det = torch.nn.functional.normalize(torch.randn((N, 128), device="cuda", generator=g), dim=1)
